@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s of the per-ray render path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 Workload (config 3 of BASELINE.json, the one the metric is quoted on): synthetic 1 M random
 Gaussians, SH degree 3, seed 1002, 1920x1080, vertical fov 60 deg, orbit radius 2.2, depth 16.
@@ -31,6 +31,16 @@ roofline = the dominant kernel, k_shade_tiles (intersection + k-buffer + SH comp
          "kernels" lists every kernel of the step with its mean time and share
 cpu_baseline = oracle/ref_cpu.cpp (reference-shaped C++/OpenMP port, float32, every core this process may use)
          on a pixel subsample
+
+Steps: value, serial_value and e2e run exactly K timed steps.  To bound the run time, the secondary legs cap K
+and report what they ran: tiles min(K, 128) frames and tiles_config4 min(K, 32) ("frames"), cpu_baseline
+min(K, 32) steps ("steps"; --impl reference runs K).
+
+--dump-outputs DIR writes the frame of the last timed step of the one-stream (serial_value) loop as DIR/frame.npy
+((W,H,3) float32; at N > 1 every rank's frame, DIR/frame_rank<r>.npy, written by rank 0), read back untimed.  It is
+not taken from the two-stream loop that gives `value`: there both streams store into one buffer, so what that loop
+leaves behind need not be a single step's frame; both loops render the same views.  The inputs are seeded, so two
+builds run with the same arguments compare output for output.
 """
 from __future__ import annotations
 
@@ -54,6 +64,7 @@ N_VIEWS = 64
 DEPTH = 16
 T_CUT = 1e-4
 FALLBACK_HBM_GBS = 6650.0   # B200_PROFILING.md fallback
+DUMP_MAX_BYTES = 64_000_000
 
 
 def parse_args():
@@ -81,6 +92,10 @@ def parse_args():
                          "trained scene do to 10-bit-per-axis Morton codes)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-stride", type=int, default=0, help="pixel subsample stride of the CPU legs (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step (one-stream loop) as DIR/frame.npy, (W,H,3) float32; "
+                         "at N > 1, rank 0 writes every rank's frame as DIR/frame_rank<r>.npy.  Above 64 MB in all, "
+                         "every file keeps the same fixed, seeded sample of pixels, as (n,3)")
     return ap.parse_args()
 
 
@@ -200,9 +215,26 @@ def cpu_leg(cfg_name, scene_arrays, W, H, focal, views, steps, warmup, stride):
             times.append(dt)
     total = sum(times)
     return {"mrays": pix.shape[0] * len(times) / total / 1e6, "ms_per_step": 1e3 * total / len(times),
-            "cores": threads, "rays_per_step": int(pix.shape[0]), "build_s": build_s,
+            "cores": threads, "rays_per_step": int(pix.shape[0]), "build_s": build_s, "steps": len(times),
             "sample": f"every {stride}th column and row of each {W}x{H} view ({pix.shape[0]} rays/step), "
                       f"{len(times)} steps, float32, K={DEPTH} closest-hit restarts over the LBVH"}
+
+
+def dump_outputs(path, frames, max_bytes=DUMP_MAX_BYTES):
+    """Write `frames` (name -> (W,H,3) float32 array) as path/<name>.npy, at most `max_bytes` in all: above that every
+    file keeps the same seeded sample of pixels, so two runs with the same arguments compare pixel for pixel."""
+    path = Path(path)
+    path.mkdir(parents=True, exist_ok=True)
+    header = 128                                        # bytes of the .npy header of an array of up to 3 dimensions
+    W, H, _ = next(iter(frames.values())).shape
+    npix = W * H
+    total = sum(a.nbytes + header for a in frames.values())
+    if total > max_bytes:
+        keep = (max_bytes - header * len(frames)) * npix // (total - header * len(frames))
+        idx = np.sort(np.random.default_rng(0).choice(npix, size=keep, replace=False))
+        frames = {k: a.reshape(npix, -1)[idx] for k, a in frames.items()}
+    for k, a in frames.items():
+        np.save(path / f"{k}.npy", np.ascontiguousarray(a, dtype=np.float32))
 
 
 def views_of(W, H):
@@ -468,6 +500,8 @@ def main():
 
     # ------------------------------------------------------------------ reference arm (CPU port)
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the CUDA path's frames (--impl ours)")
         if rank != 0:
             return 0
         focal, views = make_views(W, H, n_views, orbit_phi)
@@ -597,6 +631,16 @@ def main():
         launches += launches_per_frame
     e_end.record()
     barrier()
+    # the last step's frame, read back untimed; the two-stream loop below renders the same steps, but both streams
+    # store into the same buffer, so what it leaves there need not be one step's frame
+    last_frames = None
+    if args.dump_outputs:
+        if rank == 0:
+            last_frames = ({"frame": out.cpu().numpy()} if peer is None else
+                           {f"frame_rank{r}": peer.frame(r).cpu().numpy() for r in range(world)})
+        # the last step released its peer buffer, so the other ranks' next frames may already store into it:
+        # hold them until rank 0 has read it back
+        barrier()
     serial_ms = e_beg.elapsed_time(e_end)
     kern_ms = [a.elapsed_time(b) for a, b in ev]
     per_kernel = scene.read_kernel_times(timed_frames).astype(np.float64).mean(axis=0)   # ms of the frame's launches
@@ -638,7 +682,8 @@ def main():
             if prev is not None:
                 prev.result()
             prev = cur
-        prev.result()
+        if prev is not None:
+            prev.result()
 
     def wall(fn, n):
         fn(min(args.warmup, 3))
@@ -761,9 +806,11 @@ def main():
             stride = args.cpu_stride or (4 if W * H <= 1920 * 1080 else 8)
             r = cpu_leg(args.config, arrays, W, H, focal, views, min(args.steps, 32), 1, stride)   # ~10-20 s of CPU work
             line["cpu_baseline"] = {"value": r["mrays"], "unit": "Mrays/s", "cores": r["cores"], "kind": "port",
-                                    "sample": r["sample"]}
+                                    "steps": r["steps"], "sample": r["sample"]}
         else:
             line["cpu_baseline"] = None
+        if last_frames is not None:
+            dump_outputs(args.dump_outputs, last_frames)
         print(json.dumps(line))
     if dist is not None:
         dist.barrier()

@@ -55,7 +55,8 @@ def test_errors_are_reported_not_thrown(lib):
 
 
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
-    import importlib
+    # monkeypatch restores the module afterwards; reloading it instead would replace the ctypes classes
+    # (rtgs_camera, ...) that the already loaded library's argtypes name, and break every later render call
     from rtgs import _native
     monkeypatch.setattr(_native, "_lib", None)
     monkeypatch.setattr(_native, "LIB_PATH", tmp_path / "nope.so")
@@ -65,4 +66,3 @@ def test_missing_library_fails_loudly(monkeypatch, tmp_path):
         assert "no CPU fallback" in str(e)
     else:
         raise AssertionError("loading a missing library must raise")
-    importlib.reload(_native)
