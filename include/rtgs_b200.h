@@ -157,6 +157,26 @@ int rtgs_render(rtgs_scene* s, const rtgs_camera* cam,
                 int32_t depth, float t_cut, int32_t accumulate, int32_t full_image_pitch,
                 float* out_rgb, float* out_T, void* stream, rtgs_render_stats* stats);
 
+/* Replace the stored parameters of a scene (same n, same SH presence) from DEVICE pointers on the scene's device
+ * (layouts of rtgs_scene_create; sh NULL iff the scene has none; values must be finite), then the caller calls
+ * rtgs_scene_build_bvh.  Renders/backward before the rebuild fail with RTGS_ERR_STATE.  The copies are ordered after
+ * prior work on `stream`, and the rebuild (on the scene's own stream) after the copies.  The source buffers are read
+ * until rtgs_scene_build_bvh returns. */
+int rtgs_scene_set_gaussians_device(rtgs_scene* s, const float* pos, const float* rot_xyzw, const float* scale,
+                                    const float* color, const float* opacity, const float* sh, void* stream);
+
+/* Backward of rtgs_render for the region (x0,y0,w,h): dL_drgb (w,h,3) and optional dL_dT (w,h) are device, i-major
+ * region buffers.  Gradients are ACCUMULATED (+=) into device buffers in ORIGINAL Gaussian order, layouts of
+ * rtgs_scene_create (grad_sh (n,15,3)); any grad pointer may be NULL.  replay_rgb / replay_T (optional, (w,h,3)/(w,h))
+ * receive the image the backward recomputed - the consistency check against rtgs_render.  Independent of
+ * RTGS_OPT_RENDER_MODE / _STRIPE / _HEAVY_LISTS; uses no per-frame scene scratch.
+ * The gradient is that of the image with each pixel's layer list (the `depth` nearest entries, t_cut applied) held
+ * fixed: membership, order and the q = 3 silhouette have none; the camera pose gets none. */
+int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                         int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                         float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                         float* grad_opacity, float* grad_sh, float* replay_rgb, float* replay_T, void* stream);
+
 /* Tuning knobs of one scene's render path (no reference counterpart; defaults need no call).
  *  RTGS_OPT_RENDER_MODE      0 (default): k_tile_lists (traversal, one candidate list per 4x8-pixel tile) +
  *                            k_shade_tiles (intersection, k-buffer, compositing) + the fused kernel k_render for the

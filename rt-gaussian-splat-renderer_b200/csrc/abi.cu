@@ -468,6 +468,56 @@ int rtgs_render(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, i
     return RTGS_OK;
 }
 
+int rtgs_scene_set_gaussians_device(rtgs_scene* s, const float* pos, const float* rot_xyzw, const float* scale,
+                                    const float* color, const float* opacity, const float* sh, void* stream) {
+    RTGS_CHECK_ARG(s != nullptr);
+    RTGS_CHECK_ARG(pos && rot_xyzw && scale && color && opacity);
+    RTGS_CHECK_ARG((sh != nullptr) == s->has_sh);
+    DeviceGuard g(s->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    // renders and backward passes read the packed records, which only the rebuild refreshes
+    s->built = false;
+    const int64_t n = s->n;
+    auto cp = [&](float* d, const float* src, size_t cnt) {
+        return cudaMemcpyAsync(d, src, cnt * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    };
+    CUDA_TRY(cp(s->pos, pos, n * 3));
+    CUDA_TRY(cp(s->rot, rot_xyzw, n * 4));
+    CUDA_TRY(cp(s->scale, scale, n * 3));
+    CUDA_TRY(cp(s->color, color, n * 3));
+    CUDA_TRY(cp(s->opacity, opacity, n));
+    if (sh) CUDA_TRY(cp(s->sh, sh, n * 45));
+    // the build runs on the scene's own stream: it starts after the copies (and everything before them on `stream`,
+    // e.g. a backward pass still reading the old records)
+    cudaEvent_t ev = nullptr;
+    CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    cudaError_t e = cudaEventRecord(ev, st);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(s->own_stream, ev, 0);
+    cudaEventDestroy(ev);
+    CUDA_TRY(e);
+    return RTGS_OK;
+}
+
+int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                         int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT, float* grad_pos,
+                         float* grad_rot, float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
+                         float* replay_rgb, float* replay_T, void* stream) {
+    RTGS_CHECK_ARG(s != nullptr);
+    TRY(check_camera(cam));
+    RTGS_CHECK_ARG(dL_drgb != nullptr);
+    RTGS_CHECK_ARG(w > 0 && h > 0 && x0 >= 0 && y0 >= 0 && x0 + w <= cam->width && y0 + h <= cam->height);
+    RTGS_CHECK_ARG(depth >= 1 && depth <= RTGS_MAX_DEPTH);
+    RTGS_CHECK_ARG(t_cut >= 0.0f && t_cut < 1.0f);
+    if (!s->built) {
+        rtgs_set_error("rtgs_render_backward: call rtgs_scene_build_bvh first");
+        return RTGS_ERR_STATE;
+    }
+    DeviceGuard g(s->device);
+    float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
+    return rtgs_launch_render_backward(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads, replay_rgb,
+                                       replay_T, (cudaStream_t)stream);
+}
+
 int rtgs_scene_set_option(rtgs_scene* s, int32_t option, int64_t value) {
     RTGS_CHECK_ARG(s != nullptr);
     switch (option) {

@@ -21,8 +21,10 @@
 //                  the traversal's shared-memory list (heavy_lists.cuh), between k_tile_lists and k_shade_tiles
 //   k_render       fused.cuh (mode 1, depth > 16, fallback tiles)
 //   k_generate_rays, k_trace_closest, k_activate_ply   API companions (Camera.generate_ray_field, Scene.hit, PLY ingest)
+//   k_render_backward  gradient of the render with respect to the Gaussian parameters (backward.cuh)
 #include <stdlib.h>
 
+#include "backward.cuh"
 #include "fused.cuh"
 #include "heavy_lists.cuh"
 #include "shade.cuh"
@@ -354,21 +356,7 @@ __global__ void k_trace_closest(const float4* __restrict__ nodes, const float4* 
     int sp = 0;
     stack[sp++] = 0;
     auto slab = [&](float mnx, float mny, float mnz, float mxx, float mxy, float mxz) -> float {
-        // returns entry distance or +inf on a miss (bounding_box.py:50-89; hit iff t_min < t_max)
-        float t0 = -INFINITY, t1 = INFINITY;
-        const float mn[3] = {mnx, mny, mnz}, mx[3] = {mxx, mxy, mxz};
-#pragma unroll
-        for (int a = 0; a < 3; ++a) {
-            float ta = (mn[a] - of[a]) * idx_[a], tb = (mx[a] - of[a]) * idx_[a];
-            float lo = fminf(ta, tb), hi = fmaxf(ta, tb);
-            // inflate by a few ulp so float32 rounding can never cull a true hit
-            lo -= 4e-6f * fabsf(lo) + 1e-30f;
-            hi += 4e-6f * fabsf(hi) + 1e-30f;
-            if (ta != ta || tb != tb) { lo = -INFINITY; hi = INFINITY; }   // 0 * inf: ray inside slab plane
-            t0 = fmaxf(t0, lo);
-            t1 = fminf(t1, hi);
-        }
-        return (t0 <= t1) ? t0 : INFINITY;
+        return slab_entry(of, idx_, {mnx, mny, mnz}, {mxx, mxy, mxz});
     };
     while (sp > 0) {
         const int node = stack[--sp];
@@ -930,6 +918,33 @@ int rtgs_launch_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, i
                               cudaStream_t stream) {
     if (nrays == 0) return RTGS_OK;
     k_trace_closest<<<(int)((nrays + 127) / 128), 128, 0, stream>>>(s->nodes, s->raw, nrays, rays, idx, t12);
+    CUDA_TRY(cudaGetLastError());
+    return RTGS_OK;
+}
+
+int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h, int depth,
+                                float t_cut, const float* dL_drgb, const float* dL_dT, float* const grads[6],
+                                float* replay_rgb, float* replay_T, cudaStream_t stream) {
+    backward::BackwardParams P;
+    P.nodes = s->nodes;
+    P.geo = s->geo;
+    P.shp = s->shp;
+    P.raw = s->raw;
+    P.cam = make_camd(cam);
+    P.x0 = x0; P.y0 = y0; P.w = w; P.h = h;
+    P.tiles_j = (h + TILE_J - 1) / TILE_J;
+    P.ntiles = ((w + TILE_I - 1) / TILE_I) * P.tiles_j;
+    P.depth = depth;
+    P.t_cut = t_cut;
+    P.has_sh = s->has_sh ? 1 : 0;
+    P.dL_drgb = dL_drgb;
+    P.dL_dT = dL_dT;
+    P.g_pos = grads[0]; P.g_rot = grads[1]; P.g_scale = grads[2];
+    P.g_color = grads[3]; P.g_opacity = grads[4]; P.g_sh = s->has_sh ? grads[5] : nullptr;
+    P.replay_rgb = replay_rgb;
+    P.replay_T = replay_T;
+    const int blocks = (P.ntiles + backward::BWD_WARPS - 1) / backward::BWD_WARPS;
+    backward::k_render_backward<<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }

@@ -372,6 +372,26 @@ __device__ __forceinline__ void plane_side(float nx, float ny, float nz, float d
     hi = dist <= 0.0f || reach;
 }
 
+// ---- per-ray box test of the stack traversals (k_trace_closest, k_render_backward) -----------------
+// Entry distance of the ray (origin of, inverse direction idf) into the box [mn, mx], or +inf on a miss
+// (bounding_box.py:50-89; hit iff t_min < t_max).  Float32 slabs inflated by a few ulp, so that rounding can never
+// cull a true hit.
+__device__ __forceinline__ float slab_entry(const float (&of)[3], const float (&idf)[3], const float (&mn)[3],
+                                            const float (&mx)[3]) {
+    float t0 = -INFINITY, t1 = INFINITY;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        float ta = (mn[a] - of[a]) * idf[a], tb = (mx[a] - of[a]) * idf[a];
+        float lo = fminf(ta, tb), hi = fmaxf(ta, tb);
+        lo -= 4e-6f * fabsf(lo) + 1e-30f;
+        hi += 4e-6f * fabsf(hi) + 1e-30f;
+        if (ta != ta || tb != tb) { lo = -INFINITY; hi = INFINITY; }   // 0 * inf: ray inside slab plane
+        t0 = fmaxf(t0, lo);
+        t1 = fminf(t1, hi);
+    }
+    return (t0 <= t1) ? t0 : INFINITY;
+}
+
 // ---- float64 exact evaluation from raw parameters (rare path) ---------------------------------
 __device__ __noinline__ static ExactHit exact_eval(const float4* __restrict__ raw, const CamD& cam, int s, int pi,
                                                    int pj) {

@@ -215,6 +215,47 @@ class RayTracer:
             self.last_stats = stats.as_dict()
         return out
 
+    def render_backward(self, dL_drgb, dL_dT=None, depth: int = 16, tile=None, grads=None, replay: bool = False):
+        """Gradient of ``render_device(depth, tile)`` (with ``t_cut``) with respect to the stored Gaussian parameters,
+        the layer list of every pixel held fixed (rtgs_render_backward), on the current stream.
+
+        dL_drgb (w,h,3) and dL_dT (w,h) are CUDA float32 tensors of the region.  Returns a dict of (n,...) float32
+        gradients ``pos rot scale color opacity`` and ``sh`` (scenes with SH): ``grads`` may pass tensors of these
+        names to accumulate into (missing ones are zero-initialised).  With ``replay=True`` the dict also holds
+        ``rgb`` / ``T``, the image the backward recomputed."""
+        import torch
+        W, H = self.buf_size.x, self.buf_size.y
+        x0, y0, w, h = (0, 0, W, H) if tile is None else tile
+        n = self.scene.num_gaussians
+
+        def region(t, shape, name):
+            if t.device != self._dev or t.dtype != torch.float32 or tuple(t.shape) != shape:
+                raise ValueError(f"{name}: expected a float32 tensor of shape {shape} on {self._dev}")
+            return t.contiguous()
+
+        dL_drgb = region(dL_drgb, (w, h, 3), "dL_drgb")
+        dL_dT = None if dL_dT is None else region(dL_dT, (w, h), "dL_dT")
+        shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
+        if self.scene.has_sh:
+            shapes["sh"] = (n, 15, 3)
+        out = dict(grads or {})
+        for name, shape in shapes.items():
+            if name not in out:
+                out[name] = torch.zeros(shape, dtype=torch.float32, device=self._dev)
+            elif (out[name].dtype != torch.float32 or tuple(out[name].shape) != shape or not out[name].is_contiguous()
+                  or out[name].device != self._dev):
+                raise ValueError(f"grads[{name!r}]: expected a contiguous float32 tensor of shape {shape}")
+        if replay:
+            out["rgb"] = torch.empty((w, h, 3), dtype=torch.float32, device=self._dev)
+            out["T"] = torch.empty((w, h), dtype=torch.float32, device=self._dev)
+        cam = self.camera.native()
+        ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
+        _native.check(_native.load().rtgs_render_backward(
+            self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, dL_drgb.data_ptr(),
+            None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
+            ptr("opacity"), ptr("sh"), ptr("rgb"), ptr("T"), torch.cuda.current_stream(self._dev).cuda_stream))
+        return out
+
     def _render_into(self, depth, accumulate):
         import torch
         if depth > MAX_DEPTH:

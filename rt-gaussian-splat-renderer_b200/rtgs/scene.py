@@ -170,6 +170,38 @@ class Scene:
         self._adopt(h, n, dev, shp is not None)
         return self
 
+    def set_gaussians(self, pos, rot, scale, color, opacity, sh=None):
+        """Replace the stored parameters in place from CUDA float32 tensors on the scene's device and rebuild the
+        LBVH (rtgs_scene_set_gaussians_device + rtgs_scene_build_bvh): no host round trip, same handle.  Shapes as
+        in ``from_arrays`` (n fixed); ``sh`` must be given iff the scene has SH.  The copies are ordered after the
+        work already queued on the current stream."""
+        import torch
+        n = self._n
+        dev = torch.device("cuda", self.device)
+        want = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
+        args = dict(pos=pos, rot=rot, scale=scale, color=color, opacity=opacity)
+        if (sh is not None) != self.has_sh:
+            raise ValueError("sh must be given iff the scene has SH coefficients")
+        if sh is not None:
+            want["sh"], args["sh"] = (n, 15, 3), sh
+        for name, t in args.items():
+            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.float32:
+                raise ValueError(f"{name}: expected a float32 tensor on {dev}")
+            if tuple(t.shape) != want[name] or not t.is_contiguous():
+                raise ValueError(f"{name}: expected a contiguous tensor of shape {want[name]}, got {tuple(t.shape)}")
+        self.drain_pending()
+        lib = _native.load()
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _native.check(lib.rtgs_scene_set_gaussians_device(
+            self.handle, pos.data_ptr(), rot.data_ptr(), scale.data_ptr(), color.data_ptr(), opacity.data_ptr(),
+            None if sh is None else sh.data_ptr(), stream))
+        self._gaussian_field = self._bvh_field = self._lbvh = None
+        _native.check(lib.rtgs_scene_build_bvh(self.handle, int(self.leaf_prim)))
+        bits = C.c_int32()
+        _native.check(lib.rtgs_scene_morton_bits(self.handle, C.byref(bits)))
+        self.morton_bits = int(bits.value)
+        return self
+
     def _adopt(self, handle, n, dev, has_sh):
         self._handle = handle
         self._n = int(n)
