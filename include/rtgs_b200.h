@@ -171,11 +171,28 @@ int rtgs_scene_set_gaussians_device(rtgs_scene* s, const float* pos, const float
  * receive the image the backward recomputed - the consistency check against rtgs_render.  Independent of
  * RTGS_OPT_RENDER_MODE / _STRIPE / _HEAVY_LISTS; uses no per-frame scene scratch.
  * The gradient is that of the image with each pixel's layer list (the `depth` nearest entries, t_cut applied) held
- * fixed: membership, order and the q = 3 silhouette have none; the camera pose gets none. */
+ * fixed: membership, order and the q = 3 silhouette have none.  The camera gets none here: see
+ * rtgs_render_backward_camera. */
 int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
                          int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
                          float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
                          float* grad_opacity, float* grad_sh, float* replay_rgb, float* replay_T, void* stream);
+
+/* rtgs_render_backward plus the gradient with respect to the camera: grad_cam_pos (3), grad_cam_rot (4, the stored
+ * x,y,z,w quaternion) and grad_cam_focal (2: fx, fy), device float32, ACCUMULATED (+=), any of them NULL.  With all
+ * three NULL the call is rtgs_render_backward.  Same arguments, checks and layer-list definition otherwise.
+ * The camera enters the image only through each pixel's ray: origin o = position, direction d = Rm(q) n / |n| with
+ * n = (px, py, -1), px = (i + 0.5 - W/2) / fx, py = (j + 0.5 - H/2) / fy and Rm = as_rotation_mat3 of the stored
+ * quaternion as given (not normalised, so |d| = |q|^2).  Per layer dq/do = 2 W^T e and dq/dd = -2 sigma W^T e (the
+ * terms of the Gaussian gradient), and the SH colour depends on d / |d|.  The camera gradient is summed in float64
+ * in a fixed order and rounded to float32 once per value: two identical calls give bit-identical results.  A
+ * temporary buffer of 112 bytes per 4 tiles (4x8 pixels each) is allocated and freed stream-ordered on `stream`. */
+int rtgs_render_backward_camera(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                                int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                                float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                                float* grad_opacity, float* grad_sh,
+                                float* grad_cam_pos, float* grad_cam_rot, float* grad_cam_focal,
+                                float* replay_rgb, float* replay_T, void* stream);
 
 /* Tuning knobs of one scene's render path (no reference counterpart; defaults need no call).
  *  RTGS_OPT_RENDER_MODE      0 (default): k_tile_lists (traversal, one candidate list per 4x8-pixel tile) +

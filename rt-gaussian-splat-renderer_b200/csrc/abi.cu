@@ -498,10 +498,10 @@ int rtgs_scene_set_gaussians_device(rtgs_scene* s, const float* pos, const float
     return RTGS_OK;
 }
 
-int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
-                         int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT, float* grad_pos,
-                         float* grad_rot, float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
-                         float* replay_rgb, float* replay_T, void* stream) {
+static int render_backward(const char* name, rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0,
+                           int32_t w, int32_t h, int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                           float* const grads[6], float* const cam_grads[3], float* replay_rgb, float* replay_T,
+                           void* stream) {
     RTGS_CHECK_ARG(s != nullptr);
     TRY(check_camera(cam));
     RTGS_CHECK_ARG(dL_drgb != nullptr);
@@ -509,13 +509,33 @@ int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int3
     RTGS_CHECK_ARG(depth >= 1 && depth <= RTGS_MAX_DEPTH);
     RTGS_CHECK_ARG(t_cut >= 0.0f && t_cut < 1.0f);
     if (!s->built) {
-        rtgs_set_error("rtgs_render_backward: call rtgs_scene_build_bvh first");
+        rtgs_set_error("%s: call rtgs_scene_build_bvh first", name);
         return RTGS_ERR_STATE;
     }
     DeviceGuard g(s->device);
+    return rtgs_launch_render_backward(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads, cam_grads,
+                                       replay_rgb, replay_T, (cudaStream_t)stream);
+}
+
+int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                         int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT, float* grad_pos,
+                         float* grad_rot, float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
+                         float* replay_rgb, float* replay_T, void* stream) {
     float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
-    return rtgs_launch_render_backward(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads, replay_rgb,
-                                       replay_T, (cudaStream_t)stream);
+    float* const cam_grads[3] = {nullptr, nullptr, nullptr};
+    return render_backward("rtgs_render_backward", s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads,
+                           cam_grads, replay_rgb, replay_T, stream);
+}
+
+int rtgs_render_backward_camera(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                                int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                                float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                                float* grad_opacity, float* grad_sh, float* grad_cam_pos, float* grad_cam_rot,
+                                float* grad_cam_focal, float* replay_rgb, float* replay_T, void* stream) {
+    float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
+    float* const cam_grads[3] = {grad_cam_pos, grad_cam_rot, grad_cam_focal};
+    return render_backward("rtgs_render_backward_camera", s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads,
+                           cam_grads, replay_rgb, replay_T, stream);
 }
 
 int rtgs_scene_set_option(rtgs_scene* s, int32_t option, int64_t value) {

@@ -12,12 +12,20 @@
 //   3. back to front, with B_n = dL/dT and B_k = alpha_k (c_k.g) + (1 - alpha_k) B_{k+1} (no division):
 //        dL/dalpha_k = T_k (c_k.g - B_{k+1}),  dL/dc_k = T_k alpha_k g,
 //        alpha = opacity exp(-q):  dL/dopacity = exp(-q) dL/dalpha,  dL/dq = -alpha dL/dalpha,
-//        c = colour + sum_j Y_j sh_j (no gradient into the direction),
+//        c = colour + sum_j Y_j sh_j (the direction's gradient only with CAM, below),
 //        u = W (o - p), v = W d, sigma = u.v / |v|^2, e = u - sigma v = W (x - p), x = o - sigma d:
 //        dq/dp = -2 W^T e,  dq/dW = 2 e (x - p)^T,
 //        W = S^-1 Rm^T / c^2 (local_frame as written, Rm = quat_to_mat(q), c = |q|^2): differentiated through
 //        s, Rm(q) and c, so stored quaternions of any norm get their exact gradient.
 //      Gradients are scattered with float32 atomics to the ORIGINAL index (raw[s*3+2].z).
+// k_render_backward<true> also differentiates with respect to the camera (rtgs_render_backward_camera).  The camera
+// enters only through the ray: o, d = Rm(q_cam) dc, dc = n / |n|, n = (px, py, -1), px = (i + 0.5 - W/2) / fx.
+// Per layer dq/do = 2 W^T e, dq/dd = -2 sigma W^T e; the SH colour adds dL/dY_j = sum_k T_k alpha_k (sh_kj . g),
+// summed over the layers and taken through dY/d(d/|d|) once per pixel.  Per pixel, from dL/dd:
+// dL/dRm = dL/dd dc^T, dL/dn = (I - dc dc^T) Rm^T dL/dd / |n|, dL/dfx = -dL/dpx px / fx (fy alike).  The 14 per-pixel
+// values (o 3, Rm 9, fx, fy) are summed in float64 in a fixed order: warp shuffles, the CTA's warps in shared
+// memory, one partial record per CTA, and k_camera_grad_finalize (one CTA) over the partials, which also takes
+// dL/dRm to dL/dq_cam and adds the float32-rounded results to the caller's buffers.
 #pragma once
 #include "render_common.cuh"
 
@@ -25,6 +33,8 @@ namespace rtgs_dev {
 namespace backward {
 
 constexpr int BWD_WARPS = 4;   // warps (tiles) per CTA
+constexpr int CAM_TERMS = 14;  // per-pixel camera gradient: dL/do (3), dL/dRm (9, row-major), dL/dfx, dL/dfy
+constexpr int FIN_THREADS = 256;
 
 struct BackwardParams {
     const float4* __restrict__ nodes;
@@ -48,6 +58,7 @@ struct BackwardParams {
     float* g_sh;                 // (n,15,3)
     float* replay_rgb;           // (w,h,3) or null
     float* replay_T;             // (w,h) or null
+    double* cam_part;            // k_render_backward<true>: (CAM_TERMS, gridDim.x) per-CTA partial sums
 };
 
 // sh_basis (render_common.cuh) in float64: gaussian.py:149-163, incl. the `5z^2 - 3z` term at :160 as coded
@@ -72,12 +83,45 @@ __device__ __forceinline__ void sh_basis_d(double x, double y, double z, double 
     Y[14] = 0.25 * c3 * x * (xx - 3.0 * yy);
 }
 
+// g = sum_j gY[j] dY_j/d(x, y, z): the derivative of sh_basis_d at (x, y, z), contracted with gY
+__device__ __forceinline__ void sh_basis_vjp_d(double x, double y, double z, const double (&gY)[15], double (&g)[3]) {
+    const double c0 = 0.9772050238058398, c1 = 2.1850968611841584, c2 = 1.2615662610100802,
+                 c3 = 2.360174359706574, c4 = 5.781222885281108, c5 = 1.828183197857863, c6 = 1.4927053303604616;
+    const double xx = x * x, yy = y * y, zz = z * z;
+    g[0] = 0.5 * c0 * gY[2] + 0.5 * c1 * (y * gY[3] + z * gY[6] + x * gY[7]) + 1.5 * c3 * x * y * gY[8] +
+           0.5 * c4 * y * z * gY[9] + 0.25 * c5 * (5.0 * zz - 1.0) * gY[12] + 0.5 * c4 * x * z * gY[13] +
+           0.75 * c3 * (xx - yy) * gY[14];
+    g[1] = 0.5 * c0 * gY[0] + 0.5 * c1 * (x * gY[3] + z * gY[4] - y * gY[7]) + 0.75 * c3 * (xx - yy) * gY[8] +
+           0.5 * c4 * x * z * gY[9] + 0.25 * c5 * (5.0 * zz - 1.0) * gY[10] - 0.5 * c4 * y * z * gY[13] -
+           1.5 * c3 * x * y * gY[14];
+    g[2] = 0.5 * c0 * gY[1] + 0.5 * c1 * (y * gY[4] + x * gY[6]) + 1.5 * c2 * z * gY[5] + 0.5 * c4 * x * y * gY[9] +
+           2.5 * c5 * y * z * gY[10] + 0.25 * c6 * (10.0 * z - 3.0) * gY[11] + 2.5 * c5 * x * z * gY[12] +
+           0.25 * c4 * (xx - yy) * gY[13];
+}
+
+// The part of dL/dq that goes through Rm = quat_to_mat(q) = (w^2 - |u|^2) I + 2 u u^T + 2 w [u]x (quat_rot on the
+// basis vectors), given M = dL/dRm.  Shared by the Gaussian rotations and the camera rotation.
+__device__ __forceinline__ void rot_mat_vjp(const double (&q)[4], const double (&M)[3][3], double (&g)[4]) {
+    const double ux = q[0], uy = q[1], uz = q[2], w = q[3];
+    const double tr = M[0][0] + M[1][1] + M[2][2];
+    const double Kx = M[2][1] - M[1][2], Ky = M[0][2] - M[2][0], Kz = M[1][0] - M[0][1];
+    const double u3[3] = {ux, uy, uz}, K3[3] = {Kx, Ky, Kz};
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        const double Mu = M[i][0] * ux + M[i][1] * uy + M[i][2] * uz;
+        const double MTu = M[0][i] * ux + M[1][i] * uy + M[2][i] * uz;
+        g[i] = -2.0 * u3[i] * tr + 2.0 * (Mu + MTu) + 2.0 * w * K3[i];
+    }
+    g[3] = 2.0 * w * tr + 2.0 * (ux * Kx + uy * Ky + uz * Kz);
+}
+
 // One layer of one ray, float64 from the raw parameters: everything phases 2 and 3 need.
 struct Layer {
     double p[3], q[4], sc[3];
     double Wm[3][3];
     double e[3];      // W (x - p)
     double xp[3];     // x - p, x = o - sigma d: the max-response point
+    double sig;       // sigma = u.v / |v|^2
     double qm;        // |e|^2 = min Mahalanobis^2 along the ray
     double alpha;
     double ex;        // exp(-q)
@@ -106,6 +150,7 @@ __device__ __forceinline__ void eval_layer(const BackwardParams& P, int s, const
     L.qm = d3dot(m, m) / A;   // as exact_intersect computes it
 #pragma unroll
     for (int k = 0; k < 3; ++k) L.e[k] = u[k] - sig * v[k];
+    L.sig = sig;
     L.xp[0] = op[0] - sig * d.x;
     L.xp[1] = op[1] - sig * d.y;
     L.xp[2] = op[2] - sig * d.z;
@@ -136,14 +181,28 @@ __device__ __forceinline__ void eval_colour_d(const BackwardParams& P, int s, co
     }
 }
 
+// gY[j] += wgt * (sh_j . gr) for the SH coefficients of sorted position s (the colour's dependence on Y)
+__device__ __forceinline__ void sh_dot_d(const BackwardParams& P, int s, double wgt, const double (&gr)[3],
+                                         double (&gY)[15]) {
+    const float4* sp = P.shp + (int64_t)s * 12;
+    float v[48];
+#pragma unroll
+    for (int f = 0; f < 12; ++f) {
+        const float4 x = __ldg(sp + f);
+        v[4 * f] = x.x; v[4 * f + 1] = x.y; v[4 * f + 2] = x.z; v[4 * f + 3] = x.w;
+    }
+#pragma unroll
+    for (int j = 0; j < 15; ++j) gY[j] += wgt * (v[3 * j + 0] * gr[0] + v[3 * j + 1] * gr[1] + v[3 * j + 2] * gr[2]);
+}
+
 __device__ __forceinline__ void red_add(float* base, int64_t i, double v) {
     if (base != nullptr) atomicAdd(base + i, (float)v);
 }
 
-__global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid_constant__ BackwardParams P) {
-    const int lane = threadIdx.x & 31;
-    const int tile = blockIdx.x * BWD_WARPS + (threadIdx.x >> 5);
-    if (tile >= P.ntiles) return;
+// One pixel of k_render_backward; a pixel that contributes nothing returns early.  With CAM, its camera terms are
+// written to cam_g[CAM_TERMS] (left untouched, i.e. zero, on an early return).
+template <bool CAM>
+__device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile, int lane, double* cam_g) {
     const int ti = tile / P.tiles_j, tj = tile - ti * P.tiles_j;
     const int li = ti * TILE_I + lane / TILE_J, lj = tj * TILE_J + lane % TILE_J;   // region-relative pixel
     if (li >= P.w || lj >= P.h) return;
@@ -242,6 +301,12 @@ __global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid
     const double gr[3] = {P.dL_drgb[pix * 3 + 0], P.dL_drgb[pix * 3 + 1], P.dL_drgb[pix * 3 + 2]};
     double B = P.dL_dT != nullptr ? (double)P.dL_dT[pix] : 0.0;
     if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
+    double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};   // CAM: dL/do, dL/dd (geometry)
+    double gY[15];                                             // CAM: dL/dY_j
+    if constexpr (CAM) {
+#pragma unroll
+        for (int j = 0; j < 15; ++j) gY[j] = 0.0;
+    }
     for (int k = L - 1; k >= 0; --k) {
         const int s = ks[k];
         Layer ly;
@@ -278,6 +343,16 @@ __global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid
                 red_add(P.g_pos, g * 3 + j,
                         -2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]));
         }
+        if constexpr (CAM) {
+            // dq/do = 2 W^T e, dq/dd = -2 sigma W^T e
+#pragma unroll
+            for (int j = 0; j < 3; ++j) {
+                const double wte = 2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]);
+                gO[j] += wte;
+                gD[j] -= ly.sig * wte;
+            }
+            if (P.has_sh) sh_dot_d(P, s, wgt, gr, gY);
+        }
         if (P.g_scale == nullptr && P.g_rot == nullptr) continue;
         // G = dL/dW = 2 dq e (x - p)^T; W_kj = Rm[j][k] f_k with f_k = 1 / (s_k c^2)
         double GW[3];   // sum_j G_kj W_kj per row k
@@ -299,21 +374,117 @@ __global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid
             for (int k2 = 0; k2 < 3; ++k2) red_add(P.g_scale, g * 3 + k2, -GW[k2] / ly.sc[k2]);
         }
         if (P.g_rot != nullptr) {
-            // Rm = (w^2 - |u|^2) I + 2 u u^T + 2 w [u]x  (quat_rot on the basis vectors), c = |q|^2
-            const double ux = ly.q[0], uy = ly.q[1], uz = ly.q[2], w = ly.q[3];
-            const double tr = M[0][0] + M[1][1] + M[2][2];
-            const double Kx = M[2][1] - M[1][2], Ky = M[0][2] - M[2][0], Kz = M[1][0] - M[0][1];
-            const double u3[3] = {ux, uy, uz}, K3[3] = {Kx, Ky, Kz};
+            // through Rm(q) (rot_mat_vjp) and through c = |q|^2
+            double gq[4];
+            rot_mat_vjp(ly.q, M, gq);
             const double dLdc = -2.0 / c2 * (GW[0] + GW[1] + GW[2]);
 #pragma unroll
-            for (int i = 0; i < 3; ++i) {
-                const double Mu = M[i][0] * ux + M[i][1] * uy + M[i][2] * uz;
-                const double MTu = M[0][i] * ux + M[1][i] * uy + M[2][i] * uz;
-                red_add(P.g_rot, g * 4 + i,
-                        -2.0 * u3[i] * tr + 2.0 * (Mu + MTu) + 2.0 * w * K3[i] + 2.0 * u3[i] * dLdc);
-            }
-            red_add(P.g_rot, g * 4 + 3, 2.0 * w * tr + 2.0 * (ux * Kx + uy * Ky + uz * Kz) + 2.0 * w * dLdc);
+            for (int i = 0; i < 4; ++i) red_add(P.g_rot, g * 4 + i, gq[i] + 2.0 * ly.q[i] * dLdc);
         }
+    }
+    if constexpr (CAM) {
+        // the SH direction d / |d|: dL/dd += (I - dn dn^T) dL/ddn / |d|
+        if (P.has_sh) {
+            const double il = 1.0 / sqrt(d.x * d.x + d.y * d.y + d.z * d.z);
+            const double dn[3] = {d.x * il, d.y * il, d.z * il};
+            double gn[3];
+            sh_basis_vjp_d(dn[0], dn[1], dn[2], gY, gn);
+            const double pr = dn[0] * gn[0] + dn[1] * gn[1] + dn[2] * gn[2];
+#pragma unroll
+            for (int j = 0; j < 3; ++j) gD[j] += (gn[j] - dn[j] * pr) * il;
+        }
+        // d = Rm dc, dc = n / |n| as cam_dir computes them
+        const double px = ((double)pi + 0.5 - 0.5 * (double)cam.W) * cam.ifx;
+        const double py = ((double)pj + 0.5 - 0.5 * (double)cam.H) * cam.ify;
+        const double inv = rsqrt(px * px + py * py + 1.0);
+        const double dc[3] = {px * inv, py * inv, -inv};
+        double gdc[3];   // Rm^T dL/dd
+#pragma unroll
+        for (int j = 0; j < 3; ++j) gdc[j] = cam.R[j] * gD[0] + cam.R[3 + j] * gD[1] + cam.R[6 + j] * gD[2];
+        const double pr = dc[0] * gdc[0] + dc[1] * gdc[1] + dc[2] * gdc[2];
+        cam_g[0] = gO[0]; cam_g[1] = gO[1]; cam_g[2] = gO[2];
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) cam_g[3 + r * 3 + k] = gD[r] * dc[k];
+        cam_g[12] = -(gdc[0] - dc[0] * pr) * inv * px * cam.ifx;
+        cam_g[13] = -(gdc[1] - dc[1] * pr) * inv * py * cam.ify;
+    }
+}
+
+// The CTA's camera terms, summed in a fixed order: lanes by shuffles, then the warps in order.  Every thread of the
+// CTA must arrive.
+__device__ __forceinline__ void cam_block_reduce(const BackwardParams& P, double (&cg)[CAM_TERMS]) {
+    __shared__ double red[BWD_WARPS][CAM_TERMS];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int i = 0; i < CAM_TERMS; ++i) {
+        double v = cg[i];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
+        if (lane == 0) red[warp][i] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < CAM_TERMS) {
+        double v = red[0][threadIdx.x];
+#pragma unroll
+        for (int w = 1; w < BWD_WARPS; ++w) v += red[w][threadIdx.x];
+        P.cam_part[(int64_t)threadIdx.x * gridDim.x + blockIdx.x] = v;
+    }
+}
+
+// CAM = false: the Gaussian gradients.  CAM = true: also the camera's, as per-CTA partials in P.cam_part (finished
+// by k_camera_grad_finalize).
+template <bool CAM>
+__global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid_constant__ BackwardParams P) {
+    const int lane = threadIdx.x & 31;
+    const int tile = blockIdx.x * BWD_WARPS + (threadIdx.x >> 5);
+    if constexpr (!CAM) {
+        if (tile >= P.ntiles) return;
+        backward_pixel<false>(P, tile, lane, nullptr);
+    } else {
+        // absent pixels and tiles contribute zeros: every lane reaches the shuffles and the barrier
+        double cg[CAM_TERMS];
+#pragma unroll
+        for (int i = 0; i < CAM_TERMS; ++i) cg[i] = 0.0;
+        if (tile < P.ntiles) backward_pixel<true>(P, tile, lane, cg);
+        cam_block_reduce(P, cg);
+    }
+}
+
+// One CTA: sums the (CAM_TERMS, nparts) partials in a fixed order, takes dL/dRm to dL/dq_cam, and adds the three
+// float32-rounded results to the caller's buffers (any may be null).
+__global__ void __launch_bounds__(FIN_THREADS) k_camera_grad_finalize(const double* __restrict__ part, int nparts,
+                                                                      const __grid_constant__ CamD cam, float* g_pos,
+                                                                      float* g_rot, float* g_focal) {
+    __shared__ double red[CAM_TERMS][FIN_THREADS];
+    const int t = threadIdx.x;
+    for (int i = 0; i < CAM_TERMS; ++i) {
+        double v = 0.0;
+        for (int b = t; b < nparts; b += FIN_THREADS) v += part[(int64_t)i * nparts + b];
+        red[i][t] = v;
+    }
+    __syncthreads();
+    for (int s = FIN_THREADS / 2; s > 0; s >>= 1) {
+        if (t < s)
+            for (int i = 0; i < CAM_TERMS; ++i) red[i][t] += red[i][t + s];
+        __syncthreads();
+    }
+    if (t != 0) return;
+    if (g_pos != nullptr)
+        for (int j = 0; j < 3; ++j) g_pos[j] += (float)red[j][0];
+    if (g_rot != nullptr) {
+        // the camera uses Rm(q) unscaled: no |q| factor besides the one inside Rm
+        const double q[4] = {cam.q[0], cam.q[1], cam.q[2], cam.q[3]};
+        double M[3][3], gq[4];
+        for (int r = 0; r < 3; ++r)
+            for (int k = 0; k < 3; ++k) M[r][k] = red[3 + r * 3 + k][0];
+        rot_mat_vjp(q, M, gq);
+        for (int j = 0; j < 4; ++j) g_rot[j] += (float)gq[j];
+    }
+    if (g_focal != nullptr) {
+        g_focal[0] += (float)red[12][0];
+        g_focal[1] += (float)red[13][0];
     }
 }
 

@@ -21,7 +21,8 @@
 //                  the traversal's shared-memory list (heavy_lists.cuh), between k_tile_lists and k_shade_tiles
 //   k_render       fused.cuh (mode 1, depth > 16, fallback tiles)
 //   k_generate_rays, k_trace_closest, k_activate_ply   API companions (Camera.generate_ray_field, Scene.hit, PLY ingest)
-//   k_render_backward  gradient of the render with respect to the Gaussian parameters (backward.cuh)
+//   k_render_backward  gradient of the render with respect to the Gaussian parameters and, as
+//                      k_render_backward<true> + k_camera_grad_finalize, the camera (backward.cuh)
 #include <stdlib.h>
 
 #include "backward.cuh"
@@ -924,7 +925,7 @@ int rtgs_launch_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, i
 
 int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h, int depth,
                                 float t_cut, const float* dL_drgb, const float* dL_dT, float* const grads[6],
-                                float* replay_rgb, float* replay_T, cudaStream_t stream) {
+                                float* const cam_grads[3], float* replay_rgb, float* replay_T, cudaStream_t stream) {
     backward::BackwardParams P;
     P.nodes = s->nodes;
     P.geo = s->geo;
@@ -943,9 +944,25 @@ int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, i
     P.g_color = grads[3]; P.g_opacity = grads[4]; P.g_sh = s->has_sh ? grads[5] : nullptr;
     P.replay_rgb = replay_rgb;
     P.replay_T = replay_T;
+    P.cam_part = nullptr;
     const int blocks = (P.ntiles + backward::BWD_WARPS - 1) / backward::BWD_WARPS;
-    backward::k_render_backward<<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
-    CUDA_TRY(cudaGetLastError());
+    if (cam_grads[0] == nullptr && cam_grads[1] == nullptr && cam_grads[2] == nullptr) {
+        backward::k_render_backward<false><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+        CUDA_TRY(cudaGetLastError());
+        return RTGS_OK;
+    }
+    // per-CTA partials of the camera gradient, stream-ordered: no scene scratch, safe for calls on several streams
+    CUDA_TRY(cudaMallocAsync((void**)&P.cam_part, sizeof(double) * backward::CAM_TERMS * blocks, stream));
+    backward::k_render_backward<true><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) {
+        backward::k_camera_grad_finalize<<<1, backward::FIN_THREADS, 0, stream>>>(P.cam_part, blocks, P.cam, cam_grads[0],
+                                                                                   cam_grads[1], cam_grads[2]);
+        e = cudaGetLastError();
+    }
+    const cudaError_t ef = cudaFreeAsync(P.cam_part, stream);
+    CUDA_TRY(e);
+    CUDA_TRY(ef);
     return RTGS_OK;
 }
 

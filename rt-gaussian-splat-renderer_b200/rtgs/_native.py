@@ -64,6 +64,9 @@ SIGNATURES = {
     "rtgs_render_backward": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                        C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                        _vp]),
+    "rtgs_render_backward_camera": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32,
+                                              C.c_int32, C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                              _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rtgs_scene_set_option": (C.c_int, [_vp, C.c_int32, C.c_int64]),
     "rtgs_scene_get_option": (C.c_int, [_vp, C.c_int32, C.POINTER(C.c_int64)]),
     "rtgs_scene_set_frame_sync": (C.c_int, [_vp, _vp, _vp, C.c_uint32]),

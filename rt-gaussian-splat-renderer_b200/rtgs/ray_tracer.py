@@ -215,14 +215,17 @@ class RayTracer:
             self.last_stats = stats.as_dict()
         return out
 
-    def render_backward(self, dL_drgb, dL_dT=None, depth: int = 16, tile=None, grads=None, replay: bool = False):
+    def render_backward(self, dL_drgb, dL_dT=None, depth: int = 16, tile=None, grads=None, replay: bool = False,
+                        camera: bool = False):
         """Gradient of ``render_device(depth, tile)`` (with ``t_cut``) with respect to the stored Gaussian parameters,
         the layer list of every pixel held fixed (rtgs_render_backward), on the current stream.
 
         dL_drgb (w,h,3) and dL_dT (w,h) are CUDA float32 tensors of the region.  Returns a dict of (n,...) float32
         gradients ``pos rot scale color opacity`` and ``sh`` (scenes with SH): ``grads`` may pass tensors of these
         names to accumulate into (missing ones are zero-initialised).  With ``replay=True`` the dict also holds
-        ``rgb`` / ``T``, the image the backward recomputed."""
+        ``rgb`` / ``T``, the image the backward recomputed.  With ``camera=True`` it also holds the gradient with
+        respect to the camera (rtgs_render_backward_camera): ``camera_position`` (3,), ``camera_rotation`` (4,, the
+        x,y,z,w quaternion as stored) and ``camera_focal`` (2,), which ``grads`` may pass in the same way."""
         import torch
         W, H = self.buf_size.x, self.buf_size.y
         x0, y0, w, h = (0, 0, W, H) if tile is None else tile
@@ -238,6 +241,8 @@ class RayTracer:
         shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
         if self.scene.has_sh:
             shapes["sh"] = (n, 15, 3)
+        if camera:
+            shapes.update(camera_position=(3,), camera_rotation=(4,), camera_focal=(2,))
         out = dict(grads or {})
         for name, shape in shapes.items():
             if name not in out:
@@ -250,10 +255,16 @@ class RayTracer:
             out["T"] = torch.empty((w, h), dtype=torch.float32, device=self._dev)
         cam = self.camera.native()
         ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
-        _native.check(_native.load().rtgs_render_backward(
-            self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, dL_drgb.data_ptr(),
-            None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
-            ptr("opacity"), ptr("sh"), ptr("rgb"), ptr("T"), torch.cuda.current_stream(self._dev).cuda_stream))
+        head = (self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, dL_drgb.data_ptr(),
+                None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
+                ptr("opacity"), ptr("sh"))
+        tail = (ptr("rgb"), ptr("T"), torch.cuda.current_stream(self._dev).cuda_stream)
+        lib = _native.load()
+        if camera:
+            _native.check(lib.rtgs_render_backward_camera(
+                *head, ptr("camera_position"), ptr("camera_rotation"), ptr("camera_focal"), *tail))
+        else:
+            _native.check(lib.rtgs_render_backward(*head, *tail))
         return out
 
     def _render_into(self, depth, accumulate):

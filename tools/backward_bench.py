@@ -1,6 +1,8 @@
 #!/usr/bin/env python
-"""Time the differentiable render path on one GPU: forward (rtgs_render), backward (rtgs_render_backward),
-Scene.set_gaussians + LBVH rebuild, and one whole rtgs.autograd step, on a synthetic bench configuration.
+"""Time the differentiable render path on one GPU: forward (rtgs_render), backward (rtgs_render_backward), the
+backward with the camera gradient (rtgs_render_backward_camera, with every Gaussian gradient and camera only),
+Scene.set_gaussians + LBVH rebuild, one whole rtgs.autograd step and one rtgs.autograd.render_camera step, on a
+synthetic bench configuration.
 
     python tools/backward_bench.py [--config 1m_deg3_1080p] [--depth 16] [--t-cut 1e-4] [--iters 20] [--warmup 3]
 
@@ -110,6 +112,12 @@ def main():
     bwd_no_atomics = timed(lambda: _native.check(lib.rtgs_render_backward(
         scene.handle, ncam, 0, 0, W, H, depth, args.t_cut, d_rgb.data_ptr(), d_T.data_ptr(),
         None, None, None, None, None, None, None, None, stream())))
+    cam_grads = {k: torch.zeros(n, device=dev) for k, n in (("camera_position", 3), ("camera_rotation", 4),
+                                                              ("camera_focal", 2))}
+    bwd_cam = timed(lambda: rt.render_backward(d_rgb, d_T, depth=depth, grads={**grads, **cam_grads}, camera=True))
+    bwd_cam_only = timed(lambda: _native.check(lib.rtgs_render_backward_camera(
+        scene.handle, ncam, 0, 0, W, H, depth, args.t_cut, d_rgb.data_ptr(), d_T.data_ptr(),
+        None, None, None, None, None, None, *(cam_grads[k].data_ptr() for k in cam_grads), None, None, stream())))
     upd_med, upd_min = host_timed(lambda: scene.set_gaussians(*(params[k] for k in params)), iters=max(5, args.iters // 2))
     build_ms = scene.build_ms
 
@@ -121,6 +129,14 @@ def main():
         ((rgb * d_rgb).sum() + (T * d_T).sum()).backward()
 
     step_med, step_min = host_timed(step, iters=max(5, args.iters // 2))
+    cpos = torch.tensor(np.asarray(cam.position, np.float32), device=dev, requires_grad=True)
+    crot = torch.tensor(np.asarray(cam.rotation, np.float32), device=dev, requires_grad=True)
+
+    def camera_step():
+        rgb, T = A.render_camera(scene, cam, cpos, crot, depth=depth, t_cut=args.t_cut)
+        ((rgb * d_rgb).sum() + (T * d_T).sum()).backward()
+
+    cam_step_med, cam_step_min = host_timed(camera_step, iters=max(5, args.iters // 2))
     layers = None
     try:
         rt.render_device(depth, collect_stats=True)
@@ -137,9 +153,12 @@ def main():
             "plus back-to-front pass without atomics": round(bwd_no_atomics, 3),
             "plus atomics (full)": round(bwd, 3),
         },
+        "backward_camera_ms": {"with every Gaussian gradient": round(bwd_cam, 3),
+                               "camera only (Gaussian pointers NULL)": round(bwd_cam_only, 3)},
         "set_gaussians_and_rebuild_ms": {"median": round(upd_med, 3), "min": round(upd_min, 3),
                                          "build_device_ms": round(build_ms, 3)},
         "autograd_step_ms": {"median": round(step_med, 3), "min": round(step_min, 3)},
+        "render_camera_step_ms": {"median": round(cam_step_med, 3), "min": round(cam_step_min, 3)},
         "card": card_info(torch),
     }
     print(json.dumps(res))
