@@ -354,6 +354,30 @@ int rtgs_generate_rays(const rtgs_camera* cam, int device, float* rays, void* st
 int rtgs_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays,
                        int32_t* idx, float* t12, void* stream);
 
+/* Render arbitrary rays: non-pinhole cameras, ray batches drawn from many views, secondary rays.  rays: device
+ * (nrays,8) float32 as above, 16-byte aligned: origin o, direction d (used as given, not normalised; the SH colour
+ * uses d / |d|), start, end.  A ray's layer list is the Gaussians whose float64 exact intersection has
+ * start < t1 < end, in ascending t1 (exact ties by sorted position), truncated to `depth`, composited front to back
+ * while the incoming float32 T >= t_cut.  start = 0, end = +inf is the pixel rule of rtgs_render, so a ray of
+ * rtgs_generate_rays gives its pixel's layer list (up to the float32 rounding of d).  A ray with a non-finite o or d
+ * component, d = 0 or !(start < end) composites nothing: rgb 0, T 1.
+ * out_rgb: device (nrays,3); out_T: device (nrays) or NULL.  Stream-ordered on `stream`, no scene scratch.
+ * nrays = 0 does nothing. */
+int rtgs_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                     float* out_rgb, float* out_T, void* stream);
+
+/* Backward of rtgs_render_rays with each ray's layer list and t_cut stop held fixed (the definition of
+ * rtgs_render_backward).  dL_drgb (nrays,3) and dL_dT (nrays, or NULL) are device buffers.  The Gaussian gradients
+ * are ACCUMULATED as in rtgs_render_backward (any may be NULL).  grad_rays (nrays,8) or NULL is ACCUMULATED too:
+ * columns 0-2 dL/do, 3-5 dL/dd, 6-7 untouched (start, end and depth have no gradient); each ray's thread adds its own
+ * values, so two identical calls give bit-identical ray gradients.  Degenerate rays get no gradient.  replay_rgb /
+ * replay_T (optional) receive the image recomputed, bit-identical to rtgs_render_rays. */
+int rtgs_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                              const float* dL_drgb, const float* dL_dT,
+                              float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                              float* grad_opacity, float* grad_sh, float* grad_rays,
+                              float* replay_rgb, float* replay_T, void* stream);
+
 int rtgs_scene_destroy(rtgs_scene* s);
 
 #ifdef __cplusplus

@@ -217,6 +217,20 @@ int check_camera(const rtgs_camera* cam) {
     return RTGS_OK;
 }
 
+bool aligned(const void* p, uintptr_t bytes) { return ((uintptr_t)p & (bytes - 1)) == 0; }
+
+// The checks both ray entry points share: everything but the state of the scene, before any CUDA call.
+int check_rays(const rtgs_scene* s, int64_t nrays, const float* rays, const float* rgb, int32_t depth,
+                      float t_cut) {
+    RTGS_CHECK_ARG(s != nullptr);
+    RTGS_CHECK_ARG(nrays >= 0);
+    RTGS_CHECK_ARG(nrays == 0 || (rays != nullptr && aligned(rays, 16)));
+    RTGS_CHECK_ARG(nrays == 0 || (rgb != nullptr && aligned(rgb, 4)));
+    RTGS_CHECK_ARG(depth >= 1 && depth <= RTGS_MAX_DEPTH);
+    RTGS_CHECK_ARG(t_cut >= 0.0f && t_cut < 1.0f);
+    return RTGS_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1111,6 +1125,37 @@ int rtgs_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, int32_t*
     }
     DeviceGuard g(s->device);
     return rtgs_launch_trace_closest(s, nrays, rays, idx, t12, (cudaStream_t)stream);
+}
+
+int rtgs_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut, float* out_rgb,
+                     float* out_T, void* stream) {
+    TRY(check_rays(s, nrays, rays, out_rgb, depth, t_cut));
+    RTGS_CHECK_ARG(aligned(out_T, 4));
+    if (!s->built) {
+        rtgs_set_error("rtgs_render_rays: call rtgs_scene_build_bvh first");
+        return RTGS_ERR_STATE;
+    }
+    if (nrays == 0) return RTGS_OK;
+    DeviceGuard g(s->device);
+    return rtgs_launch_render_rays(s, nrays, rays, depth, t_cut, out_rgb, out_T, (cudaStream_t)stream);
+}
+
+int rtgs_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                              const float* dL_drgb, const float* dL_dT, float* grad_pos, float* grad_rot,
+                              float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
+                              float* grad_rays, float* replay_rgb, float* replay_T, void* stream) {
+    TRY(check_rays(s, nrays, rays, dL_drgb, depth, t_cut));
+    float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
+    for (const float* p : grads) RTGS_CHECK_ARG(aligned(p, 4));
+    RTGS_CHECK_ARG(aligned(dL_dT, 4) && aligned(grad_rays, 4) && aligned(replay_rgb, 4) && aligned(replay_T, 4));
+    if (!s->built) {
+        rtgs_set_error("rtgs_render_rays_backward: call rtgs_scene_build_bvh first");
+        return RTGS_ERR_STATE;
+    }
+    if (nrays == 0) return RTGS_OK;
+    DeviceGuard g(s->device);
+    return rtgs_launch_render_rays_backward(s, nrays, rays, depth, t_cut, dL_drgb, dL_dT, grads, grad_rays,
+                                            replay_rgb, replay_T, (cudaStream_t)stream);
 }
 
 int rtgs_scene_destroy(rtgs_scene* s) {

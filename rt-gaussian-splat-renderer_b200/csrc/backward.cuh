@@ -26,6 +26,15 @@
 // values (o 3, Rm 9, fx, fy) are summed in float64 in a fixed order: warp shuffles, the CTA's warps in shared
 // memory, one partial record per CTA, and k_camera_grad_finalize (one CTA) over the partials, which also takes
 // dL/dRm to dL/dq_cam and adds the float32-rounded results to the caller's buffers.
+//
+// The three phases take the ray (o, d) as a parameter (walk_layers, replay_layers, back_to_front), so they also serve
+// arbitrary rays (rtgs_render_rays / _backward): k_render_rays runs phases 1-2, k_render_rays_backward 1-3, one thread
+// per ray.  A ray is the (n,8) float32 record of rtgs_generate_rays: o, d (used as given, not normalised; the SH
+// colour uses d / |d|), start, end.  Its layer list is the Gaussians with start < t1 < end (float64 exact_intersect),
+// ascending t1, ties by sorted position, truncated to `depth`, composited under the t_cut rule; start = 0, end = +inf
+// is the pixel rule.  Its gradient is dL/do = sum_k 2 dq_k W^T e, dL/dd = sum_k -2 sigma dq_k W^T e plus the SH term
+// (I - dn dn^T)(dY/ddn)^T dL/dY / |d|: the gO / gD of the CAM path.  A ray with a non-finite o or d component, d = 0
+// or !(start < end) composites nothing (rgb 0, T 1) and gets no gradient.
 #pragma once
 #include "render_common.cuh"
 
@@ -59,6 +68,10 @@ struct BackwardParams {
     float* replay_rgb;           // (w,h,3) or null
     float* replay_T;             // (w,h) or null
     double* cam_part;            // k_render_backward<true>: (CAM_TERMS, gridDim.x) per-CTA partial sums
+    // the ray kernels: dL_drgb, dL_dT, replay_rgb and replay_T are then indexed by ray
+    const float* rays;           // (nrays, 8): o xyz, d xyz, start, end; 16-byte aligned
+    int64_t nrays;
+    float* g_rays;               // k_render_rays_backward<true>: (nrays, 8), columns 0-5 accumulated
 };
 
 // sh_basis (render_common.cuh) in float64: gaussian.py:149-163, incl. the `5z^2 - 3z` term at :160 as coded
@@ -199,75 +212,71 @@ __device__ __forceinline__ void red_add(float* base, int64_t i, double v) {
     if (base != nullptr) atomicAdd(base + i, (float)v);
 }
 
-// One pixel of k_render_backward; a pixel that contributes nothing returns early.  With CAM, its camera terms are
-// written to cam_g[CAM_TERMS] (left untouched, i.e. zero, on an early return).
-template <bool CAM>
-__device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile, int lane, double* cam_g) {
-    const int ti = tile / P.tiles_j, tj = tile - ti * P.tiles_j;
-    const int li = ti * TILE_I + lane / TILE_J, lj = tj * TILE_J + lane % TILE_J;   // region-relative pixel
-    if (li >= P.w || lj >= P.h) return;
-    const int pi = P.x0 + li, pj = P.y0 + lj;
-    const int64_t pix = (int64_t)li * P.h + lj;
-    const CamD& cam = P.cam;
-    const double o[3] = {cam.o[0], cam.o[1], cam.o[2]};
-    const d3 d = cam_dir(cam, (double)pi + 0.5, (double)pj + 0.5);
-    const int K = P.depth;
+// ---- the three phases of one ray (o, d): shared by the pixel kernels and the ray kernels -----------------------
 
-    // ---- phase 1: the K nearest hits (t1 > 0), ascending float64 t1, ties by sorted position ----------------
-    double kt[RTGS_MAX_DEPTH];
-    int ks[RTGS_MAX_DEPTH];
+// Phase 1: the K nearest hits, ascending float64 t1, ties by sorted position, into kt / ks; returns their count.
+// INTERVAL = false is the pixel rule t1 > 0; INTERVAL = true keeps t_start < t1 < t_end and also prunes boxes entered
+// beyond t_end (the box holds its Gaussians' ellipsoids, so none of them has a t1 before the box's entry).
+template <bool INTERVAL>
+__device__ __forceinline__ int walk_layers(const BackwardParams& P, const double (&o)[3], const d3& d, double t_start,
+                                           double t_end, double (&kt)[RTGS_MAX_DEPTH], int (&ks)[RTGS_MAX_DEPTH]) {
+    const int K = P.depth;
     int cnt = 0;
-    {
-        const float of[3] = {(float)o[0], (float)o[1], (float)o[2]};
-        const float idf[3] = {1.0f / (float)d.x, 1.0f / (float)d.y, 1.0f / (float)d.z};
-        auto slab = [&](float mnx, float mny, float mnz, float mxx, float mxy, float mxz) -> float {
-            return slab_entry(of, idf, {mnx, mny, mnz}, {mxx, mxy, mxz});
-        };
-        int stack[RTGS_MAX_TREE_DEPTH + 2];
-        int sp = 0;
-        stack[sp++] = 0;
-        while (sp > 0) {
-            const int node = stack[--sp];
-            const float4 a = __ldg(P.nodes + (int64_t)node * 4 + 0), b = __ldg(P.nodes + (int64_t)node * 4 + 1),
-                         c = __ldg(P.nodes + (int64_t)node * 4 + 2), dd = __ldg(P.nodes + (int64_t)node * 4 + 3);
-            const int ch[2] = {__float_as_int(dd.x), __float_as_int(dd.y)};
-            // The root of a single-Gaussian tree has an empty right child (half extent -inf, reference ~0 = leaf 0
-            // again): the slabs of an inverted box span every t, so it is skipped here, or leaf 0 would enter the
-            // k-buffer twice.  (A closest-hit walk can afford the duplicate; a list of layers cannot.)
-            const float te[2] = {a.w >= 0.0f ? slab(a.x - a.w, a.y - b.x, a.z - b.y, a.x + a.w, a.y + b.x, a.z + b.y)
-                                             : INFINITY,
-                                 c.y >= 0.0f ? slab(b.z - c.y, b.w - c.z, c.x - c.w, b.z + c.y, b.w + c.z, c.x + c.w)
-                                             : INFINITY};
-            const int first = te[0] <= te[1] ? 0 : 1;
-            for (int k = 1; k >= 0; --k) {
-                const int w = k == 0 ? first : 1 - first;
-                if (!(te[w] < INFINITY) || (cnt == K && (double)te[w] > kt[K - 1])) continue;
-                if (ch[w] >= 0) {
-                    stack[sp++] = ch[w];
-                    continue;
-                }
-                const int s = ~ch[w];
-                const float4 ra = __ldg(P.raw + (int64_t)s * 3 + 0), rb = __ldg(P.raw + (int64_t)s * 3 + 1),
-                             rc = __ldg(P.raw + (int64_t)s * 3 + 2);
-                const double p[3] = {ra.x, ra.y, ra.z}, q[4] = {ra.w, rb.x, rb.y, rb.z}, sc[3] = {rb.w, rc.x, rc.y};
-                const ExactHit e = exact_intersect(p, q, sc, o, d);
-                if (!(e.hit && e.t1 > 0.0)) continue;
-                const double t = e.t1;
-                if (cnt == K && !(t < kt[K - 1] || (t == kt[K - 1] && s < ks[K - 1]))) continue;
-                int at = cnt < K ? cnt++ : K - 1;
-                while (at > 0 && (t < kt[at - 1] || (t == kt[at - 1] && s < ks[at - 1]))) {
-                    kt[at] = kt[at - 1];
-                    ks[at] = ks[at - 1];
-                    --at;
-                }
-                kt[at] = t;
-                ks[at] = s;
+    const float of[3] = {(float)o[0], (float)o[1], (float)o[2]};
+    const float idf[3] = {1.0f / (float)d.x, 1.0f / (float)d.y, 1.0f / (float)d.z};
+    auto slab = [&](float mnx, float mny, float mnz, float mxx, float mxy, float mxz) -> float {
+        return slab_entry(of, idf, {mnx, mny, mnz}, {mxx, mxy, mxz});
+    };
+    int stack[RTGS_MAX_TREE_DEPTH + 2];
+    int sp = 0;
+    stack[sp++] = 0;
+    while (sp > 0) {
+        const int node = stack[--sp];
+        const float4 a = __ldg(P.nodes + (int64_t)node * 4 + 0), b = __ldg(P.nodes + (int64_t)node * 4 + 1),
+                     c = __ldg(P.nodes + (int64_t)node * 4 + 2), dd = __ldg(P.nodes + (int64_t)node * 4 + 3);
+        const int ch[2] = {__float_as_int(dd.x), __float_as_int(dd.y)};
+        // The root of a single-Gaussian tree has an empty right child (half extent -inf, reference ~0 = leaf 0
+        // again): the slabs of an inverted box span every t, so it is skipped here, or leaf 0 would enter the
+        // k-buffer twice.  (A closest-hit walk can afford the duplicate; a list of layers cannot.)
+        const float te[2] = {a.w >= 0.0f ? slab(a.x - a.w, a.y - b.x, a.z - b.y, a.x + a.w, a.y + b.x, a.z + b.y)
+                                         : INFINITY,
+                             c.y >= 0.0f ? slab(b.z - c.y, b.w - c.z, c.x - c.w, b.z + c.y, b.w + c.z, c.x + c.w)
+                                         : INFINITY};
+        const int first = te[0] <= te[1] ? 0 : 1;
+        for (int k = 1; k >= 0; --k) {
+            const int w = k == 0 ? first : 1 - first;
+            if (!(te[w] < INFINITY) || (cnt == K && (double)te[w] > kt[K - 1])) continue;
+            if (INTERVAL && (double)te[w] > t_end) continue;
+            if (ch[w] >= 0) {
+                stack[sp++] = ch[w];
+                continue;
             }
+            const int s = ~ch[w];
+            const float4 ra = __ldg(P.raw + (int64_t)s * 3 + 0), rb = __ldg(P.raw + (int64_t)s * 3 + 1),
+                         rc = __ldg(P.raw + (int64_t)s * 3 + 2);
+            const double p[3] = {ra.x, ra.y, ra.z}, q[4] = {ra.w, rb.x, rb.y, rb.z}, sc[3] = {rb.w, rc.x, rc.y};
+            const ExactHit e = exact_intersect(p, q, sc, o, d);
+            if (!(e.hit && (INTERVAL ? (e.t1 > t_start && e.t1 < t_end) : e.t1 > 0.0))) continue;
+            const double t = e.t1;
+            if (cnt == K && !(t < kt[K - 1] || (t == kt[K - 1] && s < ks[K - 1]))) continue;
+            int at = cnt < K ? cnt++ : K - 1;
+            while (at > 0 && (t < kt[at - 1] || (t == kt[at - 1] && s < ks[at - 1]))) {
+                kt[at] = kt[at - 1];
+                ks[at] = ks[at - 1];
+                --at;
+            }
+            kt[at] = t;
+            ks[at] = s;
         }
     }
+    return cnt;
+}
 
-    // ---- phase 2: the forward again; kt[k] becomes T_k --------------------------------------------------------
-    double Y[15];
+// Phase 2: the forward again over the cnt layers; kt[k] becomes T_k, Y the SH basis of d / |d|.  The image goes to
+// replay_rgb / replay_T[out] (each may be null); returns the number of layers composited under the t_cut rule.
+__device__ __forceinline__ int replay_layers(const BackwardParams& P, const double (&o)[3], const d3& d, int cnt,
+                                             double (&kt)[RTGS_MAX_DEPTH], const int (&ks)[RTGS_MAX_DEPTH],
+                                             int64_t out, double (&Y)[15]) {
     {
         const double il = 1.0 / sqrt(d.x * d.x + d.y * d.y + d.z * d.z);
         sh_basis_d(d.x * il, d.y * il, d.z * il, Y);
@@ -291,19 +300,24 @@ __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile
         L = k + 1;
     }
     if (P.replay_rgb != nullptr) {
-        P.replay_rgb[pix * 3 + 0] = (float)rgb[0];
-        P.replay_rgb[pix * 3 + 1] = (float)rgb[1];
-        P.replay_rgb[pix * 3 + 2] = (float)rgb[2];
+        P.replay_rgb[out * 3 + 0] = (float)rgb[0];
+        P.replay_rgb[out * 3 + 1] = (float)rgb[1];
+        P.replay_rgb[out * 3 + 2] = (float)rgb[2];
     }
-    if (P.replay_T != nullptr) P.replay_T[pix] = (float)T;
+    if (P.replay_T != nullptr) P.replay_T[out] = (float)T;
+    return L;
+}
 
-    // ---- phase 3: back to front ---------------------------------------------------------------------------------
-    const double gr[3] = {P.dL_drgb[pix * 3 + 0], P.dL_drgb[pix * 3 + 1], P.dL_drgb[pix * 3 + 2]};
-    double B = P.dL_dT != nullptr ? (double)P.dL_dT[pix] : 0.0;
-    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
-    double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};   // CAM: dL/do, dL/dd (geometry)
-    double gY[15];                                             // CAM: dL/dY_j
-    if constexpr (CAM) {
+// Phase 3: back to front over the L composited layers (T_k in kt) from dL/drgb = gr and B = dL/dT, scattering the
+// Gaussian gradients.  RAY_GRAD also returns the ray's own gradient: gO = dL/do, gD = dL/dd including the SH colour's
+// dependence on d / |d| (gO, gD enter as zeros).
+template <bool RAY_GRAD>
+__device__ __forceinline__ void back_to_front(const BackwardParams& P, const double (&o)[3], const d3& d, int L,
+                                              const double (&kt)[RTGS_MAX_DEPTH], const int (&ks)[RTGS_MAX_DEPTH],
+                                              const double (&Y)[15], const double (&gr)[3], double B,
+                                              double (&gO)[3], double (&gD)[3]) {
+    double gY[15];   // RAY_GRAD: dL/dY_j
+    if constexpr (RAY_GRAD) {
 #pragma unroll
         for (int j = 0; j < 15; ++j) gY[j] = 0.0;
     }
@@ -343,7 +357,7 @@ __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile
                 red_add(P.g_pos, g * 3 + j,
                         -2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]));
         }
-        if constexpr (CAM) {
+        if constexpr (RAY_GRAD) {
             // dq/do = 2 W^T e, dq/dd = -2 sigma W^T e
 #pragma unroll
             for (int j = 0; j < 3; ++j) {
@@ -382,7 +396,7 @@ __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile
             for (int i = 0; i < 4; ++i) red_add(P.g_rot, g * 4 + i, gq[i] + 2.0 * ly.q[i] * dLdc);
         }
     }
-    if constexpr (CAM) {
+    if constexpr (RAY_GRAD) {
         // the SH direction d / |d|: dL/dd += (I - dn dn^T) dL/ddn / |d|
         if (P.has_sh) {
             const double il = 1.0 / sqrt(d.x * d.x + d.y * d.y + d.z * d.z);
@@ -393,6 +407,33 @@ __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile
 #pragma unroll
             for (int j = 0; j < 3; ++j) gD[j] += (gn[j] - dn[j] * pr) * il;
         }
+    }
+}
+
+// One pixel of k_render_backward; a pixel that contributes nothing returns early.  With CAM, its camera terms are
+// written to cam_g[CAM_TERMS] (left untouched, i.e. zero, on an early return).
+template <bool CAM>
+__device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile, int lane, double* cam_g) {
+    const int ti = tile / P.tiles_j, tj = tile - ti * P.tiles_j;
+    const int li = ti * TILE_I + lane / TILE_J, lj = tj * TILE_J + lane % TILE_J;   // region-relative pixel
+    if (li >= P.w || lj >= P.h) return;
+    const int pi = P.x0 + li, pj = P.y0 + lj;
+    const int64_t pix = (int64_t)li * P.h + lj;
+    const CamD& cam = P.cam;
+    const double o[3] = {cam.o[0], cam.o[1], cam.o[2]};
+    const d3 d = cam_dir(cam, (double)pi + 0.5, (double)pj + 0.5);
+
+    double kt[RTGS_MAX_DEPTH];
+    int ks[RTGS_MAX_DEPTH];
+    const int cnt = walk_layers<false>(P, o, d, 0.0, INFINITY, kt, ks);
+    double Y[15];
+    const int L = replay_layers(P, o, d, cnt, kt, ks, pix, Y);
+    const double gr[3] = {P.dL_drgb[pix * 3 + 0], P.dL_drgb[pix * 3 + 1], P.dL_drgb[pix * 3 + 2]};
+    const double B = P.dL_dT != nullptr ? (double)P.dL_dT[pix] : 0.0;
+    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
+    double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};   // CAM: dL/do, dL/dd
+    back_to_front<CAM>(P, o, d, L, kt, ks, Y, gr, B, gO, gD);
+    if constexpr (CAM) {
         // d = Rm dc, dc = n / |n| as cam_dir computes them
         const double px = ((double)pi + 0.5 - 0.5 * (double)cam.W) * cam.ifx;
         const double py = ((double)pj + 0.5 - 0.5 * (double)cam.H) * cam.ify;
@@ -435,8 +476,11 @@ __device__ __forceinline__ void cam_block_reduce(const BackwardParams& P, double
 
 // CAM = false: the Gaussian gradients.  CAM = true: also the camera's, as per-CTA partials in P.cam_part (finished
 // by k_camera_grad_finalize).
+// The minimum CTA counts hold both instantiations at their occupancy (128 registers: 4 CTAs per SM, 168: 3); left to
+// itself ptxas gives the CAM path 178 registers without spills, which fits only 2.
 template <bool CAM>
-__global__ void __launch_bounds__(BWD_WARPS * 32) k_render_backward(const __grid_constant__ BackwardParams P) {
+__global__ void __launch_bounds__(BWD_WARPS * 32, CAM ? 3 : 4)
+    k_render_backward(const __grid_constant__ BackwardParams P) {
     const int lane = threadIdx.x & 31;
     const int tile = blockIdx.x * BWD_WARPS + (threadIdx.x >> 5);
     if constexpr (!CAM) {
@@ -485,6 +529,71 @@ __global__ void __launch_bounds__(FIN_THREADS) k_camera_grad_finalize(const doub
     if (g_focal != nullptr) {
         g_focal[0] += (float)red[12][0];
         g_focal[1] += (float)red[13][0];
+    }
+}
+
+// ---- arbitrary rays (rtgs_render_rays / rtgs_render_rays_backward): one thread per ray ----------------------------
+
+constexpr int RAY_THREADS = 128;
+
+// Ray r of the (nrays, 8) record (o xyz, d xyz, start, end; 16-byte aligned, two float4 loads).  False for a ray that
+// composites nothing: a non-finite o or d component, d = 0, or !(start < end) (NaN included).
+__device__ __forceinline__ bool load_ray(const BackwardParams& P, int64_t r, double (&o)[3], d3& d, double& t_start,
+                                         double& t_end) {
+    const float4 a = __ldg(reinterpret_cast<const float4*>(P.rays) + r * 2 + 0),
+                 b = __ldg(reinterpret_cast<const float4*>(P.rays) + r * 2 + 1);
+    o[0] = a.x; o[1] = a.y; o[2] = a.z;
+    d = d3make(a.w, b.x, b.y);
+    t_start = b.z;
+    t_end = b.w;
+    const bool finite = isfinite(a.x) && isfinite(a.y) && isfinite(a.z) && isfinite(a.w) && isfinite(b.x) &&
+                        isfinite(b.y);
+    return finite && (a.w != 0.0f || b.x != 0.0f || b.y != 0.0f) && b.z < b.w;
+}
+
+// Phases 1-2 per ray: float32 rgb to replay_rgb (n,3), T to replay_T (n) if not null.  The same code as the replay
+// of k_render_rays_backward, so the two agree bit for bit.
+__global__ void __launch_bounds__(RAY_THREADS) k_render_rays(const __grid_constant__ BackwardParams P) {
+    const int64_t r = blockIdx.x * (int64_t)RAY_THREADS + threadIdx.x;
+    if (r >= P.nrays) return;
+    double o[3], t_start, t_end;
+    d3 d;
+    double kt[RTGS_MAX_DEPTH];
+    int ks[RTGS_MAX_DEPTH];
+    const int cnt = load_ray(P, r, o, d, t_start, t_end) ? walk_layers<true>(P, o, d, t_start, t_end, kt, ks) : 0;
+    double Y[15];
+    replay_layers(P, o, d, cnt, kt, ks, r, Y);   // no layer: rgb 0, T 1
+}
+
+// Phases 1-3 per ray.  RAY_GRAD = false: the Gaussian gradients only.  RAY_GRAD = true: also dL/do and dL/dd, added
+// by the ray's own thread to g_rays[r * 8 + 0..5] (no atomics: deterministic).
+// at the occupancy of the matching k_render_backward instantiation
+template <bool RAY_GRAD>
+__global__ void __launch_bounds__(RAY_THREADS, RAY_GRAD ? 3 : 4)
+    k_render_rays_backward(const __grid_constant__ BackwardParams P) {
+    const int64_t r = blockIdx.x * (int64_t)RAY_THREADS + threadIdx.x;
+    if (r >= P.nrays) return;
+    double o[3], t_start, t_end;
+    d3 d;
+    double kt[RTGS_MAX_DEPTH];
+    int ks[RTGS_MAX_DEPTH];
+    const bool valid = load_ray(P, r, o, d, t_start, t_end);
+    const int cnt = valid ? walk_layers<true>(P, o, d, t_start, t_end, kt, ks) : 0;
+    double Y[15];
+    const int L = replay_layers(P, o, d, cnt, kt, ks, r, Y);
+    if (!valid) return;
+    const double gr[3] = {P.dL_drgb[r * 3 + 0], P.dL_drgb[r * 3 + 1], P.dL_drgb[r * 3 + 2]};
+    const double B = P.dL_dT != nullptr ? (double)P.dL_dT[r] : 0.0;
+    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
+    double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};
+    back_to_front<RAY_GRAD>(P, o, d, L, kt, ks, Y, gr, B, gO, gD);
+    if constexpr (RAY_GRAD) {
+        float* g = P.g_rays + r * 8;
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            g[j] += (float)gO[j];
+            g[3 + j] += (float)gD[j];
+        }
     }
 }
 

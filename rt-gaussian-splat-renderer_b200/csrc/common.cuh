@@ -181,6 +181,11 @@ int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, i
                                 float t_cut, const float* dL_drgb, const float* dL_dT, float* const grads[6],
                                 float* const cam_grads[3], float* replay_rgb, float* replay_T,
                                 cudaStream_t stream);  // render.cu (backward.cuh)
+int rtgs_launch_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut, float* out_rgb,
+                            float* out_T, cudaStream_t stream);  // render.cu (backward.cuh)
+int rtgs_launch_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut,
+                                     const float* dL_drgb, const float* dL_dT, float* const grads[6], float* grad_rays,
+                                     float* replay_rgb, float* replay_T, cudaStream_t stream);
 int rtgs_launch_generate_rays(const rtgs_camera* cam, float* rays, cudaStream_t stream);
 int rtgs_launch_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, int32_t* idx,
                               float* t12, cudaStream_t stream);

@@ -23,6 +23,7 @@
 //   k_generate_rays, k_trace_closest, k_activate_ply   API companions (Camera.generate_ray_field, Scene.hit, PLY ingest)
 //   k_render_backward  gradient of the render with respect to the Gaussian parameters and, as
 //                      k_render_backward<true> + k_camera_grad_finalize, the camera (backward.cuh)
+//   k_render_rays, k_render_rays_backward   the same per-ray code for arbitrary (n,8) rays (backward.cuh)
 #include <stdlib.h>
 
 #include "backward.cuh"
@@ -963,6 +964,54 @@ int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, i
     const cudaError_t ef = cudaFreeAsync(P.cam_part, stream);
     CUDA_TRY(e);
     CUDA_TRY(ef);
+    return RTGS_OK;
+}
+
+// The parameters of the ray kernels (no camera, no region); dL, gradient and output pointers are set by the caller.
+static backward::BackwardParams rays_params(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut) {
+    backward::BackwardParams P = {};
+    P.nodes = s->nodes;
+    P.geo = s->geo;
+    P.shp = s->shp;
+    P.raw = s->raw;
+    P.depth = depth;
+    P.t_cut = t_cut;
+    P.has_sh = s->has_sh ? 1 : 0;
+    P.rays = rays;
+    P.nrays = nrays;
+    return P;
+}
+
+int rtgs_launch_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut, float* out_rgb,
+                            float* out_T, cudaStream_t stream) {
+    if (nrays == 0) return RTGS_OK;
+    backward::BackwardParams P = rays_params(s, nrays, rays, depth, t_cut);
+    P.replay_rgb = out_rgb;
+    P.replay_T = out_T;
+    const unsigned blocks = (unsigned)((nrays + backward::RAY_THREADS - 1) / backward::RAY_THREADS);
+    backward::k_render_rays<<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    CUDA_TRY(cudaGetLastError());
+    return RTGS_OK;
+}
+
+int rtgs_launch_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut,
+                                     const float* dL_drgb, const float* dL_dT, float* const grads[6], float* grad_rays,
+                                     float* replay_rgb, float* replay_T, cudaStream_t stream) {
+    if (nrays == 0) return RTGS_OK;
+    backward::BackwardParams P = rays_params(s, nrays, rays, depth, t_cut);
+    P.dL_drgb = dL_drgb;
+    P.dL_dT = dL_dT;
+    P.g_pos = grads[0]; P.g_rot = grads[1]; P.g_scale = grads[2];
+    P.g_color = grads[3]; P.g_opacity = grads[4]; P.g_sh = s->has_sh ? grads[5] : nullptr;
+    P.g_rays = grad_rays;
+    P.replay_rgb = replay_rgb;
+    P.replay_T = replay_T;
+    const unsigned blocks = (unsigned)((nrays + backward::RAY_THREADS - 1) / backward::RAY_THREADS);
+    if (grad_rays == nullptr)
+        backward::k_render_rays_backward<false><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    else
+        backward::k_render_rays_backward<true><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
 

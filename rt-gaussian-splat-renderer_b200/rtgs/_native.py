@@ -96,6 +96,9 @@ SIGNATURES = {
                                                  C.c_int32, C.c_int32, C.c_float, _vp, C.c_int32]),
     "rtgs_generate_rays": (C.c_int, [C.POINTER(rtgs_camera), C.c_int, _vp, _vp]),
     "rtgs_trace_closest": (C.c_int, [_vp, C.c_int64, _vp, _vp, _vp, _vp]),
+    "rtgs_render_rays": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp]),
+    "rtgs_render_rays_backward": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp,
+                                            _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rtgs_scene_destroy": (C.c_int, [_vp]),
 }
 

@@ -14,7 +14,9 @@ optimisation loop::
 Each call rebuilds the scene's LBVH from the current values (the parameters may have moved since the last step), so
 the forward of one step and the backward of the same step see the same tree only if no other call updates the scene
 in between.  ``render_camera`` renders the scene as stored, differentiable with respect to the camera only, and
-rebuilds nothing: the loop of pose refinement or of tracking a camera against a fixed scene.
+rebuilds nothing: the loop of pose refinement or of tracking a camera against a fixed scene.  ``render_rays`` renders
+arbitrary rays (non-pinhole cameras, ray batches drawn from many views) and differentiates with respect to the rays
+too (``rtgs_render_rays`` / ``rtgs_render_rays_backward``).
 """
 from __future__ import annotations
 
@@ -128,3 +130,62 @@ def render_camera(scene, camera, position=None, rotation=None, focal=None, depth
         raise ValueError(f"depth must be in [1, {MAX_DEPTH}]")
     return _Render.apply(scene, camera, int(depth), float(t_cut), tile, False, position, rotation, focal,
                          None, None, None, None, None, None)
+
+
+class _RenderRays(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, scene, depth, t_cut, update, rays, pos, rot, scale, color, opacity, sh):
+        if update:
+            scene.set_gaussians(*(t.detach().contiguous() if t is not None else None
+                                  for t in (pos, rot, scale, color, opacity, sh)))
+        rgb, T = scene.render_rays(rays, depth, t_cut)
+        ctx.save_for_backward(rays)
+        ctx.scene, ctx.depth, ctx.t_cut, ctx.has_sh = scene, depth, t_cut, sh is not None
+        return rgb, T
+
+    @staticmethod
+    def backward(ctx, g_rgb, g_T):
+        (rays,) = ctx.saved_tensors
+        scene = ctx.scene
+        rays_c = scene._rays_arg(rays)
+        dev, lead = rays_c.device, tuple(rays_c.shape[:-1])
+        n = scene.num_gaussians
+        shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,), sh=(n, 15, 3))
+        need = dict(zip(_NAMES, ctx.needs_input_grad[5:]))
+        need["sh"] = need["sh"] and ctx.has_sh
+        grads = {k: torch.zeros(shapes[k], dtype=torch.float32, device=dev) if need[k] else None for k in _NAMES}
+        g_rays = torch.zeros(lead + (8,), dtype=torch.float32, device=dev) if ctx.needs_input_grad[4] else None
+        if g_rgb is None:
+            g_rgb = torch.zeros(lead + (3,), dtype=torch.float32, device=dev)
+        g_rgb = g_rgb.to(torch.float32).contiguous()
+        g_T = None if g_T is None else g_T.to(torch.float32).contiguous()
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        _native.check(_native.load().rtgs_render_rays_backward(
+            scene.handle, rays_c.numel() // 8, rays_c.data_ptr(), ctx.depth, ctx.t_cut, g_rgb.data_ptr(), ptr(g_T),
+            *(ptr(grads[k]) for k in _NAMES), ptr(g_rays), None, None, torch.cuda.current_stream(dev).cuda_stream))
+        return (None,) * 4 + (g_rays,) + tuple(grads[k] for k in _NAMES)
+
+
+def render_rays(scene, rays, pos=None, rot=None, scale=None, color=None, opacity=None, sh=None, depth: int = 16,
+                t_cut: float = 0.0):
+    """Composite arbitrary rays and return ``(rgb (..., 3), T (...))``, differentiable with respect to the rays and,
+    when they are given, the Gaussian parameters (``Scene.render_rays`` / ``render_rays_backward``).
+
+    ``rays`` is a CUDA float32 (..., 8) tensor on the scene's device (origin, direction, start, end); it gets a
+    gradient (dL/do, dL/dd; none for start and end) when it requires one, so any camera model written in torch is
+    differentiable through the render.  Pass either every Gaussian tensor (``sh`` iff the scene has SH), and the
+    scene is updated and rebuilt from them as in ``render``, or none, and the stored scene is rendered as it is:
+    nothing is rebuilt and nothing is read to the host.  A training step on random rays of many views::
+
+        rays = torch.cat([cam_rays[v][idx[v]] for v in views])          # (B, 8)
+        rgb, _ = rtgs.autograd.render_rays(scene, rays, pos, rot, scale, color, opacity, sh)
+        loss = ((rgb - target) ** 2).mean(); opt.zero_grad(); loss.backward(); opt.step()
+    """
+    if not 1 <= int(depth) <= MAX_DEPTH:
+        raise ValueError(f"depth must be in [1, {MAX_DEPTH}]")
+    given = [t is not None for t in (pos, rot, scale, color, opacity)]
+    if any(given) and not all(given):
+        raise ValueError("pass all of pos, rot, scale, color, opacity (and sh for a scene with SH), or none")
+    if not any(given) and sh is not None:
+        raise ValueError("sh was given without the other Gaussian tensors")
+    return _RenderRays.apply(scene, int(depth), float(t_cut), all(given), rays, pos, rot, scale, color, opacity, sh)

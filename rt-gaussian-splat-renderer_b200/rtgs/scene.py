@@ -414,3 +414,89 @@ class Scene:
             hitm = idx >= 0
             depth[hitm] = bf["depth"][self._n - 1 + inv[idx[hitm]]]
         return SceneHit(gaussian_idx=idx, intersections=d_t.cpu().numpy(), depth=depth)
+
+    # ------------------------------------------------------------------ arbitrary rays
+    def _rays_arg(self, rays):
+        """``rays`` as a contiguous, 16-byte aligned CUDA float32 (..., 8) tensor on the scene's device."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if not isinstance(rays, torch.Tensor) or rays.device != dev or rays.dtype != torch.float32:
+            raise ValueError(f"rays: expected a float32 tensor on {dev}")
+        if rays.dim() < 1 or rays.shape[-1] != 8:
+            raise ValueError(f"rays: expected shape (..., 8), got {tuple(rays.shape)}")
+        rays = rays.detach().contiguous()
+        if rays.data_ptr() % 16:
+            rays = rays.clone()
+        return rays
+
+    @staticmethod
+    def _buffer(t, shape, name, dev):
+        import torch
+        if t is None:
+            return None
+        if (not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.float32
+                or tuple(t.shape) != tuple(shape) or not t.is_contiguous()):
+            raise ValueError(f"{name}: expected a contiguous float32 tensor of shape {tuple(shape)} on {dev}")
+        return t
+
+    def render_rays(self, rays, depth: int = 16, t_cut: float = 0.0, out=None, out_T=None):
+        """Composite arbitrary rays (rtgs_render_rays) on the current stream and return ``(rgb (..., 3), T (...))``.
+
+        ``rays`` is a CUDA float32 tensor of shape (..., 8) on the scene's device: origin, direction (used as given,
+        not normalised), start, end - the record of ``Camera.generate_ray_field``, so a (W,H,8) ray field gives a
+        (W,H,3) image in the layout of ``RayTracer.render_device``.  Each ray composites its ``depth`` nearest
+        Gaussians with start < t1 < end, front to back while T >= ``t_cut``.  ``out`` / ``out_T`` may pass the output
+        tensors."""
+        import torch
+        rays = self._rays_arg(rays)
+        dev = rays.device
+        lead = tuple(rays.shape[:-1])
+        out = self._buffer(out, lead + (3,), "out", dev)
+        out_T = self._buffer(out_T, lead, "out_T", dev)
+        if out is None:
+            out = torch.empty(lead + (3,), dtype=torch.float32, device=dev)
+        if out_T is None:
+            out_T = torch.empty(lead, dtype=torch.float32, device=dev)
+        _native.check(_native.load().rtgs_render_rays(self.handle, rays.numel() // 8, rays.data_ptr(), int(depth),
+                                                      float(t_cut), out.data_ptr(), out_T.data_ptr(),
+                                                      torch.cuda.current_stream(dev).cuda_stream))
+        return out, out_T
+
+    def render_rays_backward(self, rays, dL_drgb, dL_dT=None, depth: int = 16, t_cut: float = 0.0, grads=None,
+                             rays_grad: bool = False, replay: bool = False):
+        """Gradient of ``render_rays(rays, depth, t_cut)`` with each ray's layer list held fixed
+        (rtgs_render_rays_backward), on the current stream.
+
+        dL_drgb (..., 3) and dL_dT (...) are CUDA float32 tensors shaped like the rays.  Returns a dict of (n, ...)
+        float32 gradients ``pos rot scale color opacity`` and ``sh`` (scenes with SH), as ``RayTracer.render_backward``
+        does; with ``rays_grad=True`` also ``rays`` (..., 8): dL/do in columns 0-2, dL/dd in 3-5, zeros in 6-7.
+        ``grads`` may pass tensors of these names to accumulate into (missing ones are zero-initialised).  With
+        ``replay=True`` the dict also holds ``rgb`` / ``T``, the image the backward recomputed."""
+        import torch
+        rays = self._rays_arg(rays)
+        dev = rays.device
+        lead = tuple(rays.shape[:-1])
+        dL_drgb = self._buffer(dL_drgb.contiguous(), lead + (3,), "dL_drgb", dev)
+        dL_dT = None if dL_dT is None else self._buffer(dL_dT.contiguous(), lead, "dL_dT", dev)
+        n = self._n
+        shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
+        if self.has_sh:
+            shapes["sh"] = (n, 15, 3)
+        if rays_grad:
+            shapes["rays"] = lead + (8,)
+        out = dict(grads or {})
+        for name, shape in shapes.items():
+            if name not in out:
+                out[name] = torch.zeros(shape, dtype=torch.float32, device=dev)
+            else:
+                self._buffer(out[name], shape, f"grads[{name!r}]", dev)
+        if replay:
+            out["rgb"] = torch.empty(lead + (3,), dtype=torch.float32, device=dev)
+            out["T"] = torch.empty(lead, dtype=torch.float32, device=dev)
+        ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
+        _native.check(_native.load().rtgs_render_rays_backward(
+            self.handle, rays.numel() // 8, rays.data_ptr(), int(depth), float(t_cut), dL_drgb.data_ptr(),
+            None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
+            ptr("opacity"), ptr("sh"), ptr("rays") if rays_grad else None, ptr("rgb"), ptr("T"),
+            torch.cuda.current_stream(dev).cuda_stream))
+        return out
