@@ -63,11 +63,10 @@ constexpr int STACK_SINGLE = STACK_CAP - 32 - RTGS_MAX_TREE_DEPTH;
 constexpr int CQ_CAP = 96;
 #endif
 static_assert(STACK_SINGLE >= 64, "k_render: stack too small for batched traversal");
-constexpr int BATCH = 32;
-constexpr int REC_Q = 5;                 // quads per staged record (80-byte stride: conflict-free gathers)
+constexpr int BATCH = REC_BATCH;
 
 struct __align__(16) TraversalScratch {
-    float4 rec[BATCH][REC_Q];   // precise records (render_common.cuh: stage_candidate)
+    StagedRecords rec;          // precise records (render_common.cuh: stage_candidate)
     float4 polyA[BATCH];        // coarse quadratics {c0 c1 c2 c3}
     float4 polyB[BATCH];        //                   {c4 c5 t_lo -}: t_lo = no ray of the tile enters the candidate before it
     int stack[STACK_CAP];
@@ -151,7 +150,8 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
         // direction among the tile's rays (corners and centre, with a margin for the rays in between).
         float len_max;
         {
-            double l2 = d3dot(ry.d0, ry.d0);
+            const d3 dc = cam_dir(cam, (double)i0 + 0.5 * TILE_I, (double)j0 + 0.5 * TILE_J);   // tile-centre ray
+            double l2 = d3dot(dc, dc);
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 const d3 e = cam_dir(cam, (double)(i0 + (k & 1) * TILE_I), (double)(j0 + (k >> 1) * TILE_J));
@@ -339,13 +339,13 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                 ncq -= m;
                 const int m4 = (m + 3) & ~3;
                 if (lane < m) {
-                    float4 rec[5];
-                    float poly[6];
-                    stage_candidate<true>(P, ry, tr.cq[ncq + lane], rec, poly);
+                    float4 rec[REC_QUADS];
+                    float poly[6], t_lo;
+                    stage_candidate<true>(P, ry, tr.cq[ncq + lane], rec, poly, t_lo);
 #pragma unroll
-                    for (int k = 0; k < 5; ++k) tr.rec[lane][k] = rec[k];
+                    for (int k = 0; k < REC_QUADS; ++k) tr.rec[k][lane] = rec[k];
                     tr.polyA[lane] = make_float4(poly[0], poly[1], poly[2], poly[3]);
-                    tr.polyB[lane] = make_float4(poly[4], poly[5], rec[4].w, 0.0f);
+                    tr.polyB[lane] = make_float4(poly[4], poly[5], t_lo, 0.0f);
                 } else if (lane < m4) {   // pad to a multiple of 4: never a candidate
                     tr.polyA[lane] = make_float4(1.0f, 0.0f, 0.0f, 0.0f);
                     tr.polyB[lane] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
@@ -379,7 +379,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                     if (mask != 0) {
                         const int c = __ffs(mask) - 1;
                         mask &= mask - 1;
-                        const PreciseHit h = precise_test(P, tr.rec[c], ry.dlx, ry.dly, ry.dlz, pi, pj);
+                        const PreciseHit h = precise_test(P, tr.rec, c, ry, pi, pj);
                         ST(st_f64 += h.refined);
                         if (h.hit && h.t1 <= d_T) {
                             kb_dirty = true;
@@ -502,7 +502,11 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
             const unsigned long long perm = order_hits16(P, ws.kb_t, ws.kb_i, cnt, maxcnt, lane, pi, pj, n_exact);
             ST(st_f64 += n_exact);
             float Y[15];
-            sh_basis(ry.dnx, ry.dny, ry.dnz, Y);
+            {
+                float dx, dy, dz;
+                sh_direction(cam, i0, j0, pi, pj, active, dx, dy, dz);
+                sh_basis(dx, dy, dz, Y);
+            }
             const int nmine = min(cnt, P.depth);
             const int nloop = min(maxcnt, P.depth);
 #pragma unroll 1
@@ -566,7 +570,11 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
             // eval_sh(normalize(dir)) (gaussian.py:199-200).
             {
                 float Y[15];
-                sh_basis(ry.dnx, ry.dny, ry.dnz, Y);
+                {
+                    float dx, dy, dz;
+                    sh_direction(cam, i0, j0, pi, pj, active, dx, dy, dz);
+                    sh_basis(dx, dy, dz, Y);
+                }
                 const int nmine = min(cnt, P.depth);
                 const int nloop = min(maxcnt, P.depth);
 #pragma unroll 1

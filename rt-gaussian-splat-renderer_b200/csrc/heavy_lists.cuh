@@ -45,7 +45,7 @@ constexpr float HEAVY_MARGIN = 1.0001f;  // limit = farthest 16th hit x this (fl
 
 struct __align__(16) HeavyShared {
     ListsShared l;                         // traversal stack, the tile's candidates so far, output queue
-    float4 rec[SHADE_BATCH][SHADE_REC_Q];  // staging of one batch of candidates (as ShadeShared)
+    StagedRecords rec;                     // staging of one batch of candidates (as ShadeShared)
     float4 polyA[SHADE_BATCH];
     float2 polyB[SHADE_BATCH];
 };
@@ -82,7 +82,7 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
     // ---- the depth functional --------------------------------------------------------------------------------------
     float zc[3], za[3], zo;
     {
-        const d3 dc = tr.d0;
+        const d3 dc = cam_dir(cam, (double)i0 + 0.5 * TILE_I, (double)j0 + 0.5 * TILE_J);   // tile-centre ray
         // L: the longest direction among the tile's corner and centre rays (1 for a unit camera quaternion), plus a
         // margin for the rays in between
         double l2 = d3dot(dc, dc);
@@ -197,11 +197,11 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
             __syncwarp();
             const int m4 = (m + 3) & ~3;
             if (lane < m) {
-                float4 rec[5];
-                float poly[6];
-                stage_candidate(P, tr, ws.glist[nk + lane], rec, poly);
+                float4 rec[REC_QUADS];
+                float poly[6], t_lo;
+                stage_candidate(P, tr, ws.glist[nk + lane], rec, poly, t_lo);
 #pragma unroll
-                for (int k = 0; k < 5; ++k) hs.rec[lane][k] = rec[k];
+                for (int k = 0; k < REC_QUADS; ++k) hs.rec[k][lane] = rec[k];
                 hs.polyA[lane] = make_float4(poly[0], poly[1], poly[2], poly[3]);
                 hs.polyB[lane] = make_float2(poly[4], poly[5]);
             } else if (lane < m4) {
@@ -230,7 +230,7 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
                 if (mask != 0) {
                     const int c = __ffs(mask) - 1;
                     mask &= mask - 1;
-                    const PreciseHit h = precise_test(P, hs.rec[c], tr.dlx, tr.dly, tr.dlz, pi, pj);
+                    const PreciseHit h = precise_test(P, hs.rec, c, tr, pi, pj);
                     if (h.hit && h.t1 < kmax) {
                         const int slot = kcnt < HEAVY_K ? kcnt : kslot;
                         kb[slot] = h.t1;

@@ -454,14 +454,14 @@ __device__ __forceinline__ float sqrt_approx(float x) {
 // Rays of one tile (float64 setup, camera.py:46-52).  Image-plane coordinates: px = (i + 0.5 - W/2)/fx.
 // Tile centre (px0, py0); own offset (a, b) = (px - px0, py - py0).  UNNORMALISED directions are linear
 // in (a, b):  D(a,b) = R (px0 + a, py0 + b, -1) = D0 + a Rx + b Ry;  the reference's direction is
-// d = D / sqrt(px^2 + py^2 + 1); d0 likewise for the tile centre, d = d0 + delta.
+// d = D / L with L = sqrt(px^2 + py^2 + 1), so the ray point o + t d is o + u D at u = t / L.
 struct TileRays {
-    d3 D0, d0;
-    double inv_d0d0;
-    float dlx, dly, dlz;   // delta = d - d0
-    float dnx, dny, dnz;   // normalize(d) for the SH basis (gaussian.py:200)
+    d3 D0;                 // D(0,0), the tile-centre direction
+    double inv_D0D0;       // 1 / |D0|^2
+    float L;               // the lane's L
     float pa, pb;          // (a, b)
-    float a_max, b_max, dl_max;
+    float a_max, b_max;    // |a| <= a_max, |b| <= b_max on every pixel of the tile
+    float L_lo, L_hi;      // L_lo <= L <= L_hi on every pixel of the tile
 };
 
 __device__ __forceinline__ void make_tile_rays(const CamD& cam, int i0, int j0, int pi, int pj, bool active,
@@ -469,40 +469,61 @@ __device__ __forceinline__ void make_tile_rays(const CamD& cam, int i0, int j0, 
     const double px0 = ((double)i0 + 0.5 * TILE_I - 0.5 * cam.W) * cam.ifx;
     const double py0 = ((double)j0 + 0.5 * TILE_J - 0.5 * cam.H) * cam.ify;
     r.D0 = cam_rot(cam, px0, py0, -1.0);
-    const double n0 = rsqrt(px0 * px0 + py0 * py0 + 1.0);
-    r.d0 = d3make(r.D0.x * n0, r.D0.y * n0, r.D0.z * n0);
-    r.inv_d0d0 = 1.0 / d3dot(r.d0, r.d0);
+    r.inv_D0D0 = 1.0 / d3dot(r.D0, r.D0);
     const double ad = active ? ((double)(pi - i0) + 0.5 - 0.5 * TILE_I) * cam.ifx : 0.0;
     const double bd = active ? ((double)(pj - j0) + 0.5 - 0.5 * TILE_J) * cam.ify : 0.0;
     {
         const double px = px0 + ad, py = py0 + bd;
-        const double nn = rsqrt(px * px + py * py + 1.0);
-        const d3 dw = d3make((r.D0.x + ad * cam.R[0] + bd * cam.R[1]) * nn, (r.D0.y + ad * cam.R[3] + bd * cam.R[4]) * nn,
-                             (r.D0.z + ad * cam.R[6] + bd * cam.R[7]) * nn);
-        r.dlx = (float)(dw.x - r.d0.x); r.dly = (float)(dw.y - r.d0.y); r.dlz = (float)(dw.z - r.d0.z);
-        const double il = rsqrt(d3dot(dw, dw));
-        r.dnx = (float)(dw.x * il); r.dny = (float)(dw.y * il); r.dnz = (float)(dw.z * il);
+        const double l2 = px * px + py * py + 1.0;
+        r.L = (float)(l2 * rsqrt(l2));
     }
     r.pa = (float)ad;
     r.pb = (float)bd;
-    r.a_max = (float)(0.5 * TILE_I * fabs(cam.ifx));
-    r.b_max = (float)(0.5 * TILE_J * fabs(cam.ify));
-    float m = sqrtf(r.dlx * r.dlx + r.dly * r.dly + r.dlz * r.dlz);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(FULL, m, o));
-    r.dl_max = m;
+    const double am = 0.5 * TILE_I * fabs(cam.ifx), bm = 0.5 * TILE_J * fabs(cam.ify);
+    r.a_max = (float)am;
+    r.b_max = (float)bm;
+    const double xl = fmax(fabs(px0) - am, 0.0), yl = fmax(fabs(py0) - bm, 0.0);
+    const double xh = fabs(px0) + am, yh = fabs(py0) + bm;
+    r.L_lo = __double2float_rd(sqrt(xl * xl + yl * yl + 1.0));
+    r.L_hi = __double2float_ru(sqrt(xh * xh + yh * yh + 1.0));
 }
 
-// Per-(tile, candidate) staging in float64 by one lane: the precise record (origin shifted to the
-// closest point of the tile-centre ray) and the coarse quadratic.
-//   rec: {W00 W01 W02 W10} {W11 W12 W20 W21} {W22 e0.xyz} {g0.xyz t_c} {opacity, s, band, t_lo}
-//   poly: S(a,b) = c0 + a (c1 + a c3 + b c4) + b (c2 + b c5) < 0  <=>  possibly q < 3 + band
+// normalize(d) of the lane's ray (make_tile_rays) for the SH basis (gaussian.py:200).  Taken where the colours are
+// evaluated: carried from make_tile_rays, it held three registers through the candidate loops.
+__device__ __forceinline__ void sh_direction(const CamD& cam, int i0, int j0, int pi, int pj, bool active, float& x,
+                                             float& y, float& z) {
+    const double px0 = ((double)i0 + 0.5 * TILE_I - 0.5 * cam.W) * cam.ifx;
+    const double py0 = ((double)j0 + 0.5 * TILE_J - 0.5 * cam.H) * cam.ify;
+    const d3 D0 = cam_rot(cam, px0, py0, -1.0);
+    const double ad = active ? ((double)(pi - i0) + 0.5 - 0.5 * TILE_I) * cam.ifx : 0.0;
+    const double bd = active ? ((double)(pj - j0) + 0.5 - 0.5 * TILE_J) * cam.ify : 0.0;
+    const double px = px0 + ad, py = py0 + bd;
+    const double nn = rsqrt(px * px + py * py + 1.0);
+    const d3 dw = d3make((D0.x + ad * cam.R[0] + bd * cam.R[1]) * nn, (D0.y + ad * cam.R[3] + bd * cam.R[4]) * nn,
+                         (D0.z + ad * cam.R[6] + bd * cam.R[7]) * nn);
+    const double il = rsqrt(d3dot(dw, dw));
+    x = (float)(dw.x * il); y = (float)(dw.y * il); z = (float)(dw.z * il);
+}
+
+// Staged precise records of one batch, structure of arrays: quad k of candidate c is rec[k][c], so that a warp
+// gathering 32 different candidates reads each quad in the minimum of 4 shared-memory wavefronts.
+constexpr int REC_BATCH = 32;
+constexpr int REC_QUADS = 4;
+typedef float4 StagedRecords[REC_QUADS][REC_BATCH];
+
+// Per-(tile, candidate) staging in float64 by one lane: the precise record (origin shifted to the point of
+// the tile-centre ray closest to the mean) and the coarse quadratic.
+//   rec: {G0.xyz Gx.x} {Gx.yz Gy.xy} {Gy.z e0.xyz} {u_c, opacity, s, band}
 // With o' = W (o - p) = -W v and G(a,b) = W D(a,b) = G0 + a Gx + b Gy:
+//   u_c = v.D0 / |D0|^2,  e0 = W (o + u_c D0 - p) = o' + u_c G0  (precise_test);
 //   q(a,b) = |o' x G|^2 / |G|^2 = N/Dn,  m = o' x G = M0 + a Mx + b My,
+//   poly: S(a,b) = c0 + a (c1 + a c3 + b c4) + b (c2 + b c5) < 0  <=>  possibly q < 3 + band,
 //   S = N - (3 + band) Dn - margin, margin bounding the float32 evaluation error.
+// WITH_T_LO: t_lo = a lower bound of the entry distance of every ray of the tile (only the fused kernel uses it: it
+// prunes per ray by distance); otherwise t_lo is not written.
 template <bool WITH_T_LO = false>
-__device__ __forceinline__ void stage_candidate(const RenderParams& P, const TileRays& tr, int s, float4 (&rec)[5],
-                                                float (&poly)[6]) {
+__device__ __forceinline__ void stage_candidate(const RenderParams& P, const TileRays& tr, int s,
+                                                float4 (&rec)[REC_QUADS], float (&poly)[6], float& t_lo) {
     const CamD& cam = P.cam;
     float4 g0, g1, g2, g3;
 #if SHADE_GEO_TEX
@@ -522,30 +543,31 @@ __device__ __forceinline__ void stage_candidate(const RenderParams& P, const Til
                       W20 * v.x + W21 * v.y + W22 * v.z);
     };
     const d3 v = d3make((double)g0.x - cam.o[0], (double)g0.y - cam.o[1], (double)g0.z - cam.o[2]);
-    const double tc = d3dot(v, tr.d0) * tr.inv_d0d0;
-    const d3 e0 = Wmul(d3make(tc * tr.d0.x - v.x, tc * tr.d0.y - v.y, tc * tr.d0.z - v.z));
-    const d3 gd = Wmul(tr.d0);
-    const float wn = sqrtf(g1.x * g1.x + g1.y * g1.y + g1.z * g1.z + g1.w * g1.w + g2.x * g2.x + g2.y * g2.y +
-                           g2.z * g2.z + g2.w * g2.w + g3.x * g3.x);
-    const float eb = (float)sqrt(d3dot(e0, e0)) + fabsf((float)tc) * tr.dl_max * wn;
-    const float band = 4e-6f * (3.0f + eb * eb);
-    rec[0] = g1;
-    rec[1] = g2;
-    rec[2] = make_float4(g3.x, (float)e0.x, (float)e0.y, (float)e0.z);
-    rec[3] = make_float4((float)gd.x, (float)gd.y, (float)gd.z, (float)tc);
-    // lower bound of the entry distance for every ray of the tile: t1 = tc + tau with
-    // |tau| <= (|e| + sqrt 3) / |W d|, |e| <= eb (above) and |W d| >= |W d0| - |W| |delta|max
-    // (only the fused kernel uses it: it prunes per ray by distance)
-    float t_lo = -INFINITY;
-    if (WITH_T_LO) {
-        const float gn = (float)sqrt(d3dot(gd, gd)) - wn * tr.dl_max;
-        if (gn > 0.0f) t_lo = __double2float_rd(tc - (double)((eb + 1.7320509f) / gn) * 1.000001);
-    }
-    rec[4] = make_float4(g0.w, __int_as_float(s), band, t_lo);
+    // u_c rounded first: e0 then refers exactly to the point o + u_c D0 that the record's u_c names
+    const float ucf = (float)(d3dot(v, tr.D0) * tr.inv_D0D0);
+    const double uc = ucf;
     const d3 op = Wmul(d3make(-v.x, -v.y, -v.z));
     const d3 G0 = Wmul(tr.D0);
     const d3 Gx = Wmul(d3make(cam.R[0], cam.R[3], cam.R[6]));
     const d3 Gy = Wmul(d3make(cam.R[1], cam.R[4], cam.R[7]));
+    const d3 e0 = d3make(op.x + uc * G0.x, op.y + uc * G0.y, op.z + uc * G0.z);
+    // error band of q (DESIGN.md §4): eb >= |e| = |e0 + u_c h| for every ray of the tile, h = a Gx + b Gy
+    const float hb = tr.a_max * sqrtf((float)d3dot(Gx, Gx)) + tr.b_max * sqrtf((float)d3dot(Gy, Gy));   // >= |h|
+    const float eb = (float)sqrt(d3dot(e0, e0)) + fabsf(ucf) * hb;
+    const float band = 4e-6f * (3.0f + eb * eb);
+    rec[0] = make_float4((float)G0.x, (float)G0.y, (float)G0.z, (float)Gx.x);
+    rec[1] = make_float4((float)Gx.y, (float)Gx.z, (float)Gy.x, (float)Gy.y);
+    rec[2] = make_float4((float)Gy.z, (float)e0.x, (float)e0.y, (float)e0.z);
+    rec[3] = make_float4(ucf, g0.w, __int_as_float(s), band);
+    // t1 = L (u_c + sigma) with |sigma| <= (|e| + sqrt 3) / |G0 + h|, |e| <= eb and |G0 + h| >= |G0| - hb
+    if (WITH_T_LO) {
+        t_lo = -INFINITY;
+        const float gn = sqrtf((float)d3dot(G0, G0)) - hb;
+        if (gn > 0.0f) {
+            const double u_lo = uc - (double)((eb + 1.7320509f) / gn) * 1.000001;
+            t_lo = __double2float_rd(u_lo * (u_lo >= 0.0 ? tr.L_lo : tr.L_hi));
+        }
+    }
     const d3 M0 = d3cross(op, G0), Mx = d3cross(op, Gx), My = d3cross(op, Gy);
     const double lim = 3.0 + (double)band;
     const double m00 = d3dot(M0, M0), m0x = d3dot(M0, Mx), m0y = d3dot(M0, My), mxx = d3dot(Mx, Mx),
@@ -570,8 +592,8 @@ __device__ __forceinline__ bool coarse_test(const float (&p)[6], float pa, float
     return fmaf(pa, ta, fmaf(pb, tb, p[0])) < 0.0f;
 }
 
-// The precise per-ray test of one staged candidate (float32 relative to the tile-centre ray, decisions
-// within the band re-evaluated in float64): hit?, entry distance t1, alpha = opacity * exp(-q).
+// The precise per-ray test of staged candidate c (float32 in the tile's pixel basis, decisions within the band
+// re-evaluated in float64): hit?, entry distance t1, alpha = opacity * exp(-q).
 struct PreciseHit {
     bool hit;
     float t1, alpha;
@@ -579,34 +601,35 @@ struct PreciseHit {
     bool refined;
 };
 
-__device__ __forceinline__ PreciseHit precise_test(const RenderParams& P, const float4* rc, float dlx, float dly,
-                                                   float dlz, int pi, int pj) {
-    const float4 r0 = rc[0], r1 = rc[1], r2 = rc[2], r3 = rc[3], ax = rc[4];
-    const float wx = r0.x * dlx + r0.y * dly + r0.z * dlz;
-    const float wy = r0.w * dlx + r1.x * dly + r1.y * dlz;
-    const float wz = r1.z * dlx + r1.w * dly + r2.x * dlz;
-    const float tc = r3.w;
-    const float dx = r3.x + wx, dy = r3.y + wy, dz = r3.z + wz;                 // d' = W d
-    const float ex = r2.y + tc * wx, ey = r2.z + tc * wy, ez = r2.w + tc * wz;  // W (r(tc) - p)
+__device__ __forceinline__ PreciseHit precise_test(const RenderParams& P, const StagedRecords& rec, int c,
+                                                   const TileRays& tr, int pi, int pj) {
+    const float4 r0 = rec[0][c], r1 = rec[1][c], r2 = rec[2][c], r3 = rec[3][c];
+    const float hx = fmaf(tr.pb, r1.z, tr.pa * r0.w);   // h = a Gx + b Gy
+    const float hy = fmaf(tr.pb, r1.w, tr.pa * r1.x);
+    const float hz = fmaf(tr.pb, r2.x, tr.pa * r1.y);
+    const float uc = r3.x;
+    const float dx = r0.x + hx, dy = r0.y + hy, dz = r0.z + hz;                 // d' = W D(a,b) = G0 + h
+    const float ex = fmaf(uc, hx, r2.y), ey = fmaf(uc, hy, r2.z), ez = fmaf(uc, hz, r2.w);   // W (o + u_c D - p)
     const float A = dx * dx + dy * dy + dz * dz;
     const float Bh = ex * dx + ey * dy + ez * dz;
     const float mx = ey * dz - ez * dy, my = ez * dx - ex * dz, mz = ex * dy - ey * dx;
     const float iA = rcp_approx(A);
-    float q = (mx * mx + my * my + mz * mz) * iA;   // min Mahalanobis^2 along the ray
-    // tau = -Bh/A - sqrt((3 - q)/A)  (near root relative to tc)
-    const float tau = -Bh * iA - sqrt_approx(fmaxf(3.0f - q, 0.0f) * iA);
+    float q = (mx * mx + my * my + mz * mz) * iA;   // min Mahalanobis^2 along the ray (independent of |d'|)
+    // sigma = -Bh/A - sqrt((3 - q)/A): near root in u relative to u_c;  t1 = L u_c + L sigma
+    const float tc = tr.L * uc;
+    const float tau = tr.L * (-Bh * iA - sqrt_approx(fmaxf(3.0f - q, 0.0f) * iA));
     PreciseHit h;
     h.t1 = tc + tau;
-    h.s = __float_as_int(ax.y);
+    h.s = __float_as_int(r3.z);
     h.hit = (q < 3.0f) && (h.t1 > 0.0f);
     h.refined = false;
-    const bool near_q = fabsf(q - 3.0f) < ax.z;
+    const bool near_q = fabsf(q - 3.0f) < r3.w;
     // t1 = tc + tau loses its float32 accuracy where the two terms cancel (a camera just outside a large ellipsoid:
     // tc = 0.5, tau = -0.4992 - two such hits 5e-8 apart were composited in the wrong order).  Where the entry
     // distance is smaller than |tau| it is taken from the float64 evaluation, so that every kept distance is accurate
-    // relative to ITSELF and the relative tie bands of the k-buffer hold (elsewhere its error is <= 6e-7 t1).
+    // relative to ITSELF and the relative tie bands of the k-buffer hold (elsewhere its error is <= 7e-7 t1).
     // Distances that are negative beyond rounding - the camera inside the ellipsoid - are misses either way.
-    const bool near_t = (q < 3.0f + ax.z) && h.t1 > -2e-6f * (fabsf(tc) + fabsf(tau)) && h.t1 < fabsf(tau);
+    const bool near_t = (q < 3.0f + r3.w) && h.t1 > -2e-6f * (fabsf(tc) + fabsf(tau)) && h.t1 < fabsf(tau);
     if (near_q || near_t) {
         const ExactHit e = exact_eval(P.raw, P.cam, h.s, pi, pj);
         h.hit = e.hit && (e.t1 > 0.0);
@@ -614,7 +637,7 @@ __device__ __forceinline__ PreciseHit precise_test(const RenderParams& P, const 
         h.t1 = (float)e.t1;
         h.refined = true;
     }
-    h.alpha = ax.x * __expf(-q);   // opacity * exp(-q)  (gaussian.py:197-198)
+    h.alpha = r3.y * __expf(-q);   // opacity * exp(-q)  (gaussian.py:197-198)
     return h;
 }
 
@@ -692,9 +715,14 @@ __device__ __forceinline__ void store_tile(const RenderParams& P, float* ob, int
     __syncwarp();
     const int pitch = P.full_pitch ? P.cam.H : P.h;
     const int bi = P.full_pitch ? 0 : P.x0, bj = P.full_pitch ? 0 : P.y0;
+    // The lane is read again here: the row / column values below depend on nothing else, so when they are derived
+    // from `lane` the compiler hoists all nine out of the persistent tile loops and keeps them live - spilled to local
+    // memory - across every tile.  A volatile read is not hoisted; they cost a few integer operations per tile.
+    int ln;
+    asm volatile("mov.u32 %0, %%laneid;" : "=r"(ln));
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
-        const int f = r * 32 + lane;
+        const int f = r * 32 + ln;
         const int row = f / (3 * TILE_J), col = f % (3 * TILE_J);
         const int qi = i0 + row, qj = j0 + col / 3;
         if (qi < xe && qj < ye) {

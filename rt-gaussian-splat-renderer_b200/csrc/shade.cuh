@@ -8,11 +8,12 @@
 // A warp owns one tile at a time (lane = pixel) and walks the tile's candidate list, 31 candidates (one
 // 128-byte chunk) per batch:
 //   stage    one lane per candidate, float64: origin shifted to the closest point of the tile's centre
-//            ray -> a 80-byte float32 record + a 6-coefficient quadratic in shared memory;
+//            ray -> a 64-byte float32 record in the camera's pixel basis + a 6-coefficient quadratic in shared
+//            memory;
 //   coarse   every lane evaluates every staged quadratic (broadcast shared-memory reads, 5 FMA) and
 //            keeps a 32-bit mask of the candidates its ray may hit;
 //   precise  warp-wide rounds, each lane takes the next set bit of its mask: exact decision (float32
-//            in the tile-centred frame, float64 from the raw parameters inside the error band), entry
+//            linear in the pixel offset, float64 from the raw parameters inside the error band), entry
 //            distance, alpha; the hit goes to the lane's K-entry buffer in shared memory (replace-max
 //            once K are held; the nearest hit left outside is remembered, and if it is within float32
 //            rounding of the farthest kept entry the two are compared in float64 after the list).
@@ -24,7 +25,7 @@
 // evaluation of the reference's maths, see DESIGN.md §2.
 //
 // The code is bound by the L1 data pipe (per-lane gathers of SH and staged records), not by latency:
-// 20 warps x 96 registers per SM is the measured optimum, 9.25 KB of shared memory per warp.
+// 20 warps x 96 registers per SM is the measured optimum, 9.0 KB of shared memory per warp (9232 bytes).
 #pragma once
 #include "kbuffer.cuh"
 
@@ -43,11 +44,10 @@ namespace rtgs_dev {
 #endif
 constexpr int SHADE_K = 16;          // k-buffer entries (depth <= 16)
 constexpr float TIE_BAND = 2e-6f;    // relative: float32 entry distances closer than this are compared in float64
-constexpr int SHADE_BATCH = 32;      // staged candidates per batch (a chunk fills 31)
-constexpr int SHADE_REC_Q = 5;       // quads per staged record (80-byte stride: conflict-free gathers)
+constexpr int SHADE_BATCH = REC_BATCH;   // staged candidates per batch (a chunk fills 31)
 
 struct __align__(16) ShadeShared {
-    float4 rec[SHADE_BATCH][SHADE_REC_Q];  // precise records
+    StagedRecords rec;                     // precise records; the output staging of store_tile
     float4 polyA[SHADE_BATCH];             // coarse quadratics {c0 c1 c2 c3}
     float2 polyB[SHADE_BATCH];             //                   {c4 c5}
     float kb_t[SHADE_K][32];               // per-lane hit buffer (unsorted): entry distance, sorted position, alpha
@@ -106,11 +106,11 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
             // ---- stage ---------------------------------------------------------------------
             const int m4 = (m + 3) & ~3;
             if (lane < m) {
-                float4 rec[5];
-                float poly[6];
-                stage_candidate(P, tr, s, rec, poly);
+                float4 rec[REC_QUADS];
+                float poly[6], t_lo;
+                stage_candidate(P, tr, s, rec, poly, t_lo);
 #pragma unroll
-                for (int k = 0; k < 5; ++k) ws.rec[lane][k] = rec[k];
+                for (int k = 0; k < REC_QUADS; ++k) ws.rec[k][lane] = rec[k];
                 ws.polyA[lane] = make_float4(poly[0], poly[1], poly[2], poly[3]);
                 ws.polyB[lane] = make_float2(poly[4], poly[5]);
             } else if (lane < m4) {   // pad to a multiple of 4: never a candidate
@@ -143,7 +143,7 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
                 if (mask != 0) {
                     const int c = __ffs(mask) - 1;
                     mask &= mask - 1;
-                    const PreciseHit h = precise_test(P, ws.rec[c], tr.dlx, tr.dly, tr.dlz, pi, pj);
+                    const PreciseHit h = precise_test(P, ws.rec, c, tr, pi, pj);
                     ST(S.st_f64 += h.refined);
                     if (h.hit) {
                         float xt = h.t1, xa = h.alpha;   // the hit that stays outside the buffer (full buffer)
@@ -260,7 +260,9 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
     int nl = 0;
     if (maxcnt > 0) {
         float Y[15];
-        sh_basis(tr.dnx, tr.dny, tr.dnz, Y);
+        float dx, dy, dz;
+        sh_direction(cam, i0, j0, pi, pj, active, dx, dy, dz);
+        sh_basis(dx, dy, dz, Y);
         const int nmine = min(cnt, P.depth);
 #if SHADE_SLOT_ORDER
         // Weights first: w_k = T_k alpha_k depends on the alphas and their depth order only, so the ordered pass
