@@ -157,6 +157,20 @@ int rtgs_render(rtgs_scene* s, const rtgs_camera* cam,
                 int32_t depth, float t_cut, int32_t accumulate, int32_t full_image_pitch,
                 float* out_rgb, float* out_T, void* stream, rtgs_render_stats* stats);
 
+/* rtgs_render plus a depth image.  out_depth: device float32, indexed like out_T (region or full-image pitch,
+ * RTGS_OPT_STRIPE stripes), ACCUMULATED (+=) with accumulate != 0 like out_rgb; NULL makes the call rtgs_render.
+ * For each pixel D = sum_k T_k alpha_k t*_k over the layers the colour composites (same list, order and t_cut stop),
+ * where t*_k = (p - o)^T W^T W d / |W d|^2 is the ray parameter of the point where layer k's Gaussian responds most
+ * along the ray (o, d) (W = local_frame as rendered; for a hit t* > t1 > 0).  D is not normalised: the expected depth
+ * is D / (1 - T).  Units are those of d: camera rays have |d| = |q_cam|^2, so for a unit camera quaternion t* is the
+ * Euclidean distance from the camera centre along the ray; the camera-space z depth of pixel (i, j) is
+ * t* / sqrt(px^2 + py^2 + 1) (px, py as in rtgs_render_backward_camera).  RGB and T are bit-identical to rtgs_render's,
+ * and every render mode gives the same D bit for bit. */
+int rtgs_render_depth(rtgs_scene* s, const rtgs_camera* cam,
+                      int32_t x0, int32_t y0, int32_t w, int32_t h,
+                      int32_t depth, float t_cut, int32_t accumulate, int32_t full_image_pitch,
+                      float* out_rgb, float* out_T, float* out_depth, void* stream, rtgs_render_stats* stats);
+
 /* Replace the stored parameters of a scene (same n, same SH presence) from DEVICE pointers on the scene's device
  * (layouts of rtgs_scene_create; sh NULL iff the scene has none; values must be finite), then the caller calls
  * rtgs_scene_build_bvh.  Renders/backward before the rebuild fail with RTGS_ERR_STATE.  The copies are ordered after
@@ -193,6 +207,17 @@ int rtgs_render_backward_camera(rtgs_scene* s, const rtgs_camera* cam, int32_t x
                                 float* grad_opacity, float* grad_sh,
                                 float* grad_cam_pos, float* grad_cam_rot, float* grad_cam_focal,
                                 float* replay_rgb, float* replay_T, void* stream);
+
+/* rtgs_render_backward_camera plus the depth image of rtgs_render_depth: dL_dD (w,h) device or NULL, its gradient
+ * flows to the Gaussians and the camera like dL_drgb's; replay_depth (w,h) or NULL receives the depth the backward
+ * recomputed in float64.  With both NULL the call is rtgs_render_backward_camera (the same kernels). */
+int rtgs_render_backward_depth(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                               int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                               float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                               float* grad_opacity, float* grad_sh,
+                               float* grad_cam_pos, float* grad_cam_rot, float* grad_cam_focal,
+                               float* replay_rgb, float* replay_T, const float* dL_dD, float* replay_depth,
+                               void* stream);
 
 /* Tuning knobs of one scene's render path (no reference counterpart; defaults need no call).
  *  RTGS_OPT_RENDER_MODE      0 (default): k_tile_lists (traversal, one candidate list per 4x8-pixel tile) +
@@ -366,6 +391,12 @@ int rtgs_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays,
 int rtgs_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
                      float* out_rgb, float* out_T, void* stream);
 
+/* rtgs_render_rays plus out_depth (nrays) device or NULL (then the call is rtgs_render_rays): D of rtgs_render_depth
+ * for each ray, t* in units of the ray's own d, float64 per ray.  A t* may lie beyond the ray's `end`; a degenerate
+ * ray gets D = 0.  RGB and T are bit-identical to rtgs_render_rays's. */
+int rtgs_render_rays_depth(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                           float* out_rgb, float* out_T, float* out_depth, void* stream);
+
 /* Backward of rtgs_render_rays with each ray's layer list and t_cut stop held fixed (the definition of
  * rtgs_render_backward).  dL_drgb (nrays,3) and dL_dT (nrays, or NULL) are device buffers.  The Gaussian gradients
  * are ACCUMULATED as in rtgs_render_backward (any may be NULL).  grad_rays (nrays,8) or NULL is ACCUMULATED too:
@@ -377,6 +408,16 @@ int rtgs_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, i
                               float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
                               float* grad_opacity, float* grad_sh, float* grad_rays,
                               float* replay_rgb, float* replay_T, void* stream);
+
+/* rtgs_render_rays_backward plus dL_dD (nrays) device or NULL, the gradient of rtgs_render_rays_depth's depth, which
+ * flows to the Gaussians and to grad_rays like dL_drgb's, and replay_depth (nrays) or NULL, bit-identical to
+ * rtgs_render_rays_depth's out_depth.  With both NULL the call is rtgs_render_rays_backward (the same kernels). */
+int rtgs_render_rays_backward_depth(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                                    const float* dL_drgb, const float* dL_dT,
+                                    float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                                    float* grad_opacity, float* grad_sh, float* grad_rays,
+                                    float* replay_rgb, float* replay_T, const float* dL_dD, float* replay_depth,
+                                    void* stream);
 
 int rtgs_scene_destroy(rtgs_scene* s);
 

@@ -452,20 +452,28 @@ int rtgs_scene_read_gaussians(rtgs_scene* s, float* pos, float* rot_xyzw, float*
 int rtgs_render(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h, int32_t depth,
                 float t_cut, int32_t accumulate, int32_t full_image_pitch, float* out_rgb, float* out_T, void* stream,
                 rtgs_render_stats* stats) {
+    return rtgs_render_depth(s, cam, x0, y0, w, h, depth, t_cut, accumulate, full_image_pitch, out_rgb, out_T, nullptr,
+                             stream, stats);
+}
+
+int rtgs_render_depth(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                      int32_t depth, float t_cut, int32_t accumulate, int32_t full_image_pitch, float* out_rgb,
+                      float* out_T, float* out_depth, void* stream, rtgs_render_stats* stats) {
     RTGS_CHECK_ARG(s != nullptr);
     TRY(check_camera(cam));
     RTGS_CHECK_ARG(out_rgb != nullptr);
+    RTGS_CHECK_ARG(aligned(out_depth, 4));
     RTGS_CHECK_ARG(w > 0 && h > 0 && x0 >= 0 && y0 >= 0 && x0 + w <= cam->width && y0 + h <= cam->height);
     RTGS_CHECK_ARG(depth >= 1 && depth <= RTGS_MAX_DEPTH);
     RTGS_CHECK_ARG(t_cut >= 0.0f && t_cut < 1.0f);
     if (!s->built) {
-        rtgs_set_error("rtgs_render: call rtgs_scene_build_bvh first");
+        rtgs_set_error("%s: call rtgs_scene_build_bvh first", out_depth ? "rtgs_render_depth" : "rtgs_render");
         return RTGS_ERR_STATE;
     }
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
-    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, accumulate, full_image_pitch, out_rgb, out_T, st,
-                           stats != nullptr));
+    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, accumulate, full_image_pitch, out_rgb, out_T, out_depth,
+                           st, stats != nullptr));
     if (stats) {
         unsigned long long hs[32];
         CUDA_TRY(cudaMemcpyAsync(hs, s->stats_dev, sizeof(hs), cudaMemcpyDeviceToHost, st));
@@ -514,11 +522,12 @@ int rtgs_scene_set_gaussians_device(rtgs_scene* s, const float* pos, const float
 
 static int render_backward(const char* name, rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0,
                            int32_t w, int32_t h, int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
-                           float* const grads[6], float* const cam_grads[3], float* replay_rgb, float* replay_T,
-                           void* stream) {
+                           const float* dL_dD, float* const grads[6], float* const cam_grads[3], float* replay_rgb,
+                           float* replay_T, float* replay_depth, void* stream) {
     RTGS_CHECK_ARG(s != nullptr);
     TRY(check_camera(cam));
     RTGS_CHECK_ARG(dL_drgb != nullptr);
+    RTGS_CHECK_ARG(aligned(dL_dD, 4) && aligned(replay_depth, 4));
     RTGS_CHECK_ARG(w > 0 && h > 0 && x0 >= 0 && y0 >= 0 && x0 + w <= cam->width && y0 + h <= cam->height);
     RTGS_CHECK_ARG(depth >= 1 && depth <= RTGS_MAX_DEPTH);
     RTGS_CHECK_ARG(t_cut >= 0.0f && t_cut < 1.0f);
@@ -527,8 +536,8 @@ static int render_backward(const char* name, rtgs_scene* s, const rtgs_camera* c
         return RTGS_ERR_STATE;
     }
     DeviceGuard g(s->device);
-    return rtgs_launch_render_backward(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads, cam_grads,
-                                       replay_rgb, replay_T, (cudaStream_t)stream);
+    return rtgs_launch_render_backward(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, dL_dD, grads, cam_grads,
+                                       replay_rgb, replay_T, replay_depth, (cudaStream_t)stream);
 }
 
 int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
@@ -537,8 +546,8 @@ int rtgs_render_backward(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int3
                          float* replay_rgb, float* replay_T, void* stream) {
     float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
     float* const cam_grads[3] = {nullptr, nullptr, nullptr};
-    return render_backward("rtgs_render_backward", s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads,
-                           cam_grads, replay_rgb, replay_T, stream);
+    return render_backward("rtgs_render_backward", s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, nullptr, grads,
+                           cam_grads, replay_rgb, replay_T, nullptr, stream);
 }
 
 int rtgs_render_backward_camera(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
@@ -546,10 +555,23 @@ int rtgs_render_backward_camera(rtgs_scene* s, const rtgs_camera* cam, int32_t x
                                 float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
                                 float* grad_opacity, float* grad_sh, float* grad_cam_pos, float* grad_cam_rot,
                                 float* grad_cam_focal, float* replay_rgb, float* replay_T, void* stream) {
+    return rtgs_render_backward_depth(s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grad_pos, grad_rot,
+                                      grad_scale, grad_color, grad_opacity, grad_sh, grad_cam_pos, grad_cam_rot,
+                                      grad_cam_focal, replay_rgb, replay_T, nullptr, nullptr, stream);
+}
+
+int rtgs_render_backward_depth(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t y0, int32_t w, int32_t h,
+                               int32_t depth, float t_cut, const float* dL_drgb, const float* dL_dT,
+                               float* grad_pos, float* grad_rot, float* grad_scale, float* grad_color,
+                               float* grad_opacity, float* grad_sh, float* grad_cam_pos, float* grad_cam_rot,
+                               float* grad_cam_focal, float* replay_rgb, float* replay_T, const float* dL_dD,
+                               float* replay_depth, void* stream) {
     float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
     float* const cam_grads[3] = {grad_cam_pos, grad_cam_rot, grad_cam_focal};
-    return render_backward("rtgs_render_backward_camera", s, cam, x0, y0, w, h, depth, t_cut, dL_drgb, dL_dT, grads,
-                           cam_grads, replay_rgb, replay_T, stream);
+    const bool with_depth = dL_dD != nullptr || replay_depth != nullptr;
+    return render_backward(with_depth ? "rtgs_render_backward_depth" : "rtgs_render_backward_camera", s, cam, x0, y0,
+                           w, h, depth, t_cut, dL_drgb, dL_dT, dL_dD, grads, cam_grads, replay_rgb, replay_T,
+                           replay_depth, stream);
 }
 
 int rtgs_scene_set_option(rtgs_scene* s, int32_t option, int64_t value) {
@@ -849,7 +871,7 @@ static int submit_banded(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int3
     s->band_schedule = sched;
     s->band_flags_cur_dev = hs.flags_dev;
     const int r = rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb,
-                                     host_T ? hs.stage_T : nullptr, s->own_stream, false);
+                                     host_T ? hs.stage_T : nullptr, nullptr, s->own_stream, false);
     s->bands_active = 0;
     s->band_flags_cur_dev = nullptr;
     if (r != RTGS_OK) return r;
@@ -929,8 +951,8 @@ static int submit_whole(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32
     // head of frame f+1 overlaps the tail of frame f on the device
     static const bool one_stream = getenv("RTGS_SUBMIT_ONE_STREAM") != nullptr;   // experiment: serialised renders
     cudaStream_t rs = (s->host_head == 0 || one_stream) ? s->own_stream : s->own_stream2;
-    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, rs,
-                           false));
+    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, nullptr,
+                           rs, false));
     CUDA_TRY(cudaEventRecord(hs.done, rs));
     CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, hs.done, 0));
     CUDA_TRY(cudaMemcpyAsync(host_rgb, hs.stage_rgb, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->copy_stream));
@@ -987,7 +1009,7 @@ int rtgs_render_host_submit_packed(rtgs_scene* s, const rtgs_camera* cam, int32_
         hs.stage_packed_pixels = px;
     }
     cudaStream_t rs = s->host_head == 0 ? s->own_stream : s->own_stream2;
-    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, nullptr, rs, false));
+    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, nullptr, nullptr, rs, false));
     TRY(rtgs_launch_pack_pixels(hs.stage_rgb, hs.stage_packed, (int64_t)px, format, rs));
     CUDA_TRY(cudaEventRecord(hs.done, rs));
     CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, hs.done, 0));
@@ -1029,7 +1051,7 @@ int rtgs_render_host(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t 
     const bool pinned = d_rgb != nullptr && (!host_T || d_T != nullptr);
     if (pinned && host_mode() == 1) {
         // zero-copy: the render kernel writes the framebuffer into mapped host memory
-        TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, d_rgb, d_T, st, false));
+        TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, d_rgb, d_T, nullptr, st, false));
         CUDA_TRY(cudaStreamSynchronize(st));
         return RTGS_OK;
     }
@@ -1039,8 +1061,8 @@ int rtgs_render_host(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t 
     }
     rtgs_scene::HostSlot& hs = s->host_slot[0];
     TRY(ensure_stage(hs, px));
-    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, st,
-                           false));
+    TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, nullptr,
+                           st, false));
     if (pinned) {
         CUDA_TRY(cudaMemcpyAsync(host_rgb, hs.stage_rgb, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (host_T) CUDA_TRY(cudaMemcpyAsync(host_T, hs.stage_T, px * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1129,33 +1151,51 @@ int rtgs_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, int32_t*
 
 int rtgs_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut, float* out_rgb,
                      float* out_T, void* stream) {
+    return rtgs_render_rays_depth(s, nrays, rays, depth, t_cut, out_rgb, out_T, nullptr, stream);
+}
+
+int rtgs_render_rays_depth(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                           float* out_rgb, float* out_T, float* out_depth, void* stream) {
     TRY(check_rays(s, nrays, rays, out_rgb, depth, t_cut));
-    RTGS_CHECK_ARG(aligned(out_T, 4));
+    RTGS_CHECK_ARG(aligned(out_T, 4) && aligned(out_depth, 4));
     if (!s->built) {
-        rtgs_set_error("rtgs_render_rays: call rtgs_scene_build_bvh first");
+        rtgs_set_error("%s: call rtgs_scene_build_bvh first", out_depth ? "rtgs_render_rays_depth" : "rtgs_render_rays");
         return RTGS_ERR_STATE;
     }
     if (nrays == 0) return RTGS_OK;
     DeviceGuard g(s->device);
-    return rtgs_launch_render_rays(s, nrays, rays, depth, t_cut, out_rgb, out_T, (cudaStream_t)stream);
+    return rtgs_launch_render_rays(s, nrays, rays, depth, t_cut, out_rgb, out_T, out_depth, (cudaStream_t)stream);
 }
 
 int rtgs_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
                               const float* dL_drgb, const float* dL_dT, float* grad_pos, float* grad_rot,
                               float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
                               float* grad_rays, float* replay_rgb, float* replay_T, void* stream) {
+    return rtgs_render_rays_backward_depth(s, nrays, rays, depth, t_cut, dL_drgb, dL_dT, grad_pos, grad_rot,
+                                           grad_scale, grad_color, grad_opacity, grad_sh, grad_rays, replay_rgb,
+                                           replay_T, nullptr, nullptr, stream);
+}
+
+int rtgs_render_rays_backward_depth(rtgs_scene* s, int64_t nrays, const float* rays, int32_t depth, float t_cut,
+                                    const float* dL_drgb, const float* dL_dT, float* grad_pos, float* grad_rot,
+                                    float* grad_scale, float* grad_color, float* grad_opacity, float* grad_sh,
+                                    float* grad_rays, float* replay_rgb, float* replay_T, const float* dL_dD,
+                                    float* replay_depth, void* stream) {
     TRY(check_rays(s, nrays, rays, dL_drgb, depth, t_cut));
     float* const grads[6] = {grad_pos, grad_rot, grad_scale, grad_color, grad_opacity, grad_sh};
     for (const float* p : grads) RTGS_CHECK_ARG(aligned(p, 4));
     RTGS_CHECK_ARG(aligned(dL_dT, 4) && aligned(grad_rays, 4) && aligned(replay_rgb, 4) && aligned(replay_T, 4));
+    RTGS_CHECK_ARG(aligned(dL_dD, 4) && aligned(replay_depth, 4));
+    const bool with_depth = dL_dD != nullptr || replay_depth != nullptr;
     if (!s->built) {
-        rtgs_set_error("rtgs_render_rays_backward: call rtgs_scene_build_bvh first");
+        rtgs_set_error("%s: call rtgs_scene_build_bvh first",
+                       with_depth ? "rtgs_render_rays_backward_depth" : "rtgs_render_rays_backward");
         return RTGS_ERR_STATE;
     }
     if (nrays == 0) return RTGS_OK;
     DeviceGuard g(s->device);
-    return rtgs_launch_render_rays_backward(s, nrays, rays, depth, t_cut, dL_drgb, dL_dT, grads, grad_rays,
-                                            replay_rgb, replay_T, (cudaStream_t)stream);
+    return rtgs_launch_render_rays_backward(s, nrays, rays, depth, t_cut, dL_drgb, dL_dT, dL_dD, grads, grad_rays,
+                                            replay_rgb, replay_T, replay_depth, (cudaStream_t)stream);
 }
 
 int rtgs_scene_destroy(rtgs_scene* s) {

@@ -72,6 +72,9 @@ struct BackwardParams {
     const float* rays;           // (nrays, 8): o xyz, d xyz, start, end; 16-byte aligned
     int64_t nrays;
     float* g_rays;               // k_render_rays_backward<true>: (nrays, 8), columns 0-5 accumulated
+    // DEPTH instantiations (DESIGN.md §12): D = sum_k T_k alpha_k t*_k, t*_k = -sigma_k; indexed like dL_dT / replay_T
+    const float* dL_dD;          // or null (no depth gradient)
+    float* replay_depth;         // or null
 };
 
 // sh_basis (render_common.cuh) in float64: gaussian.py:149-163, incl. the `5z^2 - 3z` term at :160 as coded
@@ -135,6 +138,8 @@ struct Layer {
     double e[3];      // W (x - p)
     double xp[3];     // x - p, x = o - sigma d: the max-response point
     double sig;       // sigma = u.v / |v|^2
+    double v[3];      // W d
+    double A;         // |v|^2
     double qm;        // |e|^2 = min Mahalanobis^2 along the ray
     double alpha;
     double ex;        // exp(-q)
@@ -164,6 +169,9 @@ __device__ __forceinline__ void eval_layer(const BackwardParams& P, int s, const
 #pragma unroll
     for (int k = 0; k < 3; ++k) L.e[k] = u[k] - sig * v[k];
     L.sig = sig;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) L.v[k] = v[k];
+    L.A = A;
     L.xp[0] = op[0] - sig * d.x;
     L.xp[1] = op[1] - sig * d.y;
     L.xp[2] = op[2] - sig * d.z;
@@ -273,7 +281,9 @@ __device__ __forceinline__ int walk_layers(const BackwardParams& P, const double
 }
 
 // Phase 2: the forward again over the cnt layers; kt[k] becomes T_k, Y the SH basis of d / |d|.  The image goes to
-// replay_rgb / replay_T[out] (each may be null); returns the number of layers composited under the t_cut rule.
+// replay_rgb / replay_T[out] (each may be null), with DEPTH the composited t* = -sigma to replay_depth[out]; returns
+// the number of layers composited under the t_cut rule.
+template <bool DEPTH = false>
 __device__ __forceinline__ int replay_layers(const BackwardParams& P, const double (&o)[3], const d3& d, int cnt,
                                              double (&kt)[RTGS_MAX_DEPTH], const int (&ks)[RTGS_MAX_DEPTH],
                                              int64_t out, double (&Y)[15]) {
@@ -281,7 +291,7 @@ __device__ __forceinline__ int replay_layers(const BackwardParams& P, const doub
         const double il = 1.0 / sqrt(d.x * d.x + d.y * d.y + d.z * d.z);
         sh_basis_d(d.x * il, d.y * il, d.z * il, Y);
     }
-    double T = 1.0, rgb[3] = {0.0, 0.0, 0.0};
+    double T = 1.0, rgb[3] = {0.0, 0.0, 0.0}, D = 0.0;
     float Tf = 1.0f;   // the forward's float32 transmittance decides the t_cut rule
     int L = 0;
     for (int k = 0; k < cnt; ++k) {
@@ -295,6 +305,7 @@ __device__ __forceinline__ int replay_layers(const BackwardParams& P, const doub
         rgb[0] += wgt * c[0];
         rgb[1] += wgt * c[1];
         rgb[2] += wgt * c[2];
+        if constexpr (DEPTH) D -= wgt * ly.sig;
         T *= 1.0 - ly.alpha;
         Tf *= 1.0f - (float)ly.alpha;
         L = k + 1;
@@ -305,17 +316,19 @@ __device__ __forceinline__ int replay_layers(const BackwardParams& P, const doub
         P.replay_rgb[out * 3 + 2] = (float)rgb[2];
     }
     if (P.replay_T != nullptr) P.replay_T[out] = (float)T;
+    if (DEPTH && P.replay_depth != nullptr) P.replay_depth[out] = (float)D;
     return L;
 }
 
 // Phase 3: back to front over the L composited layers (T_k in kt) from dL/drgb = gr and B = dL/dT, scattering the
 // Gaussian gradients.  RAY_GRAD also returns the ray's own gradient: gO = dL/do, gD = dL/dd including the SH colour's
-// dependence on d / |d| (gO, gD enter as zeros).
-template <bool RAY_GRAD>
+// dependence on d / |d| (gO, gD enter as zeros).  DEPTH adds dL/dD = gDep: t*_k enters like one more colour channel,
+// and through t* = -sigma, dL/dsigma_k = -T_k alpha_k gDep with dsigma/du = v / A, dsigma/dv = (e - sigma v) / A.
+template <bool RAY_GRAD, bool DEPTH = false>
 __device__ __forceinline__ void back_to_front(const BackwardParams& P, const double (&o)[3], const d3& d, int L,
                                               const double (&kt)[RTGS_MAX_DEPTH], const int (&ks)[RTGS_MAX_DEPTH],
                                               const double (&Y)[15], const double (&gr)[3], double B,
-                                              double (&gO)[3], double (&gD)[3]) {
+                                              double (&gO)[3], double (&gD)[3], double gDep = 0.0) {
     double gY[15];   // RAY_GRAD: dL/dY_j
     if constexpr (RAY_GRAD) {
 #pragma unroll
@@ -328,7 +341,8 @@ __device__ __forceinline__ void back_to_front(const BackwardParams& P, const dou
         double c[3];
         eval_colour_d(P, s, Y, c);
         const double Tk = kt[k], a = ly.alpha;
-        const double cg = c[0] * gr[0] + c[1] * gr[1] + c[2] * gr[2];
+        double cg = c[0] * gr[0] + c[1] * gr[1] + c[2] * gr[2];
+        if constexpr (DEPTH) cg -= ly.sig * gDep;
         const double dA = Tk * (cg - B);
         B = a * cg + (1.0 - a) * B;
         const double wgt = Tk * a;
@@ -350,25 +364,41 @@ __device__ __forceinline__ void back_to_front(const BackwardParams& P, const dou
         }
         red_add(P.g_opacity, g, ly.ex * dA);
         const double dq = -a * dA;
-        if (P.g_pos != nullptr) {
-            // dq/dp = -2 W^T e
+        // DEPTH: hu = dL/du = dL/dsigma v / A, hv = dL/dv = dL/dsigma (e - sigma v) / A
+        double hu[3], hv[3];
+        if constexpr (DEPTH) {
+            const double ds = -wgt * gDep / ly.A;
 #pragma unroll
-            for (int j = 0; j < 3; ++j)
-                red_add(P.g_pos, g * 3 + j,
-                        -2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]));
+            for (int i = 0; i < 3; ++i) {
+                hu[i] = ds * ly.v[i];
+                hv[i] = ds * (ly.e[i] - ly.sig * ly.v[i]);
+            }
+        }
+        if (P.g_pos != nullptr) {
+            // dq/dp = -2 W^T e;  du/dp = -W
+#pragma unroll
+            for (int j = 0; j < 3; ++j) {
+                double gp = -2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]);
+                if constexpr (DEPTH) gp -= ly.Wm[0][j] * hu[0] + ly.Wm[1][j] * hu[1] + ly.Wm[2][j] * hu[2];
+                red_add(P.g_pos, g * 3 + j, gp);
+            }
         }
         if constexpr (RAY_GRAD) {
-            // dq/do = 2 W^T e, dq/dd = -2 sigma W^T e
+            // dq/do = 2 W^T e, dq/dd = -2 sigma W^T e;  du/do = W, dv/dd = W
 #pragma unroll
             for (int j = 0; j < 3; ++j) {
                 const double wte = 2.0 * dq * (ly.Wm[0][j] * ly.e[0] + ly.Wm[1][j] * ly.e[1] + ly.Wm[2][j] * ly.e[2]);
                 gO[j] += wte;
                 gD[j] -= ly.sig * wte;
+                if constexpr (DEPTH) {
+                    gO[j] += ly.Wm[0][j] * hu[0] + ly.Wm[1][j] * hu[1] + ly.Wm[2][j] * hu[2];
+                    gD[j] += ly.Wm[0][j] * hv[0] + ly.Wm[1][j] * hv[1] + ly.Wm[2][j] * hv[2];
+                }
             }
             if (P.has_sh) sh_dot_d(P, s, wgt, gr, gY);
         }
         if (P.g_scale == nullptr && P.g_rot == nullptr) continue;
-        // G = dL/dW = 2 dq e (x - p)^T; W_kj = Rm[j][k] f_k with f_k = 1 / (s_k c^2)
+        // G = dL/dW = 2 dq e (x - p)^T (DEPTH: + hu (o - p)^T + hv d^T); W_kj = Rm[j][k] f_k with f_k = 1 / (s_k c^2)
         double GW[3];   // sum_j G_kj W_kj per row k
         double M[3][3]; // dL/dRm
         const double c2 = ly.q[0] * ly.q[0] + ly.q[1] * ly.q[1] + ly.q[2] * ly.q[2] + ly.q[3] * ly.q[3];
@@ -378,7 +408,8 @@ __device__ __forceinline__ void back_to_front(const BackwardParams& P, const dou
             GW[k2] = 0.0;
 #pragma unroll
             for (int j = 0; j < 3; ++j) {
-                const double G = 2.0 * dq * ly.e[k2] * ly.xp[j];
+                double G = 2.0 * dq * ly.e[k2] * ly.xp[j];
+                if constexpr (DEPTH) G += hu[k2] * (o[j] - ly.p[j]) + hv[k2] * (j == 0 ? d.x : j == 1 ? d.y : d.z);
                 GW[k2] += G * ly.Wm[k2][j];
                 M[j][k2] = G * f;
             }
@@ -411,8 +442,8 @@ __device__ __forceinline__ void back_to_front(const BackwardParams& P, const dou
 }
 
 // One pixel of k_render_backward; a pixel that contributes nothing returns early.  With CAM, its camera terms are
-// written to cam_g[CAM_TERMS] (left untouched, i.e. zero, on an early return).
-template <bool CAM>
+// written to cam_g[CAM_TERMS] (left untouched, i.e. zero, on an early return).  DEPTH: dL_dD and replay_depth.
+template <bool CAM, bool DEPTH>
 __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile, int lane, double* cam_g) {
     const int ti = tile / P.tiles_j, tj = tile - ti * P.tiles_j;
     const int li = ti * TILE_I + lane / TILE_J, lj = tj * TILE_J + lane % TILE_J;   // region-relative pixel
@@ -427,12 +458,13 @@ __device__ __forceinline__ void backward_pixel(const BackwardParams& P, int tile
     int ks[RTGS_MAX_DEPTH];
     const int cnt = walk_layers<false>(P, o, d, 0.0, INFINITY, kt, ks);
     double Y[15];
-    const int L = replay_layers(P, o, d, cnt, kt, ks, pix, Y);
+    const int L = replay_layers<DEPTH>(P, o, d, cnt, kt, ks, pix, Y);
     const double gr[3] = {P.dL_drgb[pix * 3 + 0], P.dL_drgb[pix * 3 + 1], P.dL_drgb[pix * 3 + 2]};
     const double B = P.dL_dT != nullptr ? (double)P.dL_dT[pix] : 0.0;
-    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
+    const double gDep = DEPTH && P.dL_dD != nullptr ? (double)P.dL_dD[pix] : 0.0;
+    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0 && gDep == 0.0) return;
     double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};   // CAM: dL/do, dL/dd
-    back_to_front<CAM>(P, o, d, L, kt, ks, Y, gr, B, gO, gD);
+    back_to_front<CAM, DEPTH>(P, o, d, L, kt, ks, Y, gr, B, gO, gD, gDep);
     if constexpr (CAM) {
         // d = Rm dc, dc = n / |n| as cam_dir computes them
         const double px = ((double)pi + 0.5 - 0.5 * (double)cam.W) * cam.ifx;
@@ -475,23 +507,24 @@ __device__ __forceinline__ void cam_block_reduce(const BackwardParams& P, double
 }
 
 // CAM = false: the Gaussian gradients.  CAM = true: also the camera's, as per-CTA partials in P.cam_part (finished
-// by k_camera_grad_finalize).
+// by k_camera_grad_finalize).  DEPTH: the depth terms as well (rtgs_render_backward_depth), at the occupancy of the
+// plain instantiation with the same CAM.
 // The minimum CTA counts hold both instantiations at their occupancy (128 registers: 4 CTAs per SM, 168: 3); left to
 // itself ptxas gives the CAM path 178 registers without spills, which fits only 2.
-template <bool CAM>
+template <bool CAM, bool DEPTH = false>
 __global__ void __launch_bounds__(BWD_WARPS * 32, CAM ? 3 : 4)
     k_render_backward(const __grid_constant__ BackwardParams P) {
     const int lane = threadIdx.x & 31;
     const int tile = blockIdx.x * BWD_WARPS + (threadIdx.x >> 5);
     if constexpr (!CAM) {
         if (tile >= P.ntiles) return;
-        backward_pixel<false>(P, tile, lane, nullptr);
+        backward_pixel<false, DEPTH>(P, tile, lane, nullptr);
     } else {
         // absent pixels and tiles contribute zeros: every lane reaches the shuffles and the barrier
         double cg[CAM_TERMS];
 #pragma unroll
         for (int i = 0; i < CAM_TERMS; ++i) cg[i] = 0.0;
-        if (tile < P.ntiles) backward_pixel<true>(P, tile, lane, cg);
+        if (tile < P.ntiles) backward_pixel<true, DEPTH>(P, tile, lane, cg);
         cam_block_reduce(P, cg);
     }
 }
@@ -551,8 +584,9 @@ __device__ __forceinline__ bool load_ray(const BackwardParams& P, int64_t r, dou
     return finite && (a.w != 0.0f || b.x != 0.0f || b.y != 0.0f) && b.z < b.w;
 }
 
-// Phases 1-2 per ray: float32 rgb to replay_rgb (n,3), T to replay_T (n) if not null.  The same code as the replay
-// of k_render_rays_backward, so the two agree bit for bit.
+// Phases 1-2 per ray: float32 rgb to replay_rgb (n,3), T to replay_T (n) if not null, with DEPTH the depth to
+// replay_depth (n) if not null.  The same code as the replay of k_render_rays_backward, so the two agree bit for bit.
+template <bool DEPTH = false>
 __global__ void __launch_bounds__(RAY_THREADS) k_render_rays(const __grid_constant__ BackwardParams P) {
     const int64_t r = blockIdx.x * (int64_t)RAY_THREADS + threadIdx.x;
     if (r >= P.nrays) return;
@@ -562,13 +596,13 @@ __global__ void __launch_bounds__(RAY_THREADS) k_render_rays(const __grid_consta
     int ks[RTGS_MAX_DEPTH];
     const int cnt = load_ray(P, r, o, d, t_start, t_end) ? walk_layers<true>(P, o, d, t_start, t_end, kt, ks) : 0;
     double Y[15];
-    replay_layers(P, o, d, cnt, kt, ks, r, Y);   // no layer: rgb 0, T 1
+    replay_layers<DEPTH>(P, o, d, cnt, kt, ks, r, Y);   // no layer: rgb 0, T 1, depth 0
 }
 
 // Phases 1-3 per ray.  RAY_GRAD = false: the Gaussian gradients only.  RAY_GRAD = true: also dL/do and dL/dd, added
 // by the ray's own thread to g_rays[r * 8 + 0..5] (no atomics: deterministic).
-// at the occupancy of the matching k_render_backward instantiation
-template <bool RAY_GRAD>
+// at the occupancy of the matching k_render_backward instantiation.  DEPTH: dL_dD and replay_depth.
+template <bool RAY_GRAD, bool DEPTH = false>
 __global__ void __launch_bounds__(RAY_THREADS, RAY_GRAD ? 3 : 4)
     k_render_rays_backward(const __grid_constant__ BackwardParams P) {
     const int64_t r = blockIdx.x * (int64_t)RAY_THREADS + threadIdx.x;
@@ -580,13 +614,14 @@ __global__ void __launch_bounds__(RAY_THREADS, RAY_GRAD ? 3 : 4)
     const bool valid = load_ray(P, r, o, d, t_start, t_end);
     const int cnt = valid ? walk_layers<true>(P, o, d, t_start, t_end, kt, ks) : 0;
     double Y[15];
-    const int L = replay_layers(P, o, d, cnt, kt, ks, r, Y);
+    const int L = replay_layers<DEPTH>(P, o, d, cnt, kt, ks, r, Y);
     if (!valid) return;
     const double gr[3] = {P.dL_drgb[r * 3 + 0], P.dL_drgb[r * 3 + 1], P.dL_drgb[r * 3 + 2]};
     const double B = P.dL_dT != nullptr ? (double)P.dL_dT[r] : 0.0;
-    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0) return;
+    const double gDep = DEPTH && P.dL_dD != nullptr ? (double)P.dL_dD[r] : 0.0;
+    if (gr[0] == 0.0 && gr[1] == 0.0 && gr[2] == 0.0 && B == 0.0 && gDep == 0.0) return;
     double gO[3] = {0.0, 0.0, 0.0}, gD[3] = {0.0, 0.0, 0.0};
-    back_to_front<RAY_GRAD>(P, o, d, L, kt, ks, Y, gr, B, gO, gD);
+    back_to_front<RAY_GRAD, DEPTH>(P, o, d, L, kt, ks, Y, gr, B, gO, gD, gDep);
     if constexpr (RAY_GRAD) {
         float* g = P.g_rays + r * 8;
 #pragma unroll

@@ -175,17 +175,18 @@ struct rtgs_scene {
 int rtgs_lbvh_build(rtgs_scene* s);   // lbvh.cu
 int rtgs_launch_render(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h,
                        int depth, float t_cut, int accumulate, int full_pitch, float* out_rgb,
-                       float* out_T, cudaStream_t stream, bool want_stats);  // render.cu
+                       float* out_T, float* out_depth, cudaStream_t stream, bool want_stats);  // render.cu
 int rtgs_heavy_lists_mode(const rtgs_scene* s);
 int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h, int depth,
-                                float t_cut, const float* dL_drgb, const float* dL_dT, float* const grads[6],
-                                float* const cam_grads[3], float* replay_rgb, float* replay_T,
-                                cudaStream_t stream);  // render.cu (backward.cuh)
+                                float t_cut, const float* dL_drgb, const float* dL_dT, const float* dL_dD,
+                                float* const grads[6], float* const cam_grads[3], float* replay_rgb, float* replay_T,
+                                float* replay_depth, cudaStream_t stream);  // render.cu (backward.cuh)
 int rtgs_launch_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut, float* out_rgb,
-                            float* out_T, cudaStream_t stream);  // render.cu (backward.cuh)
+                            float* out_T, float* out_depth, cudaStream_t stream);  // render.cu (backward.cuh)
 int rtgs_launch_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut,
-                                     const float* dL_drgb, const float* dL_dT, float* const grads[6], float* grad_rays,
-                                     float* replay_rgb, float* replay_T, cudaStream_t stream);
+                                     const float* dL_drgb, const float* dL_dT, const float* dL_dD,
+                                     float* const grads[6], float* grad_rays, float* replay_rgb, float* replay_T,
+                                     float* replay_depth, cudaStream_t stream);
 int rtgs_launch_generate_rays(const rtgs_camera* cam, float* rays, cudaStream_t stream);
 int rtgs_launch_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, int32_t* idx,
                               float* t12, cudaStream_t stream);

@@ -93,8 +93,9 @@ struct __align__(16) WarpShared {
 };
 
 // STATS = true compiles the per-render counters in (rtgs_render with a stats pointer); the timed path
-// uses STATS = false so that the 64-bit counters do not occupy registers.
-template <int K, bool STATS>
+// uses STATS = false so that the 64-bit counters do not occupy registers.  DEPTH = true also composites the ray
+// distance of every layer into P.out_depth (rtgs_render_depth; render_common.cuh: composite_depth).
+template <int K, bool STATS, bool DEPTH = false>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_render(const __grid_constant__ RenderParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     WarpShared<K>& ws = reinterpret_cast<WarpShared<K>*>(smem_raw)[threadIdx.x >> 5];
@@ -493,7 +494,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) maxcnt = max(maxcnt, __shfl_xor_sync(FULL, maxcnt, o));
         __syncwarp();
-        float T = 1.0f, cr = 0.0f, cg = 0.0f, cb = 0.0f;
+        float T = 1.0f, cr = 0.0f, cg = 0.0f, cb = 0.0f, D = 0.0f;
         int nl = 0;
         if constexpr (K == 16) {
             // ---- order the hits (bitonic network over register keys, near ties by float64: kbuffer.cuh) and composite
@@ -524,6 +525,13 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                     T *= 1.0f - alpha;
                     ++nl;
                 }
+            }
+            if constexpr (DEPTH) {
+                D = composite_depth(P, i0, j0, pi, pj, active, nmine, nloop, [&](int k, int& s, float& a) {
+                    const int slot = (int)((perm >> (4 * k)) & 15u);
+                    s = ws.kb_i[slot][lane];
+                    a = ws.kb_a[slot][lane];
+                });
             }
             __syncwarp();
         } else {
@@ -592,10 +600,16 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                         ++nl;
                     }
                 }
+                if constexpr (DEPTH) {
+                    D = composite_depth(P, i0, j0, pi, pj, active, nmine, nloop, [&](int k, int& s, float& a) {
+                        s = ws.c.so_i[k][lane];
+                        a = ws.c.so_a[k][lane];
+                    });
+                }
             }
         }
         grant_wait(P, grant);
-        store_tile(P, reinterpret_cast<float*>(&ws.kb_t[0][0]), lane, i0, j0, pi, pj, active, cr, cg, cb, T);
+        store_tile<DEPTH>(P, reinterpret_cast<float*>(&ws.kb_t[0][0]), lane, i0, j0, pi, pj, active, cr, cg, cb, T, D);
         tile_done(P, band_count, tile, lane);
         if (active) {
             ST(st_rays += 1);

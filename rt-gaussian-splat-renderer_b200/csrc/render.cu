@@ -187,7 +187,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, HEAVY_CTAS) k_heavy_lists(
 constexpr int SHADE_WARPS = K2_WARPS;   // warps per CTA
 static_assert(sizeof(ShadeShared) * K2_WARPS * K2_CTAS <= 227 * 1024, "shared-memory budget per SM");
 
-template <bool STATS>
+template <bool STATS, bool DEPTH = false>
 __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_shade_tiles(const __grid_constant__ RenderParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ShadeShared& ws = reinterpret_cast<ShadeShared*>(smem_raw)[threadIdx.x >> 5];
@@ -210,7 +210,7 @@ __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_shade_tiles(const
             tile_done(P, BC, tile, lane);
             continue;
         }
-        shade_tile<STATS>(P, ws, S, G, BC, tile, lane);
+        shade_tile<STATS, DEPTH>(P, ws, S, G, BC, tile, lane);
     }
     band_flush(P, BC, lane);
     flush_shade_stats<STATS>(P, S, lane);
@@ -223,7 +223,7 @@ union __align__(16) FrameShared {
 };
 static_assert(sizeof(FrameShared) * K2_WARPS * K2_CTAS <= 227 * 1024, "shared-memory budget per SM");
 
-template <bool STATS>
+template <bool STATS, bool DEPTH = false>
 __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_frame(const __grid_constant__ RenderParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     FrameShared& ws = reinterpret_cast<FrameShared*>(smem_raw)[threadIdx.x >> 5];
@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_frame(const __gri
                 }
             }
             __syncwarp();
-            shade_tile<STATS>(P, ws.shade, SS, G, BC, tile, lane);
+            shade_tile<STATS, DEPTH>(P, ws.shade, SS, G, BC, tile, lane);
             __syncwarp();
         }
     }
@@ -298,8 +298,8 @@ __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_frame(const __gri
             Q.use_fallback_list = 3;
             Q.final_kernel = 1;
             int grid = (int)min((fb + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (unsigned)P.tail_grid);
-            k_render<16, STATS><<<grid, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<16>) * WARPS_PER_CTA,
-                                  cudaStreamTailLaunch>>>(Q);
+            k_render<16, STATS, DEPTH><<<grid, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<16>) * WARPS_PER_CTA,
+                                         cudaStreamTailLaunch>>>(Q);
         } else
 #endif
         if (P.final_kernel) {
@@ -468,17 +468,17 @@ int persistent_blocks(rtgs_scene* s, Kernel kernel, int threads, size_t smem, in
     return RTGS_OK;
 }
 
-template <int K, bool STATS>
+template <int K, bool STATS, bool DEPTH>
 int prepare_render_k(rtgs_scene* s, int* blocks) {
     static int cache[16] = {0};
-    return persistent_blocks(s, k_render<K, STATS>, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<K>) * WARPS_PER_CTA,
+    return persistent_blocks(s, k_render<K, STATS, DEPTH>, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<K>) * WARPS_PER_CTA,
                              cache, "k_render", blocks);
 }
 
-template <int K, bool STATS>
+template <int K, bool STATS, bool DEPTH>
 int launch_render_k(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const RenderParams& P, cudaStream_t stream) {
     int nb = 0;
-    int r = prepare_render_k<K, STATS>(s, &nb);
+    int r = prepare_render_k<K, STATS, DEPTH>(s, &nb);
     if (r != RTGS_OK) return r;
     const size_t smem = sizeof(fused::WarpShared<K>) * WARPS_PER_CTA;
     int grid = s->sm_count * nb;
@@ -494,9 +494,14 @@ int launch_render_k(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const Ren
         if (!seen && grid > small) grid = small;
     }
     if (grid < 1) grid = 1;
-    k_render<K, STATS><<<grid, WARPS_PER_CTA * 32, smem, stream>>>(P);
+    k_render<K, STATS, DEPTH><<<grid, WARPS_PER_CTA * 32, smem, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
+}
+
+template <bool STATS, bool DEPTH>
+int launch_fused(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const RenderParams& P, cudaStream_t stream, int K) {
+    return K > 16 ? launch_render_k<32, STATS, DEPTH>(s, fs, P, stream) : launch_render_k<16, STATS, DEPTH>(s, fs, P, stream);
 }
 
 template <bool STATS>
@@ -544,12 +549,12 @@ int launch_heavy_lists(rtgs_scene* s, rtgs_scene::FrameScratch& fs, RenderParams
     return RTGS_OK;
 }
 
-template <bool STATS>
+template <bool STATS, bool DEPTH>
 int launch_shade_tiles(rtgs_scene* s, const RenderParams& P, cudaStream_t stream, bool dependent) {
     static int cache[16] = {0};
     const size_t smem = sizeof(ShadeShared) * SHADE_WARPS;
     int nb = 0;
-    int r = persistent_blocks(s, k_shade_tiles<STATS>, SHADE_WARPS * 32, smem, cache, "k_shade_tiles", &nb);
+    int r = persistent_blocks(s, k_shade_tiles<STATS, DEPTH>, SHADE_WARPS * 32, smem, cache, "k_shade_tiles", &nb);
     if (r != RTGS_OK) return r;
     int grid = s->sm_count * nb;
     const int need = (P.ntiles + SHADE_WARPS - 1) / SHADE_WARPS;
@@ -568,24 +573,24 @@ int launch_shade_tiles(rtgs_scene* s, const RenderParams& P, cudaStream_t stream
         at[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at;
         cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, k_shade_tiles<STATS>, P));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, k_shade_tiles<STATS, DEPTH>, P));
         return RTGS_OK;
     }
-    k_shade_tiles<STATS><<<grid, SHADE_WARPS * 32, smem, stream>>>(P);
+    k_shade_tiles<STATS, DEPTH><<<grid, SHADE_WARPS * 32, smem, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
 
-template <bool STATS>
+template <bool STATS, bool DEPTH>
 int launch_frame(rtgs_scene* s, RenderParams& P, cudaStream_t stream) {
     static int cache[16] = {0};
     const size_t smem = sizeof(FrameShared) * SHADE_WARPS;
     int nb = 0;
-    int r = persistent_blocks(s, k_frame<STATS>, SHADE_WARPS * 32, smem, cache, "k_frame", &nb);
+    int r = persistent_blocks(s, k_frame<STATS, DEPTH>, SHADE_WARPS * 32, smem, cache, "k_frame", &nb);
     if (r != RTGS_OK) return r;
     if (P.tail_launch) {   // the device-side launch of the fused kernel needs its shared memory opted in as well
         int nbk = 0;
-        if ((r = prepare_render_k<16, STATS>(s, &nbk)) != RTGS_OK) return r;
+        if ((r = prepare_render_k<16, STATS, DEPTH>(s, &nbk)) != RTGS_OK) return r;
         P.tail_grid = s->sm_count * nbk;
     }
     int grid = s->sm_count * nb;
@@ -593,7 +598,7 @@ int launch_frame(rtgs_scene* s, RenderParams& P, cudaStream_t stream) {
     const int need = (P.ntiles / TILES_PER_GROUP + SHADE_WARPS - 1) / SHADE_WARPS;
     if (grid > need) grid = need;
     if (grid < 1) grid = 1;
-    k_frame<STATS><<<grid, SHADE_WARPS * 32, smem, stream>>>(P);
+    k_frame<STATS, DEPTH><<<grid, SHADE_WARPS * 32, smem, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
@@ -685,7 +690,7 @@ int ensure_lists(rtgs_scene* s, rtgs_scene::FrameScratch& fs, int ntiles) {
 
 static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const rtgs_camera* cam, int x0, int y0, int w,
                             int h, int depth, float t_cut, int accumulate, int full_pitch, float* out_rgb,
-                            float* out_T, cudaStream_t stream, bool want_stats);
+                            float* out_T, float* out_depth, cudaStream_t stream, bool want_stats);
 
 // A frame's render scratch (work counters, candidate lists) is reused by later frames, which is safe in stream
 // order.  The scene has two scratch sets: a stream keeps the set it used last, a new stream takes the set that has
@@ -693,7 +698,7 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
 // wait for each other and overlap on the device; a third stream, or statistics / banded delivery (whose counters
 // exist once), are ordered behind what they share.
 int rtgs_launch_render(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h, int depth,
-                       float t_cut, int accumulate, int full_pitch, float* out_rgb, float* out_T,
+                       float t_cut, int accumulate, int full_pitch, float* out_rgb, float* out_T, float* out_depth,
                        cudaStream_t stream, bool want_stats) {
     const bool exclusive = want_stats || s->bands_active > 0;   // uses stats_dev / band_done: one frame at a time
     int pick = -1;
@@ -709,7 +714,7 @@ int rtgs_launch_render(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, in
     }
     s->exclusive_inflight = exclusive;
     const int r = launch_render_on(s, fs, cam, x0, y0, w, h, depth, t_cut, accumulate, full_pitch, out_rgb, out_T,
-                                   stream, want_stats);
+                                   out_depth, stream, want_stats);
     // the hand-over pointers apply to one frame
     s->sync_arrive = nullptr;
     s->sync_grant = nullptr;
@@ -726,7 +731,7 @@ int rtgs_launch_render(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, in
 
 static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const rtgs_camera* cam, int x0, int y0, int w,
                             int h, int depth, float t_cut, int accumulate, int full_pitch, float* out_rgb,
-                            float* out_T, cudaStream_t stream, bool want_stats) {
+                            float* out_T, float* out_depth, cudaStream_t stream, bool want_stats) {
     RenderParams P;
     P.nodes = s->nodes;
     P.nodes4 = s->nodes4;
@@ -794,6 +799,10 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     P.final_kernel = 0;
     P.self_clean = 0;
     P.tail_grid = 0;
+    P.out_depth = out_depth;
+    // out_depth selects the DEPTH instantiation of every kernel that composites; without it the frame runs the kernels
+    // of a plain render
+    const bool with_depth = out_depth != nullptr;
     if (s->bands_active > 0) {
         P.nbands = s->bands_active;
         P.band_macro_cols = s->band_macro_cols;
@@ -821,10 +830,11 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
         if (ev) CUDA_TRY(cudaEventRecord(ev[k], stream));
         return RTGS_OK;
     };
-    auto fused_kernel = [&](int K) -> int {
-        if (K > 16) return want_stats ? launch_render_k<32, true>(s, fs, P, stream) : launch_render_k<32, false>(s, fs, P, stream);
-        return want_stats ? launch_render_k<16, true>(s, fs, P, stream) : launch_render_k<16, false>(s, fs, P, stream);
-    };
+    // f<STATS, DEPTH>(...) for this frame's statistics and depth flags
+#define RTGS_BY_FLAGS(f, ...)                                                                                         \
+    (want_stats ? (with_depth ? f<true, true>(__VA_ARGS__) : f<true, false>(__VA_ARGS__))                               \
+                : (with_depth ? f<false, true>(__VA_ARGS__) : f<false, false>(__VA_ARGS__)))
+    auto fused_kernel = [&](int K) -> int { return RTGS_BY_FLAGS(launch_fused, s, fs, P, stream, K); };
     int r;
     if (mode == 1) {
         if ((r = mark(0)) != RTGS_OK || (r = mark(1)) != RTGS_OK || (r = mark(2)) != RTGS_OK) return r;
@@ -850,7 +860,7 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
         P.final_kernel = tail ? 1 : 0;
         P.self_clean = tail ? 1 : 0;
         if ((r = mark(0)) != RTGS_OK || (r = mark(1)) != RTGS_OK) return r;
-        if ((r = want_stats ? launch_frame<true>(s, P, stream) : launch_frame<false>(s, P, stream)) != RTGS_OK) return r;
+        if ((r = RTGS_BY_FLAGS(launch_frame, s, P, stream)) != RTGS_OK) return r;
         if ((r = mark(2)) != RTGS_OK) return r;
         if (ran) *ran = 2;
         if (!tail) {
@@ -890,12 +900,12 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     if (heavy_first) {
         P.use_fallback_list = 1;
         P.early_trigger = 1;
-        if ((r = launch_render_k<16, false>(s, fs, P, stream)) != RTGS_OK) return r;
+        if ((r = RTGS_BY_FLAGS(launch_fused, s, fs, P, stream, 16)) != RTGS_OK) return r;
         P.use_fallback_list = 0;
         P.early_trigger = 0;
-        if ((r = launch_shade_tiles<false>(s, P, stream, true)) != RTGS_OK) return r;
+        if ((r = RTGS_BY_FLAGS(launch_shade_tiles, s, P, stream, true)) != RTGS_OK) return r;
     } else {
-        if ((r = want_stats ? launch_shade_tiles<true>(s, P, stream, false) : launch_shade_tiles<false>(s, P, stream, false)) != RTGS_OK) return r;
+        if ((r = RTGS_BY_FLAGS(launch_shade_tiles, s, P, stream, false)) != RTGS_OK) return r;
     }
     if ((r = mark(2)) != RTGS_OK) return r;
     P.use_fallback_list = heavy_first ? 2 : 3;
@@ -906,6 +916,7 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     if ((r = fused_kernel(16)) != RTGS_OK) return r;
     if (ran) *ran = 7;
     return mark(3);
+#undef RTGS_BY_FLAGS
 }
 
 int rtgs_launch_generate_rays(const rtgs_camera* cam, float* rays, cudaStream_t stream) {
@@ -925,8 +936,9 @@ int rtgs_launch_trace_closest(rtgs_scene* s, int64_t nrays, const float* rays, i
 }
 
 int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, int y0, int w, int h, int depth,
-                                float t_cut, const float* dL_drgb, const float* dL_dT, float* const grads[6],
-                                float* const cam_grads[3], float* replay_rgb, float* replay_T, cudaStream_t stream) {
+                                float t_cut, const float* dL_drgb, const float* dL_dT, const float* dL_dD,
+                                float* const grads[6], float* const cam_grads[3], float* replay_rgb, float* replay_T,
+                                float* replay_depth, cudaStream_t stream) {
     backward::BackwardParams P;
     P.nodes = s->nodes;
     P.geo = s->geo;
@@ -945,16 +957,22 @@ int rtgs_launch_render_backward(rtgs_scene* s, const rtgs_camera* cam, int x0, i
     P.g_color = grads[3]; P.g_opacity = grads[4]; P.g_sh = s->has_sh ? grads[5] : nullptr;
     P.replay_rgb = replay_rgb;
     P.replay_T = replay_T;
+    P.dL_dD = dL_dD;
+    P.replay_depth = replay_depth;
     P.cam_part = nullptr;
+    // the DEPTH instantiations only when a depth pointer is given: otherwise the kernels of the plain backward
+    const bool with_depth = dL_dD != nullptr || replay_depth != nullptr;
     const int blocks = (P.ntiles + backward::BWD_WARPS - 1) / backward::BWD_WARPS;
     if (cam_grads[0] == nullptr && cam_grads[1] == nullptr && cam_grads[2] == nullptr) {
-        backward::k_render_backward<false><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+        if (with_depth) backward::k_render_backward<false, true><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+        else backward::k_render_backward<false><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
         CUDA_TRY(cudaGetLastError());
         return RTGS_OK;
     }
     // per-CTA partials of the camera gradient, stream-ordered: no scene scratch, safe for calls on several streams
     CUDA_TRY(cudaMallocAsync((void**)&P.cam_part, sizeof(double) * backward::CAM_TERMS * blocks, stream));
-    backward::k_render_backward<true><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+    if (with_depth) backward::k_render_backward<true, true><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
+    else backward::k_render_backward<true><<<blocks, backward::BWD_WARPS * 32, 0, stream>>>(P);
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) {
         backward::k_camera_grad_finalize<<<1, backward::FIN_THREADS, 0, stream>>>(P.cam_part, blocks, P.cam, cam_grads[0],
@@ -983,20 +1001,23 @@ static backward::BackwardParams rays_params(rtgs_scene* s, int64_t nrays, const 
 }
 
 int rtgs_launch_render_rays(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut, float* out_rgb,
-                            float* out_T, cudaStream_t stream) {
+                            float* out_T, float* out_depth, cudaStream_t stream) {
     if (nrays == 0) return RTGS_OK;
     backward::BackwardParams P = rays_params(s, nrays, rays, depth, t_cut);
     P.replay_rgb = out_rgb;
     P.replay_T = out_T;
+    P.replay_depth = out_depth;
     const unsigned blocks = (unsigned)((nrays + backward::RAY_THREADS - 1) / backward::RAY_THREADS);
-    backward::k_render_rays<<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    if (out_depth != nullptr) backward::k_render_rays<true><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    else backward::k_render_rays<<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
 
 int rtgs_launch_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* rays, int depth, float t_cut,
-                                     const float* dL_drgb, const float* dL_dT, float* const grads[6], float* grad_rays,
-                                     float* replay_rgb, float* replay_T, cudaStream_t stream) {
+                                     const float* dL_drgb, const float* dL_dT, const float* dL_dD,
+                                     float* const grads[6], float* grad_rays, float* replay_rgb, float* replay_T,
+                                     float* replay_depth, cudaStream_t stream) {
     if (nrays == 0) return RTGS_OK;
     backward::BackwardParams P = rays_params(s, nrays, rays, depth, t_cut);
     P.dL_drgb = dL_drgb;
@@ -1006,11 +1027,18 @@ int rtgs_launch_render_rays_backward(rtgs_scene* s, int64_t nrays, const float* 
     P.g_rays = grad_rays;
     P.replay_rgb = replay_rgb;
     P.replay_T = replay_T;
+    P.dL_dD = dL_dD;
+    P.replay_depth = replay_depth;
     const unsigned blocks = (unsigned)((nrays + backward::RAY_THREADS - 1) / backward::RAY_THREADS);
-    if (grad_rays == nullptr)
+    const bool with_depth = dL_dD != nullptr || replay_depth != nullptr;
+    if (grad_rays == nullptr && !with_depth)
         backward::k_render_rays_backward<false><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
-    else
+    else if (grad_rays == nullptr)
+        backward::k_render_rays_backward<false, true><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    else if (!with_depth)
         backward::k_render_rays_backward<true><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
+    else
+        backward::k_render_rays_backward<true, true><<<blocks, backward::RAY_THREADS, 0, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }

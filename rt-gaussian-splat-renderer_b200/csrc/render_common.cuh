@@ -127,6 +127,7 @@ struct RenderParams {
     int final_kernel;         // this launch is the frame's last kernel: its last CTA completes the frame (frame_complete)
     int self_clean;           // ... and zeroes the work counters for the next frame (no memset between frames)
     int tail_grid;            // CTAs of a device-side k_render launch (2 per SM)
+    float* out_depth;         // DEPTH instantiations: composited ray distance per pixel, indexed like out_T; may be null
 };
 
 // System-scope hand-over of a framebuffer that other GPUs read or write (see RenderParams::grant).
@@ -488,10 +489,9 @@ __device__ __forceinline__ void make_tile_rays(const CamD& cam, int i0, int j0, 
     r.L_hi = __double2float_ru(sqrt(xh * xh + yh * yh + 1.0));
 }
 
-// normalize(d) of the lane's ray (make_tile_rays) for the SH basis (gaussian.py:200).  Taken where the colours are
-// evaluated: carried from make_tile_rays, it held three registers through the candidate loops.
-__device__ __forceinline__ void sh_direction(const CamD& cam, int i0, int j0, int pi, int pj, bool active, float& x,
-                                             float& y, float& z) {
+// The lane's ray direction d = D(a,b) / L in float64, in the pixel basis of make_tile_rays (the reference's d, whose
+// length is |q_cam|^2).
+__device__ __forceinline__ d3 lane_direction(const CamD& cam, int i0, int j0, int pi, int pj, bool active) {
     const double px0 = ((double)i0 + 0.5 * TILE_I - 0.5 * cam.W) * cam.ifx;
     const double py0 = ((double)j0 + 0.5 * TILE_J - 0.5 * cam.H) * cam.ify;
     const d3 D0 = cam_rot(cam, px0, py0, -1.0);
@@ -499,10 +499,56 @@ __device__ __forceinline__ void sh_direction(const CamD& cam, int i0, int j0, in
     const double bd = active ? ((double)(pj - j0) + 0.5 - 0.5 * TILE_J) * cam.ify : 0.0;
     const double px = px0 + ad, py = py0 + bd;
     const double nn = rsqrt(px * px + py * py + 1.0);
-    const d3 dw = d3make((D0.x + ad * cam.R[0] + bd * cam.R[1]) * nn, (D0.y + ad * cam.R[3] + bd * cam.R[4]) * nn,
-                         (D0.z + ad * cam.R[6] + bd * cam.R[7]) * nn);
+    return d3make((D0.x + ad * cam.R[0] + bd * cam.R[1]) * nn, (D0.y + ad * cam.R[3] + bd * cam.R[4]) * nn,
+                  (D0.z + ad * cam.R[6] + bd * cam.R[7]) * nn);
+}
+
+// normalize(d) of the lane's ray (make_tile_rays) for the SH basis (gaussian.py:200).  Taken where the colours are
+// evaluated: carried from make_tile_rays, it held three registers through the candidate loops.
+__device__ __forceinline__ void sh_direction(const CamD& cam, int i0, int j0, int pi, int pj, bool active, float& x,
+                                             float& y, float& z) {
+    const d3 dw = lane_direction(cam, i0, j0, pi, pj, active);
     const double il = rsqrt(d3dot(dw, dw));
     x = (float)(dw.x * il); y = (float)(dw.y * il); z = (float)(dw.z * il);
+}
+
+// ---- depth (DESIGN.md §12) ------------------------------------------------------------------------------------
+// t* = (p - o)^T W^T W d / |W d|^2, the ray parameter of the point where the Gaussian at sorted position s responds
+// most along the ray (o, d): float64 from its 64-byte geometry record {p, opacity}{W row-major}{rgb}.  Every route
+// calls this with the same record and lane_direction, so their depth images agree bit for bit.
+__device__ __forceinline__ float layer_depth(const RenderParams& P, int s, const d3& d) {
+    float4 g0, g1, g2, g3;
+    ldg256(P.geo + (int64_t)s * 4 + 0, g0, g1);
+    ldg256(P.geo + (int64_t)s * 4 + 2, g2, g3);
+    const double vx = (double)g0.x - P.cam.o[0], vy = (double)g0.y - P.cam.o[1], vz = (double)g0.z - P.cam.o[2];
+    const double u0 = (double)g1.x * vx + (double)g1.y * vy + (double)g1.z * vz;
+    const double u1 = (double)g1.w * vx + (double)g2.x * vy + (double)g2.y * vz;
+    const double u2 = (double)g2.z * vx + (double)g2.w * vy + (double)g3.x * vz;
+    const double w0 = (double)g1.x * d.x + (double)g1.y * d.y + (double)g1.z * d.z;
+    const double w1 = (double)g1.w * d.x + (double)g2.x * d.y + (double)g2.y * d.z;
+    const double w2 = (double)g2.z * d.x + (double)g2.w * d.y + (double)g3.x * d.z;
+    return (float)((u0 * w0 + u1 * w1 + u2 * w2) / (w0 * w0 + w1 * w1 + w2 * w2));
+}
+
+// D = sum_k T_k alpha_k t*_k over the layers the colour loop composited: the same order, the same float32 T and
+// t_cut stop, the same fmaf as a colour channel.  layer(k, s, alpha) gives the k-th nearest entry.  A pass of its
+// own after the colour loop, so that the SH basis is dead by then and the colour loop is that of the plain kernels.
+template <typename LayerAt>
+__device__ __forceinline__ float composite_depth(const RenderParams& P, int i0, int j0, int pi, int pj, bool active,
+                                                 int nmine, int nloop, LayerAt layer) {
+    const d3 d = lane_direction(P.cam, i0, j0, pi, pj, active);
+    float T = 1.0f, D = 0.0f;
+#pragma unroll 1
+    for (int k = 0; k < nloop; ++k) {
+        if (k < nmine && T >= P.t_cut) {
+            int s;
+            float alpha;
+            layer(k, s, alpha);
+            D = fmaf(T * alpha, layer_depth(P, s, d), D);
+            T *= 1.0f - alpha;
+        }
+    }
+    return D;
 }
 
 // Staged precise records of one batch, structure of arrays: quad k of candidate c is rec[k][c], so that a warp
@@ -704,9 +750,11 @@ __device__ __forceinline__ void eval_colour(const RenderParams& P, int s, const 
 }
 
 // Framebuffer write of one tile: staged through `ob` (>= 96 floats of shared memory) so that every store
-// instruction covers whole 32-byte sectors (each tile column is 8 pixels = 96 contiguous bytes).
+// instruction covers whole 32-byte sectors (each tile column is 8 pixels = 96 contiguous bytes).  DEPTH: D goes to
+// out_depth with out_T's indexing (+= with `accumulate`, as the colour).
+template <bool DEPTH = false>
 __device__ __forceinline__ void store_tile(const RenderParams& P, float* ob, int lane, int i0, int j0, int pi, int pj,
-                                           bool active, float cr, float cg, float cb, float T) {
+                                           bool active, float cr, float cg, float cb, float T, float D = 0.0f) {
     const int xe = P.x0 + P.w, ye = P.y0 + P.h;
     __syncwarp();
     ob[lane * 3 + 0] = cr;
@@ -732,7 +780,12 @@ __device__ __forceinline__ void store_tile(const RenderParams& P, float* ob, int
         }
     }
     if (active && P.out_T) P.out_T[(int64_t)(pi - bi) * pitch + (pj - bj)] = T;
-    __syncwarp();   // every lane's RGB and T stores are ordered before whatever lane 0 releases next (tile_done)
+    if (DEPTH && active && P.out_depth) {
+        float* o = P.out_depth + (int64_t)(pi - bi) * pitch + (pj - bj);
+        if (P.accumulate) *o += D;
+        else *o = D;
+    }
+    __syncwarp();   // every lane's RGB, T and depth stores are ordered before whatever lane 0 releases next (tile_done)
 }
 
 }  // namespace rtgs_dev

@@ -62,8 +62,9 @@ struct ShadeStats {
                        st_ins = 0;
 };
 
-// Shade tile `tile` (a valid id < P.ntiles whose descriptor has been published).
-template <bool STATS>
+// Shade tile `tile` (a valid id < P.ntiles whose descriptor has been published).  DEPTH: also the composited ray
+// distance (render_common.cuh: composite_depth) to P.out_depth.
+template <bool STATS, bool DEPTH = false>
 __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& ws, ShadeStats& S, PeerGrant& G,
                                            BandCount& BC, int tile, int lane) {
     constexpr int K = SHADE_K;
@@ -256,7 +257,7 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
     ST(S.st_f64 += n_exact);
 
     // ---- compositing: accum += T * alpha * rgb ; T *= 1 - alpha   (ray_tracer.py:96-98) ---------
-    float T = 1.0f, cr = 0.0f, cg = 0.0f, cb = 0.0f;
+    float T = 1.0f, cr = 0.0f, cg = 0.0f, cb = 0.0f, D = 0.0f;
     int nl = 0;
     if (maxcnt > 0) {
         float Y[15];
@@ -310,9 +311,17 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
             }
         }
 #endif
+        if constexpr (DEPTH) {
+            static_assert(!(DEPTH && SHADE_SLOT_ORDER), "SHADE_SLOT_ORDER overwrites the alphas composite_depth reads");
+            D = composite_depth(P, i0, j0, pi, pj, active, nmine, min(maxcnt, P.depth), [&](int k, int& s, float& a) {
+                const int slot = (int)((perm >> (4 * k)) & 15u);
+                s = ws.kb_i[slot][lane];
+                a = ws.kb_a[slot][lane];
+            });
+        }
     }
     grant_wait(P, G);
-    store_tile(P, reinterpret_cast<float*>(&ws.rec[0][0]), lane, i0, j0, pi, pj, active, cr, cg, cb, T);
+    store_tile<DEPTH>(P, reinterpret_cast<float*>(&ws.rec[0][0]), lane, i0, j0, pi, pj, active, cr, cg, cb, T, D);
     tile_done(P, BC, tile, lane);
     if (active) {
         ST(S.st_rays += 1);

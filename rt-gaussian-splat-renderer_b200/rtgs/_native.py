@@ -60,6 +60,9 @@ SIGNATURES = {
     "rtgs_render": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                               C.c_int32, C.c_float, C.c_int32, C.c_int32, _vp, _vp, _vp,
                               C.POINTER(rtgs_render_stats)]),
+    "rtgs_render_depth": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                    C.c_int32, C.c_float, C.c_int32, C.c_int32, _vp, _vp, _vp, _vp,
+                                    C.POINTER(rtgs_render_stats)]),
     "rtgs_scene_set_gaussians_device": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rtgs_render_backward": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                        C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
@@ -67,6 +70,9 @@ SIGNATURES = {
     "rtgs_render_backward_camera": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32,
                                               C.c_int32, C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                               _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rtgs_render_backward_depth": (C.c_int, [_vp, C.POINTER(rtgs_camera), C.c_int32, C.c_int32, C.c_int32,
+                                             C.c_int32, C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                             _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rtgs_scene_set_option": (C.c_int, [_vp, C.c_int32, C.c_int64]),
     "rtgs_scene_get_option": (C.c_int, [_vp, C.c_int32, C.POINTER(C.c_int64)]),
     "rtgs_scene_set_frame_sync": (C.c_int, [_vp, _vp, _vp, C.c_uint32]),
@@ -97,8 +103,11 @@ SIGNATURES = {
     "rtgs_generate_rays": (C.c_int, [C.POINTER(rtgs_camera), C.c_int, _vp, _vp]),
     "rtgs_trace_closest": (C.c_int, [_vp, C.c_int64, _vp, _vp, _vp, _vp]),
     "rtgs_render_rays": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp]),
+    "rtgs_render_rays_depth": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp, _vp]),
     "rtgs_render_rays_backward": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp, _vp, _vp,
                                             _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rtgs_render_rays_backward_depth": (C.c_int, [_vp, C.c_int64, _vp, C.c_int32, C.c_float, _vp, _vp, _vp, _vp,
+                                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rtgs_scene_destroy": (C.c_int, [_vp]),
 }
 

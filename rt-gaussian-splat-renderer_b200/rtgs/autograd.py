@@ -17,6 +17,11 @@ in between.  ``render_camera`` renders the scene as stored, differentiable with 
 rebuilds nothing: the loop of pose refinement or of tracking a camera against a fixed scene.  ``render_rays`` renders
 arbitrary rays (non-pinhole cameras, ray batches drawn from many views) and differentiates with respect to the rays
 too (``rtgs_render_rays`` / ``rtgs_render_rays_backward``).
+
+All three take ``with_depth=True`` to return ``(rgb, T, D)`` as well: D = sum_k T_k alpha_k t*_k, t*_k the ray parameter
+of layer k's max-response point (``rtgs_render_depth`` / ``rtgs_render_rays_depth``), differentiable like the colour.
+D is not normalised; D / (1 - T) is the expected distance along the ray.  The backward takes the ``_depth`` entry
+point only when D received a gradient.
 """
 from __future__ import annotations
 
@@ -48,7 +53,7 @@ def _native_camera(camera, position, rotation, focal):
 
 class _Render(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, scene, camera, depth, t_cut, tile, update, cam_position, cam_rotation, cam_focal,
+    def forward(ctx, scene, camera, depth, t_cut, tile, update, with_depth, cam_position, cam_rotation, cam_focal,
                 pos, rot, scale, color, opacity, sh):
         if update:
             params = [t.detach().contiguous() if t is not None else None
@@ -60,45 +65,56 @@ class _Render(torch.autograd.Function):
         rgb = torch.empty((w, h, 3), dtype=torch.float32, device=dev)
         T = torch.empty((w, h), dtype=torch.float32, device=dev)
         cam = _native_camera(camera, cam_position, cam_rotation, cam_focal)
-        _native.check(_native.load().rtgs_render(scene.handle, cam, x0, y0, w, h, int(depth), float(t_cut), 0, 0,
-                                                 rgb.data_ptr(), T.data_ptr(),
-                                                 torch.cuda.current_stream(dev).cuda_stream, None))
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        head = (scene.handle, cam, x0, y0, w, h, int(depth), float(t_cut), 0, 0, rgb.data_ptr(), T.data_ptr())
+        if with_depth:
+            D = torch.empty((w, h), dtype=torch.float32, device=dev)
+            _native.check(_native.load().rtgs_render_depth(*head, D.data_ptr(), stream, None))
+        else:
+            _native.check(_native.load().rtgs_render(*head, stream, None))
         ctx.scene, ctx.cam, ctx.region, ctx.depth, ctx.t_cut = scene, cam, (x0, y0, w, h), int(depth), float(t_cut)
         ctx.has_sh = sh is not None
         ctx.cam_devices = tuple(None if t is None else t.device for t in (cam_position, cam_rotation, cam_focal))
         ctx.dev = dev
-        return rgb, T
+        if not with_depth:
+            return rgb, T
+        ctx.set_materialize_grads(False)   # g_D is None unless D was used: then the plain backward runs
+        return rgb, T, D
 
     @staticmethod
-    def backward(ctx, g_rgb, g_T):
+    def backward(ctx, g_rgb, g_T, g_D=None):
         scene, dev = ctx.scene, ctx.dev
         x0, y0, w, h = ctx.region
         n = scene.num_gaussians
         shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,), sh=(n, 15, 3))
-        need = dict(zip(_NAMES, ctx.needs_input_grad[9:]))
+        need = dict(zip(_NAMES, ctx.needs_input_grad[10:]))
         need["sh"] = need["sh"] and ctx.has_sh
         grads = {k: torch.zeros(shapes[k], dtype=torch.float32, device=dev) if need[k] else None for k in _NAMES}
         cam_grads = [torch.zeros(shape, dtype=torch.float32, device=dev) if nd else None
-                     for shape, nd in zip(_CAM_SHAPES.values(), ctx.needs_input_grad[6:9])]
+                     for shape, nd in zip(_CAM_SHAPES.values(), ctx.needs_input_grad[7:10])]
         if g_rgb is None:
             g_rgb = torch.zeros((w, h, 3), dtype=torch.float32, device=dev)
         g_rgb = g_rgb.to(torch.float32).contiguous()
         g_T = None if g_T is None else g_T.to(torch.float32).contiguous()
+        g_D = None if g_D is None else g_D.to(torch.float32).contiguous()
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         lib = _native.load()
         head = (scene.handle, ctx.cam, x0, y0, w, h, ctx.depth, ctx.t_cut, g_rgb.data_ptr(), ptr(g_T),
                 *(ptr(grads[k]) for k in _NAMES))
         tail = (None, None, torch.cuda.current_stream(dev).cuda_stream)
-        if any(g is not None for g in cam_grads):
+        if g_D is not None:
+            _native.check(lib.rtgs_render_backward_depth(*head, *(ptr(g) for g in cam_grads), None, None,
+                                                         g_D.data_ptr(), None, tail[2]))
+        elif any(g is not None for g in cam_grads):
             _native.check(lib.rtgs_render_backward_camera(*head, *(ptr(g) for g in cam_grads), *tail))
         else:
             _native.check(lib.rtgs_render_backward(*head, *tail))
         cam_grads = [None if g is None else g.to(d) for g, d in zip(cam_grads, ctx.cam_devices)]
-        return (None,) * 6 + tuple(cam_grads) + tuple(grads[k] for k in _NAMES)
+        return (None,) * 7 + tuple(cam_grads) + tuple(grads[k] for k in _NAMES)
 
 
 def render(scene, camera, pos, rot, scale, color, opacity, sh=None, depth: int = 16, t_cut: float = 0.0, tile=None, *,
-           cam_position=None, cam_rotation=None, cam_focal=None):
+           cam_position=None, cam_rotation=None, cam_focal=None, with_depth: bool = False):
     """Render ``camera`` from the given parameters and return ``(rgb (w,h,3), T (w,h))``, differentiable with respect to
     every parameter tensor that requires a gradient.  The tensors are CUDA float32 on the scene's device with the
     shapes of ``Scene.from_arrays`` (``sh`` iff the scene has SH); the scene's stored parameters become these values.
@@ -107,15 +123,16 @@ def render(scene, camera, pos, rot, scale, color, opacity, sh=None, depth: int =
     ``cam_position`` (3,), ``cam_rotation`` (4,, x,y,z,w, used as given like ``Camera.rotation``) and ``cam_focal``
     (2,) are optional float32 tensors on any device that replace the camera's values for this call and receive
     gradients when they require them (each on its own device).  The render takes the camera by value, so their
-    values are read to the host in the forward: CUDA tensors cost one synchronisation."""
+    values are read to the host in the forward: CUDA tensors cost one synchronisation.  ``with_depth=True`` returns
+    ``(rgb, T, D (w,h))`` (module docstring)."""
     if not 1 <= int(depth) <= MAX_DEPTH:
         raise ValueError(f"depth must be in [1, {MAX_DEPTH}]")
-    return _Render.apply(scene, camera, int(depth), float(t_cut), tile, True, cam_position, cam_rotation, cam_focal,
-                         pos, rot, scale, color, opacity, sh)
+    return _Render.apply(scene, camera, int(depth), float(t_cut), tile, True, bool(with_depth), cam_position,
+                         cam_rotation, cam_focal, pos, rot, scale, color, opacity, sh)
 
 
 def render_camera(scene, camera, position=None, rotation=None, focal=None, depth: int = 16, t_cut: float = 0.0,
-                  tile=None):
+                  tile=None, *, with_depth: bool = False):
     """Render the scene as stored and return ``(rgb (w,h,3), T (w,h))``, differentiable with respect to the camera
     only: ``position`` (3,), ``rotation`` (4,) and ``focal`` (2,) are float32 tensors as in ``render`` (their values
     are read to the host in the forward, one synchronisation for CUDA tensors); the ones left None are the camera's.
@@ -125,49 +142,58 @@ def render_camera(scene, camera, position=None, rotation=None, focal=None, depth
         for _ in range(steps):
             rgb, _ = rtgs.autograd.render_camera(scene, camera, position, rotation)
             loss = ((rgb - target) ** 2).mean(); opt.zero_grad(); loss.backward(); opt.step()
+
+    ``with_depth=True`` returns ``(rgb, T, D (w,h))``: RGB-D tracking adds a loss on D / (1 - T).
     """
     if not 1 <= int(depth) <= MAX_DEPTH:
         raise ValueError(f"depth must be in [1, {MAX_DEPTH}]")
-    return _Render.apply(scene, camera, int(depth), float(t_cut), tile, False, position, rotation, focal,
-                         None, None, None, None, None, None)
+    return _Render.apply(scene, camera, int(depth), float(t_cut), tile, False, bool(with_depth), position, rotation,
+                         focal, None, None, None, None, None, None)
 
 
 class _RenderRays(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, scene, depth, t_cut, update, rays, pos, rot, scale, color, opacity, sh):
+    def forward(ctx, scene, depth, t_cut, update, with_depth, rays, pos, rot, scale, color, opacity, sh):
         if update:
             scene.set_gaussians(*(t.detach().contiguous() if t is not None else None
                                   for t in (pos, rot, scale, color, opacity, sh)))
-        rgb, T = scene.render_rays(rays, depth, t_cut)
+        out = scene.render_rays(rays, depth, t_cut, with_depth=with_depth)
         ctx.save_for_backward(rays)
         ctx.scene, ctx.depth, ctx.t_cut, ctx.has_sh = scene, depth, t_cut, sh is not None
-        return rgb, T
+        if with_depth:
+            ctx.set_materialize_grads(False)   # g_D is None unless D was used: then the plain backward runs
+        return out
 
     @staticmethod
-    def backward(ctx, g_rgb, g_T):
+    def backward(ctx, g_rgb, g_T, g_D=None):
         (rays,) = ctx.saved_tensors
         scene = ctx.scene
         rays_c = scene._rays_arg(rays)
         dev, lead = rays_c.device, tuple(rays_c.shape[:-1])
         n = scene.num_gaussians
         shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,), sh=(n, 15, 3))
-        need = dict(zip(_NAMES, ctx.needs_input_grad[5:]))
+        need = dict(zip(_NAMES, ctx.needs_input_grad[6:]))
         need["sh"] = need["sh"] and ctx.has_sh
         grads = {k: torch.zeros(shapes[k], dtype=torch.float32, device=dev) if need[k] else None for k in _NAMES}
-        g_rays = torch.zeros(lead + (8,), dtype=torch.float32, device=dev) if ctx.needs_input_grad[4] else None
+        g_rays = torch.zeros(lead + (8,), dtype=torch.float32, device=dev) if ctx.needs_input_grad[5] else None
         if g_rgb is None:
             g_rgb = torch.zeros(lead + (3,), dtype=torch.float32, device=dev)
         g_rgb = g_rgb.to(torch.float32).contiguous()
         g_T = None if g_T is None else g_T.to(torch.float32).contiguous()
+        g_D = None if g_D is None else g_D.to(torch.float32).contiguous()
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        _native.check(_native.load().rtgs_render_rays_backward(
-            scene.handle, rays_c.numel() // 8, rays_c.data_ptr(), ctx.depth, ctx.t_cut, g_rgb.data_ptr(), ptr(g_T),
-            *(ptr(grads[k]) for k in _NAMES), ptr(g_rays), None, None, torch.cuda.current_stream(dev).cuda_stream))
-        return (None,) * 4 + (g_rays,) + tuple(grads[k] for k in _NAMES)
+        args = (scene.handle, rays_c.numel() // 8, rays_c.data_ptr(), ctx.depth, ctx.t_cut, g_rgb.data_ptr(), ptr(g_T),
+                *(ptr(grads[k]) for k in _NAMES), ptr(g_rays), None, None)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if g_D is None:
+            _native.check(_native.load().rtgs_render_rays_backward(*args, stream))
+        else:
+            _native.check(_native.load().rtgs_render_rays_backward_depth(*args, g_D.data_ptr(), None, stream))
+        return (None,) * 5 + (g_rays,) + tuple(grads[k] for k in _NAMES)
 
 
 def render_rays(scene, rays, pos=None, rot=None, scale=None, color=None, opacity=None, sh=None, depth: int = 16,
-                t_cut: float = 0.0):
+                t_cut: float = 0.0, *, with_depth: bool = False):
     """Composite arbitrary rays and return ``(rgb (..., 3), T (...))``, differentiable with respect to the rays and,
     when they are given, the Gaussian parameters (``Scene.render_rays`` / ``render_rays_backward``).
 
@@ -180,6 +206,9 @@ def render_rays(scene, rays, pos=None, rot=None, scale=None, color=None, opacity
         rays = torch.cat([cam_rays[v][idx[v]] for v in views])          # (B, 8)
         rgb, _ = rtgs.autograd.render_rays(scene, rays, pos, rot, scale, color, opacity, sh)
         loss = ((rgb - target) ** 2).mean(); opt.zero_grad(); loss.backward(); opt.step()
+
+    ``with_depth=True`` returns ``(rgb, T, D (...))``, D in units of each ray's d: sensor or LiDAR depth supervision
+    on ray batches.
     """
     if not 1 <= int(depth) <= MAX_DEPTH:
         raise ValueError(f"depth must be in [1, {MAX_DEPTH}]")
@@ -188,4 +217,5 @@ def render_rays(scene, rays, pos=None, rot=None, scale=None, color=None, opacity
         raise ValueError("pass all of pos, rot, scale, color, opacity (and sh for a scene with SH), or none")
     if not any(given) and sh is not None:
         raise ValueError("sh was given without the other Gaussian tensors")
-    return _RenderRays.apply(scene, int(depth), float(t_cut), all(given), rays, pos, rot, scale, color, opacity, sh)
+    return _RenderRays.apply(scene, int(depth), float(t_cut), all(given), bool(with_depth), rays, pos, rot, scale, color,
+                             opacity, sh)

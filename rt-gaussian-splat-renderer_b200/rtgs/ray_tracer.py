@@ -198,25 +198,34 @@ class RayTracer:
         if prev is not None:
             yield k, prev.result()
 
-    def render_device(self, depth: int = 16, tile=None, out=None, out_T=None, collect_stats: bool = False):
-        """Render into device memory (a torch CUDA tensor) on the current stream; no host copy."""
+    def render_device(self, depth: int = 16, tile=None, out=None, out_T=None, collect_stats: bool = False,
+                      out_depth=None):
+        """Render into device memory (a torch CUDA tensor) on the current stream; no host copy.  ``out_depth`` (w,h)
+        float32 on the device also receives the composited ray distance D (rtgs_render_depth): D / (1 - T) is the
+        expected distance along each pixel's ray."""
         import torch
         W, H = self.buf_size.x, self.buf_size.y
         x0, y0, w, h = (0, 0, W, H) if tile is None else tile
         if out is None:
             out = torch.empty((w, h, 3), dtype=torch.float32, device=self._dev)
+        if out_depth is not None and (out_depth.device != self._dev or out_depth.dtype != torch.float32
+                                      or tuple(out_depth.shape) != (w, h) or not out_depth.is_contiguous()):
+            raise ValueError(f"out_depth: expected a contiguous float32 tensor of shape {(w, h)} on {self._dev}")
         stats = _native.rtgs_render_stats() if collect_stats else None
         cam = self.camera.native()
-        _native.check(_native.load().rtgs_render(
-            self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, 0, 0, out.data_ptr(),
-            None if out_T is None else out_T.data_ptr(), torch.cuda.current_stream(self._dev).cuda_stream,
-            None if stats is None else C.byref(stats)))
+        args = (self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, 0, 0, out.data_ptr(),
+                None if out_T is None else out_T.data_ptr())
+        tail = (torch.cuda.current_stream(self._dev).cuda_stream, None if stats is None else C.byref(stats))
+        if out_depth is None:
+            _native.check(_native.load().rtgs_render(*args, *tail))
+        else:
+            _native.check(_native.load().rtgs_render_depth(*args, out_depth.data_ptr(), *tail))
         if stats is not None:
             self.last_stats = stats.as_dict()
         return out
 
     def render_backward(self, dL_drgb, dL_dT=None, depth: int = 16, tile=None, grads=None, replay: bool = False,
-                        camera: bool = False):
+                        camera: bool = False, dL_dD=None):
         """Gradient of ``render_device(depth, tile)`` (with ``t_cut``) with respect to the stored Gaussian parameters,
         the layer list of every pixel held fixed (rtgs_render_backward), on the current stream.
 
@@ -225,7 +234,9 @@ class RayTracer:
         names to accumulate into (missing ones are zero-initialised).  With ``replay=True`` the dict also holds
         ``rgb`` / ``T``, the image the backward recomputed.  With ``camera=True`` it also holds the gradient with
         respect to the camera (rtgs_render_backward_camera): ``camera_position`` (3,), ``camera_rotation`` (4,, the
-        x,y,z,w quaternion as stored) and ``camera_focal`` (2,), which ``grads`` may pass in the same way."""
+        x,y,z,w quaternion as stored) and ``camera_focal`` (2,), which ``grads`` may pass in the same way.
+        ``dL_dD`` (w,h) is the gradient with respect to the depth of ``render_device(out_depth=...)``
+        (rtgs_render_backward_depth); with it, ``replay=True`` also returns ``depth``."""
         import torch
         W, H = self.buf_size.x, self.buf_size.y
         x0, y0, w, h = (0, 0, W, H) if tile is None else tile
@@ -238,6 +249,7 @@ class RayTracer:
 
         dL_drgb = region(dL_drgb, (w, h, 3), "dL_drgb")
         dL_dT = None if dL_dT is None else region(dL_dT, (w, h), "dL_dT")
+        dL_dD = None if dL_dD is None else region(dL_dD, (w, h), "dL_dD")
         shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
         if self.scene.has_sh:
             shapes["sh"] = (n, 15, 3)
@@ -253,6 +265,8 @@ class RayTracer:
         if replay:
             out["rgb"] = torch.empty((w, h, 3), dtype=torch.float32, device=self._dev)
             out["T"] = torch.empty((w, h), dtype=torch.float32, device=self._dev)
+            if dL_dD is not None:
+                out["depth"] = torch.empty((w, h), dtype=torch.float32, device=self._dev)
         cam = self.camera.native()
         ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
         head = (self.scene.handle, cam, x0, y0, w, h, int(depth), self.t_cut, dL_drgb.data_ptr(),
@@ -260,7 +274,11 @@ class RayTracer:
                 ptr("opacity"), ptr("sh"))
         tail = (ptr("rgb"), ptr("T"), torch.cuda.current_stream(self._dev).cuda_stream)
         lib = _native.load()
-        if camera:
+        if dL_dD is not None:
+            _native.check(lib.rtgs_render_backward_depth(
+                *head, ptr("camera_position"), ptr("camera_rotation"), ptr("camera_focal"), *tail[:2],
+                dL_dD.data_ptr(), ptr("depth"), tail[2]))
+        elif camera:
             _native.check(lib.rtgs_render_backward_camera(
                 *head, ptr("camera_position"), ptr("camera_rotation"), ptr("camera_focal"), *tail))
         else:

@@ -439,14 +439,16 @@ class Scene:
             raise ValueError(f"{name}: expected a contiguous float32 tensor of shape {tuple(shape)} on {dev}")
         return t
 
-    def render_rays(self, rays, depth: int = 16, t_cut: float = 0.0, out=None, out_T=None):
+    def render_rays(self, rays, depth: int = 16, t_cut: float = 0.0, out=None, out_T=None, out_depth=None,
+                    with_depth: bool = False):
         """Composite arbitrary rays (rtgs_render_rays) on the current stream and return ``(rgb (..., 3), T (...))``.
 
         ``rays`` is a CUDA float32 tensor of shape (..., 8) on the scene's device: origin, direction (used as given,
         not normalised), start, end - the record of ``Camera.generate_ray_field``, so a (W,H,8) ray field gives a
         (W,H,3) image in the layout of ``RayTracer.render_device``.  Each ray composites its ``depth`` nearest
         Gaussians with start < t1 < end, front to back while T >= ``t_cut``.  ``out`` / ``out_T`` may pass the output
-        tensors."""
+        tensors.  With ``out_depth`` (...) or ``with_depth=True`` it returns ``(rgb, T, D)``: D = sum_k T_k alpha_k t*_k,
+        t*_k the ray parameter (units of the ray's d) of layer k's max-response point (rtgs_render_rays_depth)."""
         import torch
         rays = self._rays_arg(rays)
         dev = rays.device
@@ -457,13 +459,20 @@ class Scene:
             out = torch.empty(lead + (3,), dtype=torch.float32, device=dev)
         if out_T is None:
             out_T = torch.empty(lead, dtype=torch.float32, device=dev)
-        _native.check(_native.load().rtgs_render_rays(self.handle, rays.numel() // 8, rays.data_ptr(), int(depth),
-                                                      float(t_cut), out.data_ptr(), out_T.data_ptr(),
-                                                      torch.cuda.current_stream(dev).cuda_stream))
-        return out, out_T
+        out_depth = self._buffer(out_depth, lead, "out_depth", dev)
+        if out_depth is None and with_depth:
+            out_depth = torch.empty(lead, dtype=torch.float32, device=dev)
+        head = (self.handle, rays.numel() // 8, rays.data_ptr(), int(depth), float(t_cut), out.data_ptr(),
+                out_T.data_ptr())
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if out_depth is None:
+            _native.check(_native.load().rtgs_render_rays(*head, stream))
+            return out, out_T
+        _native.check(_native.load().rtgs_render_rays_depth(*head, out_depth.data_ptr(), stream))
+        return out, out_T, out_depth
 
     def render_rays_backward(self, rays, dL_drgb, dL_dT=None, depth: int = 16, t_cut: float = 0.0, grads=None,
-                             rays_grad: bool = False, replay: bool = False):
+                             rays_grad: bool = False, replay: bool = False, dL_dD=None):
         """Gradient of ``render_rays(rays, depth, t_cut)`` with each ray's layer list held fixed
         (rtgs_render_rays_backward), on the current stream.
 
@@ -471,13 +480,16 @@ class Scene:
         float32 gradients ``pos rot scale color opacity`` and ``sh`` (scenes with SH), as ``RayTracer.render_backward``
         does; with ``rays_grad=True`` also ``rays`` (..., 8): dL/do in columns 0-2, dL/dd in 3-5, zeros in 6-7.
         ``grads`` may pass tensors of these names to accumulate into (missing ones are zero-initialised).  With
-        ``replay=True`` the dict also holds ``rgb`` / ``T``, the image the backward recomputed."""
+        ``replay=True`` the dict also holds ``rgb`` / ``T``, the image the backward recomputed.  ``dL_dD`` (...) is the
+        gradient with respect to the depth of ``render_rays(with_depth=True)`` (rtgs_render_rays_backward_depth); with
+        it, ``replay=True`` also returns ``depth``."""
         import torch
         rays = self._rays_arg(rays)
         dev = rays.device
         lead = tuple(rays.shape[:-1])
         dL_drgb = self._buffer(dL_drgb.contiguous(), lead + (3,), "dL_drgb", dev)
         dL_dT = None if dL_dT is None else self._buffer(dL_dT.contiguous(), lead, "dL_dT", dev)
+        dL_dD = None if dL_dD is None else self._buffer(dL_dD.contiguous(), lead, "dL_dD", dev)
         n = self._n
         shapes = dict(pos=(n, 3), rot=(n, 4), scale=(n, 3), color=(n, 3), opacity=(n,))
         if self.has_sh:
@@ -493,10 +505,16 @@ class Scene:
         if replay:
             out["rgb"] = torch.empty(lead + (3,), dtype=torch.float32, device=dev)
             out["T"] = torch.empty(lead, dtype=torch.float32, device=dev)
+            if dL_dD is not None:
+                out["depth"] = torch.empty(lead, dtype=torch.float32, device=dev)
         ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
-        _native.check(_native.load().rtgs_render_rays_backward(
-            self.handle, rays.numel() // 8, rays.data_ptr(), int(depth), float(t_cut), dL_drgb.data_ptr(),
-            None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
-            ptr("opacity"), ptr("sh"), ptr("rays") if rays_grad else None, ptr("rgb"), ptr("T"),
-            torch.cuda.current_stream(dev).cuda_stream))
+        args = (self.handle, rays.numel() // 8, rays.data_ptr(), int(depth), float(t_cut), dL_drgb.data_ptr(),
+                None if dL_dT is None else dL_dT.data_ptr(), ptr("pos"), ptr("rot"), ptr("scale"), ptr("color"),
+                ptr("opacity"), ptr("sh"), ptr("rays") if rays_grad else None, ptr("rgb"), ptr("T"))
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if dL_dD is None:
+            _native.check(_native.load().rtgs_render_rays_backward(*args, stream))
+        else:
+            _native.check(_native.load().rtgs_render_rays_backward_depth(*args, dL_dD.data_ptr(), ptr("depth"),
+                                                                         stream))
         return out
