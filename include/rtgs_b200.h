@@ -251,7 +251,7 @@ typedef enum rtgs_option {
     RTGS_OPT_STRIPE = 3,
     RTGS_OPT_MORTON_BITS = 4,
     RTGS_OPT_HEAVY_LISTS = 6,    /* tiles of groups whose frustum holds more candidates than the traversal's shared-memory
-                                  * list: 0 (default; env RTGS_HEAVY_SLAB) = rendered by the fused kernel k_render; 1 = listed
+                                  * list: 0 (default) = rendered by the fused kernel k_render; 1 = listed
                                   * in depth slabs by k_heavy_lists once a frame of the scene has had such groups, 2 = from
                                   * the first frame on (csrc/heavy_lists.cuh; same pixels, bit for bit).  Mode 0 renders only. */
     RTGS_OPT_HEAVY_LIMIT = 7,    /* a group is heavy above this many candidates (default -1: the capacity of the shared
@@ -269,9 +269,8 @@ int rtgs_scene_get_option(const rtgs_scene* s, int32_t option, int64_t* value);
  * bracket its kernels with CUDA events on the render stream (a ring of n frames; 0 switches it off).
  * rtgs_scene_read_kernel_times synchronises the device and returns, for the last `frames` renders (oldest
  * first), RTGS_NUM_KERNELS floats each, the milliseconds of the frame's (up to) three launches in order:
- * mode 0: k_tile_lists, k_shade_tiles, k_render; mode 2: 0, k_frame (a device-side tail launch of k_render
- * included), host-launched k_render if any; mode 1: 0, 0, k_render.  Fails with RTGS_ERR_STATE if fewer
- * frames were timed. */
+ * mode 0: k_tile_lists, k_shade_tiles, k_render; mode 2: 0, k_frame, k_render (the hand-over tiles); mode 1:
+ * 0, 0, k_render.  Fails with RTGS_ERR_STATE if fewer frames were timed. */
 #define RTGS_NUM_KERNELS 3
 int rtgs_scene_read_kernel_times(rtgs_scene* s, int32_t frames, float* ms /* frames * RTGS_NUM_KERNELS */);
 

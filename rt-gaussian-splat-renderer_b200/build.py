@@ -25,10 +25,6 @@ FLAGS = [
     "-Xcompiler", "-fPIC",
     "-Xptxas", "-v",
 ] + os.environ.get("RTGS_NVCC_EXTRA", "").split()
-# RTGS_CDP=1: k_frame tail-launches k_render from the device (CUDA dynamic parallelism): relocatable device code
-CDP = os.environ.get("RTGS_CDP", "0") == "1"
-if CDP:
-    FLAGS += ["-rdc=true", "-DRTGS_CDP=1"]
 
 
 def _stale() -> bool:
@@ -66,7 +62,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
     if verbose:
         print("\n".join(log))
     cmd = [NVCC, "-shared", "-o", str(LIB), *[str(o) for _, o, _ in results],
-           "-gencode", "arch=compute_100a,code=sm_100a"] + (["-rdc=true", "-lcudadevrt"] if CDP else [])
+           "-gencode", "arch=compute_100a,code=sm_100a"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         sys.stderr.write(r.stdout + r.stderr)

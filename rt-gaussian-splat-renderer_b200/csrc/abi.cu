@@ -2,7 +2,6 @@
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
-#include <time.h>
 
 #include <cmath>
 #include <new>
@@ -51,7 +50,6 @@ void free_scene(rtgs_scene* s) {
     cudaFree(s->sh); cudaFree(s->morton); cudaFree(s->sorted_idx); cudaFree(s->child); cudaFree(s->parent);
     cudaFree(s->morton64);
     if (s->shp_tex) cudaDestroyTextureObject(s->shp_tex);
-    if (s->geo_tex) cudaDestroyTextureObject(s->geo_tex);
     cudaFree(s->aabb); cudaFree(s->geo); cudaFree(s->shp); cudaFree(s->raw); cudaFree(s->nodes); cudaFree(s->leafbox); cudaFree(s->nodes4);
     for (auto& fs : s->scratch) {
         cudaFree(fs.tile_desc); cudaFree(fs.list_pool); cudaFree(fs.fallback_tiles); cudaFree(fs.fallback_tiles2); cudaFree(fs.ready);
@@ -137,29 +135,14 @@ int alloc_scene(int device, int64_t n, bool has_sh, rtgs_scene** out) {
     TRY(dev_alloc(&s->parent, 2 * n - 1));
     TRY(dev_alloc(&s->aabb, (2 * n - 1) * 6));
     TRY(dev_alloc(&s->geo, n * 4));
-#if SHADE_GEO_TEX
-    {
-        cudaResourceDesc rd = {};
-        rd.resType = cudaResourceTypeLinear;
-        rd.res.linear.devPtr = s->geo;
-        rd.res.linear.desc = cudaCreateChannelDesc<float4>();
-        rd.res.linear.sizeInBytes = (size_t)n * 4 * sizeof(float4);
-        cudaTextureDesc td = {};
-        td.readMode = cudaReadModeElementType;
-        CUDA_TRY(cudaCreateTextureObject(&s->geo_tex, &rd, &td, nullptr));
-    }
-#endif
     if (has_sh) {
         // the SH records and a linear float4 texture over them (eval_colour fetches part of a record through the
-        // texture path: the LSU pipe bounds the shading, the TEX pipe has throughput to spare)
+        // texture path: the LSU pipe bounds the shading, the TEX pipe has throughput to spare).  Scenes too large for
+        // one linear texture get no texture and eval_colour loads the whole record.
         TRY(dev_alloc(&s->shp, n * 12));
         const char* tex_env = getenv("RTGS_SH_TEX");     // "0": no texture, loads only (what huge scenes get; tests)
-        const bool tex_off = SHADE_SH_TEX_RUNTIME && tex_env != nullptr && atoi(tex_env) == 0;
-        if (!tex_off && (n <= rtgs_dev::SH_TEX_MAX_RECORDS || !SHADE_SH_TEX_RUNTIME)) {
-            if (n > rtgs_dev::SH_TEX_MAX_RECORDS) {
-                rtgs_set_error("too many Gaussians with SH for the record texture (%lld)", (long long)n);
-                return RTGS_ERR_INVALID;
-            }
+        const bool tex_off = tex_env != nullptr && atoi(tex_env) == 0;
+        if (!tex_off && n <= rtgs_dev::SH_TEX_MAX_RECORDS) {
             cudaResourceDesc rd = {};
             rd.resType = cudaResourceTypeLinear;
             rd.res.linear.devPtr = s->shp;
@@ -814,21 +797,6 @@ int rtgs_host_free(void* p) {
     return RTGS_OK;
 }
 
-// How rtgs_render_host delivers the image to a pinned destination:
-//   0 = render to device memory, then one DMA;
-//   1 = the kernel stores straight into the mapped host buffer (zero-copy; 32..96-byte PCIe writes);
-//   2 = (default) render to device memory in bands of 32-pixel columns; the kernels raise a host-visible flag
-//       per finished band and this thread queues the band's DMA while the later bands are still rendering.
-// RTGS_HOST_MODE overrides the default.
-static int host_mode() {
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("RTGS_HOST_MODE");
-        mode = e ? atoi(e) : 2;
-    }
-    return mode;
-}
-
 static void* pinned_device_ptr(const void* host) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, host) != cudaSuccess) {
@@ -863,12 +831,9 @@ static int submit_banded(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int3
     const int mrows = (w + 31) / 32;                       // 32-pixel macro-tile columns of the region
     const int bmc = (mrows + 23) / 24 > 0 ? (mrows + 23) / 24 : 1;
     const int nb = (mrows + bmc - 1) / bmc;                // <= 24 bands (RTGS_MAX_BANDS 32)
-    static const int sched = getenv("RTGS_BAND_SCHEDULE") ? atoi(getenv("RTGS_BAND_SCHEDULE")) : 2;
     for (int b = 0; b < nb; ++b) hs.flags[b] = 0;
-    static const bool nosignal = getenv("RTGS_BAND_NOSIGNAL") != nullptr;   // experiment: kernels do not count bands
-    s->bands_active = nosignal ? 0 : nb;
+    s->bands_active = nb;
     s->band_macro_cols = bmc;
-    s->band_schedule = sched;
     s->band_flags_cur_dev = hs.flags_dev;
     const int r = rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb,
                                      host_T ? hs.stage_T : nullptr, nullptr, s->own_stream, false);
@@ -876,7 +841,7 @@ static int submit_banded(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int3
     s->band_flags_cur_dev = nullptr;
     if (r != RTGS_OK) return r;
     CUDA_TRY(cudaEventRecord(hs.done, s->own_stream));
-    hs.nb = nb; hs.bmc = bmc; hs.sched = sched; hs.w = w; hs.h = h;
+    hs.nb = nb; hs.bmc = bmc; hs.w = w; hs.h = h;
     hs.host_rgb = host_rgb; hs.host_T = host_T;
     s->host_head ^= 1;
     ++s->host_inflight;
@@ -891,24 +856,18 @@ static int collect_banded(rtgs_scene* s) {
     --s->host_inflight;
     const int nb = hs.nb, bmc = hs.bmc, w = hs.w, h = hs.h, mrows = (w + 31) / 32;
     volatile int* flags = hs.flags;
-    static const bool dbg = getenv("RTGS_DEBUG_BANDS") != nullptr;
-    static int dbg_frame = 0;
-    struct timespec ts0; clock_gettime(CLOCK_MONOTONIC, &ts0);
-    auto now_us = [&]() { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t); return (t.tv_sec - ts0.tv_sec) * 1e6 + (t.tv_nsec - ts0.tv_nsec) * 1e-3; };
-    double tflag[RTGS_MAX_BANDS];
     int qi = 0;
     for (int b = 0; b < nb; ++b) {
         long spins = 0;
         while (flags[b] == 0) {
             if ((++spins & 0xfff) == 0 && cudaEventQuery(hs.done) != cudaErrorNotReady) break;   // done or failed
         }
-        tflag[b] = now_us();
-        // the band's schedule positions -> macro-tile columns (edges inwards, render_common.cuh): at most two
-        // contiguous runs of columns
+        // the band's schedule positions -> macro-tile columns (rotated, render_common.cuh): at most two contiguous
+        // runs of columns
         const int p0 = b * bmc, p1 = (b + 1) * bmc < mrows ? (b + 1) * bmc : mrows;
         int lo[2] = {mrows, mrows}, hi[2] = {-1, -1};      // two runs: columns left / right of the middle
         for (int p = p0; p < p1; ++p) {
-            const int col = rtgs_dev::macro_column(mrows, p, hs.sched), k = col * 2 >= mrows ? 1 : 0;
+            const int col = rtgs_dev::macro_column(mrows, p, 2), k = col * 2 >= mrows ? 1 : 0;
             lo[k] = col < lo[k] ? col : lo[k];
             hi[k] = col > hi[k] ? col : hi[k];
         }
@@ -916,8 +875,6 @@ static int collect_banded(rtgs_scene* s) {
             if (hi[k] < 0) continue;
             const size_t c0 = (size_t)lo[k] * 32, c1 = (size_t)(hi[k] + 1) * 32 < (size_t)w ? (size_t)(hi[k] + 1) * 32 : (size_t)w;
             cudaStream_t cs = (qi++ & 1) ? s->copy_stream2 : s->copy_stream;
-            static const bool nocopy = getenv("RTGS_BAND_NOCOPY") != nullptr;   // experiment: no DMA at all
-            if (nocopy) continue;
             CUDA_TRY(cudaMemcpyAsync(hs.host_rgb + c0 * h * 3, hs.stage_rgb + c0 * h * 3,
                                      (c1 - c0) * h * 3 * sizeof(float), cudaMemcpyDeviceToHost, cs));
             if (hs.host_T)
@@ -925,16 +882,9 @@ static int collect_banded(rtgs_scene* s) {
                                          cudaMemcpyDeviceToHost, cs));
         }
     }
-    const double t_enq = now_us();
     CUDA_TRY(cudaEventSynchronize(hs.done));
-    const double t_k = now_us();
     CUDA_TRY(cudaStreamSynchronize(s->copy_stream));
     CUDA_TRY(cudaStreamSynchronize(s->copy_stream2));
-    if (dbg && ++dbg_frame == 20) {
-        fprintf(stderr, "bands %d: enq_done %.0f kernels_done %.0f copies_done %.0f us; flags:", nb, t_enq, t_k, now_us());
-        for (int b = 0; b < nb; ++b) fprintf(stderr, " %.0f", tflag[b]);
-        fprintf(stderr, "\n");
-    }
     return RTGS_OK;
 }
 
@@ -949,8 +899,7 @@ static int submit_whole(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32
     TRY(ensure_stage(hs, px));
     // the two frames in flight render on alternating streams (each with its own frame scratch, render.cu), so the
     // head of frame f+1 overlaps the tail of frame f on the device
-    static const bool one_stream = getenv("RTGS_SUBMIT_ONE_STREAM") != nullptr;   // experiment: serialised renders
-    cudaStream_t rs = (s->host_head == 0 || one_stream) ? s->own_stream : s->own_stream2;
+    cudaStream_t rs = s->host_head == 0 ? s->own_stream : s->own_stream2;
     TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, nullptr,
                            rs, false));
     CUDA_TRY(cudaEventRecord(hs.done, rs));
@@ -977,8 +926,6 @@ int rtgs_render_host_submit(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, i
         rtgs_set_error("rtgs_render_host_submit: the destination must be pinned host memory (rtgs_host_alloc)");
         return RTGS_ERR_INVALID;
     }
-    static const bool banded = getenv("RTGS_SUBMIT_BANDED") != nullptr;   // experiment: band pipeline here too
-    if (banded) return submit_banded(s, cam, x0, y0, w, h, depth, t_cut, host_rgb, host_T);
     return submit_whole(s, cam, x0, y0, w, h, depth, t_cut, host_rgb, host_T);
 }
 
@@ -1044,31 +991,18 @@ int rtgs_render_host(rtgs_scene* s, const rtgs_camera* cam, int32_t x0, int32_t 
         return RTGS_ERR_STATE;
     }
     DeviceGuard g(s->device);
-    const size_t px = (size_t)w * h;
-    cudaStream_t st = s->own_stream;
-    float* d_rgb = (float*)pinned_device_ptr(host_rgb);
-    float* d_T = host_T ? (float*)pinned_device_ptr(host_T) : nullptr;
-    const bool pinned = d_rgb != nullptr && (!host_T || d_T != nullptr);
-    if (pinned && host_mode() == 1) {
-        // zero-copy: the render kernel writes the framebuffer into mapped host memory
-        TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, d_rgb, d_T, nullptr, st, false));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        return RTGS_OK;
-    }
-    if (pinned && host_mode() == 2) {
+    if (pinned_device_ptr(host_rgb) && (!host_T || pinned_device_ptr(host_T))) {
+        // a pinned destination: the band copies run while the later bands are still rendering
         TRY(submit_banded(s, cam, x0, y0, w, h, depth, t_cut, host_rgb, host_T));
         return collect_banded(s);
     }
+    // pageable memory: render, one DMA into the scene's pinned buffer, then a host copy
+    const size_t px = (size_t)w * h;
+    cudaStream_t st = s->own_stream;
     rtgs_scene::HostSlot& hs = s->host_slot[0];
     TRY(ensure_stage(hs, px));
     TRY(rtgs_launch_render(s, cam, x0, y0, w, h, depth, t_cut, 0, 0, hs.stage_rgb, host_T ? hs.stage_T : nullptr, nullptr,
                            st, false));
-    if (pinned) {
-        CUDA_TRY(cudaMemcpyAsync(host_rgb, hs.stage_rgb, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (host_T) CUDA_TRY(cudaMemcpyAsync(host_T, hs.stage_T, px * sizeof(float), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        return RTGS_OK;
-    }
     TRY(ensure_pinned(s, px));
     CUDA_TRY(cudaMemcpyAsync(s->pinned_rgb, hs.stage_rgb, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (host_T) CUDA_TRY(cudaMemcpyAsync(s->pinned_T, hs.stage_T, px * sizeof(float), cudaMemcpyDeviceToHost, st));

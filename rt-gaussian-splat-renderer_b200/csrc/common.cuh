@@ -83,7 +83,6 @@ struct rtgs_scene {
     // packed render records
     float4* geo = nullptr;
     float4* shp = nullptr;
-    cudaTextureObject_t geo_tex = 0;   // (experiment) geo as a linear float4 texture
     cudaTextureObject_t shp_tex = 0;   // shp as a linear float4 texture (eval_colour); 0 when the scene exceeds one texture
     float4* raw = nullptr;
     float4* nodes = nullptr;
@@ -130,8 +129,8 @@ struct rtgs_scene {
     int64_t opt_pool_chunks = -1;             // RTGS_OPT_LIST_POOL_CHUNKS (-1 = default sizing)
     int opt_stripe_mod = 1, opt_stripe_rem = 0;   // RTGS_OPT_STRIPE
     int opt_render_mode = -1;                 // RTGS_OPT_RENDER_MODE (-1 = RTGS_RENDER_MODE env or 0)
-    int opt_heavy_lists = -1;                 // RTGS_OPT_HEAVY_LISTS (-1 = RTGS_HEAVY_SLAB env or 1)
-    int opt_heavy_limit = -1;                 // RTGS_OPT_HEAVY_LIMIT (-1 = RTGS_HEAVY_LIMIT env or the shared-memory capacity)
+    int opt_heavy_lists = -1;                 // RTGS_OPT_HEAVY_LISTS (-1 = 0)
+    int opt_heavy_limit = -1;                 // RTGS_OPT_HEAVY_LIMIT (-1 = the shared-memory capacity)
     // rtgs_render_host: device staging + band flags, double-buffered so that two frames can be in flight
     // (rtgs_render_host_submit / _collect: frame f+1 renders while the last bands of frame f are copied out)
     struct HostSlot {
@@ -144,7 +143,7 @@ struct rtgs_scene {
         int* flags_dev = nullptr;
         cudaEvent_t done = nullptr;           // recorded behind the frame's last kernel
         cudaEvent_t copied = nullptr;         // recorded behind the frame's whole-image DMA (pipelined delivery)
-        int nb = 0, bmc = 0, sched = 0, w = 0, h = 0;
+        int nb = 0, bmc = 0, w = 0, h = 0;
         float* host_rgb = nullptr;
         float* host_T = nullptr;
     };
@@ -163,7 +162,6 @@ struct rtgs_scene {
     int* band_flags_dev = nullptr;            // device alias of band_flags
     int bands_active = 0;                     // set by rtgs_render_host around its launch
     int band_macro_cols = 0;
-    int band_schedule = 0;                    // macro-column order of the banded launch (render_common.cuh)
 
     // per-kernel timing ring (RTGS_OPT_KERNEL_TIMING): 4 events per frame slot
     std::vector<cudaEvent_t> timing_events;

@@ -23,8 +23,8 @@
 // distance and alpha.  Hits are appended to a per-lane K-entry buffer in shared memory (replace-max
 // when full); after the traversal each lane ranks its entries and composites front to back.
 //
-// It renders depth > 16 (K = 32), RTGS_OPT_RENDER_MODE = 1, and - launched behind the list kernels, by the host
-// or by k_frame's last CTA as a device-side tail launch - the tiles on the fallback list.
+// It renders depth > 16 (K = 32), RTGS_OPT_RENDER_MODE = 1, and - launched behind the list kernels - the tiles on
+// the two hand-over lists.
 //
 // Numerics.  The reference's f32 formulation (B^2 - 4AC with a cofactor inverse) is ill-conditioned
 // (SURVEY.md §7 hard part 1), and parity is defined against a float64 evaluation of the
@@ -38,30 +38,11 @@
 namespace rtgs_dev {
 namespace fused {
 
-#ifndef FUSED_POP_PRUNE
-#define FUSED_POP_PRUNE 0     // 1: a stacked node is tested against the CURRENT cut again when it is popped (measured: 1.335 -> 1.364 ms)
-#endif
-#ifndef FUSED_NARROW_START
-#define FUSED_NARROW_START 0  // n > 0: n nodes per step while no ray is closed yet (measured: 8 -> 1.77 ms, 4 -> 1.94 ms vs 1.335)
-#endif
-#ifndef RTGS_STACK_CAP
-#define RTGS_STACK_CAP 512
-#endif
-constexpr int STACK_CAP = RTGS_STACK_CAP;
-#ifndef FUSED_TWO_LEVEL
-#define FUSED_TWO_LEVEL 0     // 1: a step pops two-level nodes (four grandchild boxes per lane; measured on the surface-like
-                              // scene: 1.368 -> 1.396 ms, fewer steps but as many instructions), 0: binary nodes
-#endif
-// Above STACK_SINGLE the traversal pops one node at a time (depth first).  Binary nodes: a batch step grows the stack
-// by <= 32 (two children per popped node), a single pop by <= 1 per level descended, i.e. by <= RTGS_MAX_TREE_DEPTH in
-// all.  Two-level nodes: <= 3 x 32 per batch step, <= 3 per single pop, which descends two levels.
-#if FUSED_TWO_LEVEL
-constexpr int STACK_SINGLE = STACK_CAP - 96 - 3 * ((RTGS_MAX_TREE_DEPTH + 1) / 2);
-constexpr int CQ_CAP = 160;   // < 32 waiting + <= 128 leaves of one step
-#else
+constexpr int STACK_CAP = 512;
+// Above STACK_SINGLE the traversal pops one node at a time (depth first).  A batch step grows the stack by <= 32 (two
+// children per popped node), a single pop by <= 1 per level descended, i.e. by <= RTGS_MAX_TREE_DEPTH in all.
 constexpr int STACK_SINGLE = STACK_CAP - 32 - RTGS_MAX_TREE_DEPTH;
 constexpr int CQ_CAP = 96;
-#endif
 static_assert(STACK_SINGLE >= 64, "k_render: stack too small for batched traversal");
 constexpr int BATCH = REC_BATCH;
 
@@ -70,9 +51,6 @@ struct __align__(16) TraversalScratch {
     float4 polyA[BATCH];        // coarse quadratics {c0 c1 c2 c3}
     float4 polyB[BATCH];        //                   {c4 c5 t_lo -}: t_lo = no ray of the tile enters the candidate before it
     int stack[STACK_CAP];
-#if FUSED_POP_PRUNE
-    float sdist[STACK_CAP];     // squared distance of the stacked node's box from the camera (pruned again when popped)
-#endif
     int cq[CQ_CAP];
     Frustum open;               // pyramid of the rays that still lack hits (distance pruning, below)
 };
@@ -104,13 +82,13 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
     const unsigned lt_mask = (1u << lane) - 1u;
     const CamD& cam = P.cam;
     const int xe = P.x0 + P.w, ye = P.y0 + P.h;
-    // work items: every tile id, or (fallback mode) the tiles the traversal and / or the shading handed over
-    const int n1 = (P.use_fallback_list & 1) ? (int)min(P.counters[CTR_FALLBACK], (unsigned)P.ntiles) : 0;
-    const int n2 = (P.use_fallback_list & 2) ? (int)min(P.counters[CTR_FALLBACK2], (unsigned)P.ntiles) : 0;
-    unsigned int* const cursor = P.counters + (P.use_fallback_list == 2 ? CTR_WORK4 : CTR_WORK3);
-    if (P.early_trigger) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    // work items: every tile id (cursor CTR_WORK2, as for the shading), or (fallback mode) the tiles the traversal,
+    // then the shading handed over (cursor CTR_WORK3)
+    const int n1 = P.use_fallback_list ? (int)min(P.counters[CTR_FALLBACK], (unsigned)P.ntiles) : 0;
+    const int n2 = P.use_fallback_list ? (int)min(P.counters[CTR_FALLBACK2], (unsigned)P.ntiles) : 0;
+    unsigned int* const cursor = P.counters + (P.use_fallback_list ? CTR_WORK3 : CTR_WORK2);
 
-    if ((P.use_fallback_list & 1) && blockIdx.x == 0 && threadIdx.x == 0) {
+    if (P.use_fallback_list && blockIdx.x == 0 && threadIdx.x == 0) {
         // pool demand of this frame (for the host's sizing) and whether any frame so far needed the fallback
         *reinterpret_cast<volatile int*>(P.mirror) = (int)min(P.counters[CTR_POOL], 0x7fffffffu);
         if (P.counters[CTR_FALLBACK] != 0) *reinterpret_cast<volatile int*>(P.mirror + 1) = 1;
@@ -193,97 +171,20 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
         };
 
         int top = 1, ncq = 0;
-        if (lane == 0) {
-            tr.stack[0] = 0;
-#if FUSED_POP_PRUNE
-            tr.sdist[0] = 0.0f;
-#endif
-        }
+        if (lane == 0) tr.stack[0] = 0;
         __syncwarp();
 
         // ================================ traversal ==========================================
 #pragma unroll 1
         while (top > 0 || ncq > 0) {
             if (top > 0) {
-                const int wide = (FUSED_NARROW_START > 0 && cut2 < 0.0f) ? FUSED_NARROW_START : 32;
-                const int take = top > STACK_SINGLE ? 1 : min(wide, top);
+                const int take = top > STACK_SINGLE ? 1 : min(32, top);
                 int node = -1;
-                if (lane < take) {
-                    node = tr.stack[top - 1 - lane];
-#if FUSED_POP_PRUNE
-                    // the cut may have tightened since this node was pushed: beyond it (and no open ray left) it is
-                    // dropped without fetching its record.  (With open rays it is kept: its box was inside their
-                    // pyramid or inside the cut when it was pushed, and the children are tested against both again.)
-                    if (cut2 >= 0.0f && open_mask == 0 && tr.sdist[top - 1 - lane] > cut2) node = -1;
-#endif
-                }
+                if (lane < take) node = tr.stack[top - 1 - lane];
                 top -= take;
                 __syncwarp();
-#if FUSED_TWO_LEVEL
-                // every lane takes a whole two-level node (lbvh.cu: k_pack_nodes4: the records of both children side
-                // by side): four grandchild boxes per lane, one step descends two tree levels - half as many
-                // dependent steps per tile, which is what a tile that looks along a surface is made of
-                bool hb[4];
-                int cb[4];
-                float db[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) { hb[k] = false; cb[k] = 0; db[k] = 0.0f; }
-                if (node >= 0) {
-                    const float4* rec = P.nodes4 + (int64_t)node * 8;
-                    float4 q[8];
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) ldg256(rec + 2 * k, q[2 * k], q[2 * k + 1]);   // all four loads in flight
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const float4 a = q[4 * h], b = q[4 * h + 1], c = q[4 * h + 2], d = q[4 * h + 3];
-                        cb[2 * h] = __float_as_int(d.x);
-                        cb[2 * h + 1] = __float_as_int(d.y);
-                        hb[2 * h] = box_in_frustum(fr, a.x, a.y, a.z, a.w, b.x, b.y);
-                        hb[2 * h + 1] = box_in_frustum(fr, b.z, b.w, c.x, c.y, c.z, c.w);
-                        db[2 * h] = box_dist2(a.x, a.y, a.z, a.w, b.x, b.y);
-                        db[2 * h + 1] = box_dist2(b.z, b.w, c.x, c.y, c.z, c.w);
-                        if (cut2 >= 0.0f) {
-                            if (hb[2 * h] && db[2 * h] > cut2)
-                                hb[2 * h] = open_mask != 0 && (open_all || box_in_frustum(tr.open, a.x, a.y, a.z, a.w, b.x, b.y));
-                            if (hb[2 * h + 1] && db[2 * h + 1] > cut2)
-                                hb[2 * h + 1] = open_mask != 0 && (open_all || box_in_frustum(tr.open, b.z, b.w, c.x, c.y, c.z, c.w));
-                        }
-                    }
-                    // farthest first (pushed first, popped last): sorting network on four
-                    auto cswap = [&](int i, int j) {
-                        if (db[i] < db[j]) {
-                            const float td = db[i]; db[i] = db[j]; db[j] = td;
-                            const int tc = cb[i]; cb[i] = cb[j]; cb[j] = tc;
-                            const bool th = hb[i]; hb[i] = hb[j]; hb[j] = th;
-                        }
-                    };
-                    cswap(0, 1); cswap(2, 3); cswap(0, 2); cswap(1, 3); cswap(1, 2);
-                }
-                ST(st_nodes += 4ull * (unsigned)take);
-                ST(st_steps += 1);
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const bool in = hb[k] && cb[k] >= 0;
-                    const unsigned m = __ballot_sync(FULL, in);
-                    if (in) {
-                        tr.stack[top + __popc(m & lt_mask)] = cb[k];
-#if FUSED_POP_PRUNE
-                        tr.sdist[top + __popc(m & lt_mask)] = db[k];
-#endif
-                    }
-                    top += __popc(m);
-                }
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const bool lf = hb[k] && cb[k] < 0;
-                    const unsigned m = __ballot_sync(FULL, lf);
-                    if (lf) tr.cq[ncq + __popc(m & lt_mask)] = ~cb[k];
-                    ncq += __popc(m);
-                }
-#else
                 bool h0 = false, h1 = false;
                 int c0 = 0, c1 = 0;
-                float dd0 = 0.0f, dd1 = 0.0f;
                 if (node >= 0) {
                     float4 a, b, c, d;
                     ldg256(P.nodes + (int64_t)node * 4 + 0, a, b);
@@ -294,7 +195,6 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                     h1 = box_in_frustum(fr, b.z, b.w, c.x, c.y, c.z, c.w);
                     const float d0 = box_dist2(a.x, a.y, a.z, a.w, b.x, b.y);
                     const float d1 = box_dist2(b.z, b.w, c.x, c.y, c.z, c.w);
-                    dd0 = d0; dd1 = d1;
                     if (cut2 >= 0.0f) {
                         if (h0 && d0 > cut2)
                             h0 = open_mask != 0 && (open_all || box_in_frustum(tr.open, a.x, a.y, a.z, a.w, b.x, b.y));
@@ -304,32 +204,20 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
                     if (d1 > d0) {   // child 1 is pushed last, i.e. popped first: make it the nearer one
                         const int ci = c0; c0 = c1; c1 = ci;
                         const bool hi = h0; h0 = h1; h1 = hi;
-                        const float di = dd0; dd0 = dd1; dd1 = di;
                     }
                 }
                 ST(st_nodes += 2ull * (unsigned)take);
                 ST(st_steps += 1);
                 const unsigned mI0 = __ballot_sync(FULL, h0 && c0 >= 0), mI1 = __ballot_sync(FULL, h1 && c1 >= 0);
                 const unsigned mL0 = __ballot_sync(FULL, h0 && c0 < 0), mL1 = __ballot_sync(FULL, h1 && c1 < 0);
-                if (h0 && c0 >= 0) {
-                    tr.stack[top + __popc(mI0 & lt_mask)] = c0;
-#if FUSED_POP_PRUNE
-                    tr.sdist[top + __popc(mI0 & lt_mask)] = dd0;
-#endif
-                }
+                if (h0 && c0 >= 0) tr.stack[top + __popc(mI0 & lt_mask)] = c0;
                 const int topa = top + __popc(mI0);
-                if (h1 && c1 >= 0) {
-                    tr.stack[topa + __popc(mI1 & lt_mask)] = c1;
-#if FUSED_POP_PRUNE
-                    tr.sdist[topa + __popc(mI1 & lt_mask)] = dd1;
-#endif
-                }
+                if (h1 && c1 >= 0) tr.stack[topa + __popc(mI1 & lt_mask)] = c1;
                 top = topa + __popc(mI1);
                 if (h0 && c0 < 0) tr.cq[ncq + __popc(mL0 & lt_mask)] = ~c0;
                 const int ncqa = ncq + __popc(mL0);
                 if (h1 && c1 < 0) tr.cq[ncqa + __popc(mL1 & lt_mask)] = ~c1;
                 ncq = ncqa + __popc(mL1);
-#endif
                 ST(st_max_stack = max(st_max_stack, (unsigned)top));
                 __syncwarp();
             }
@@ -642,7 +530,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (K <= 16 ? 2 : 1)) k_rende
         }
         if (lane == 0) atomicMax(P.stats + ST_MAX_FUSED_STACK, (unsigned long long)st_max_stack);
     }
-    if (P.final_kernel) cta_finish(P, P.use_fallback_list == 1 ? CTR_DONE3 : CTR_DONE2);
+    if (P.final_kernel) cta_finish(P, CTR_DONE2);
 }
 #undef ST
 

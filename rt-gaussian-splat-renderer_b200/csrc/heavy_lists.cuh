@@ -14,7 +14,7 @@
 //      entry distances of its 16 nearest hits;
 //   3. while some ray holds fewer than 16 hits, or its 16th hit lies behind the nearest deferred depth, the cap is
 //      raised and the deferred list re-scanned.  The new cap is a rank statistic of the deferred depths (the
-//      slab_rank-th smallest of the 32 lanes' nearest deferred depths), so a pass activates a few dozen entries
+//      SLAB_RANK-th smallest of the 32 lanes' nearest deferred depths), so a pass activates a few dozen entries
 //      whatever the local density: no steps through empty space, no plunge into a surface; a pass that overflows
 //      the shared list is repeated with a nearer cap.
 //
@@ -42,6 +42,9 @@ constexpr int HEAVY_K = 16;              // hits a ray keeps (the k-buffer depth
 constexpr int HEAVY_MAX_ITERS = 128;     // passes per tile before it is handed to the fused kernel
 constexpr int HEAVY_LIST_LIMIT = GLIST_CAP - 4 * LISTS_TAKE;
 constexpr float HEAVY_MARGIN = 1.0001f;  // limit = farthest 16th hit x this (float32 rounding of depths and distances)
+// The cap of a pass is the SLAB_RANK-th smallest of the 32 lanes' nearest deferred depths (surface-like scene, heavy
+// lists from the first frame: 2.48 ms per frame at 24, 2.54 ms at 16; profiles/r02_heavy_lists_probe.log).
+constexpr int SLAB_RANK = 24;
 
 struct __align__(16) HeavyShared {
     ListsShared l;                         // traversal stack, the tile's candidates so far, output queue
@@ -259,7 +262,7 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
     __syncwarp();
     drain(-INFINITY, -INFINITY);
     // The cap of a pass comes from the depths of what is deferred: every lane remembers the nearest depth among the
-    // entries it deferred itself (entries are spread over the lanes as they come), and the cap is the slab_rank-th
+    // entries it deferred itself (entries are spread over the lanes as they come), and the cap is the SLAB_RANK-th
     // smallest of those 32 values - so a pass activates a few dozen entries whatever the local density is: no steps
     // through empty space, no plunge into a surface.  The first pass of a tile whose neighbour has just been walked
     // goes straight to that tile's limit (`hint`).
@@ -270,7 +273,7 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
     float want = INFINITY;   // the farthest HEAVY_K-th hit x HEAVY_MARGIN
 #pragma unroll 1
     while (!failed) {
-        // what the pass deferred: count n_out, nearest depth zm, slab_rank-th of the lanes' nearest depths zr
+        // what the pass deferred: count n_out, nearest depth zm, SLAB_RANK-th of the lanes' nearest depths zr
         ST(HS.max_deferred = max(HS.max_deferred, (unsigned)n_out));
         float zs = zmin;
 #pragma unroll
@@ -283,7 +286,7 @@ __device__ __noinline__ float heavy_tile(const RenderParams& P, HeavyShared& hs,
             }
         }
         const float zm = __shfl_sync(FULL, zs, 0);
-        float zr = __shfl_sync(FULL, zs, P.slab_rank);
+        float zr = __shfl_sync(FULL, zs, SLAB_RANK);
         if (!(zr < INFINITY)) {                  // fewer lanes than that hold entries: the farthest of them
             float f = zs < INFINITY ? zs : -INFINITY;
 #pragma unroll

@@ -14,9 +14,10 @@
 //                  publication of its tile's group).  Claims are ordered - a tile is only ever claimed after its
 //                  group - so a waiting warp always waits for a warp that is running.  No kernel boundary inside the
 //                  frame: the lowest LATENCY of a single frame that is spread over >= 4 GPUs (few groups per SM).
-//                  The last CTA completes the frame: it mirrors the list-pool demand to the host, tail-launches the
-//                  fused kernel from the device (RTGS_CDP builds) if some tile went to a hand-over list, signals the
-//                  `arrive` counter of a multi-GPU gather and zeroes the work counters for the next frame.
+//                  Its last CTA mirrors the list-pool demand to the host.  The host queues k_render behind it for the
+//                  tiles on the hand-over lists (it returns at once when they are empty); that launch completes the
+//                  frame: it signals the `arrive` counter of a multi-GPU gather and zeroes the work counters for the
+//                  next frame.
 //   k_heavy_lists  (mode 0, opt-in RTGS_OPT_HEAVY_LISTS) depth-capped lists for the tiles of groups whose frustum overflows
 //                  the traversal's shared-memory list (heavy_lists.cuh), between k_tile_lists and k_shade_tiles
 //   k_render       fused.cuh (mode 1, depth > 16, fallback tiles)
@@ -31,10 +32,6 @@
 #include "heavy_lists.cuh"
 #include "shade.cuh"
 #include "tile_lists.cuh"
-
-#ifndef RTGS_CDP
-#define RTGS_CDP 0   // 1: k_frame tail-launches k_render from the device (needs -rdc=true and cudadevrt)
-#endif
 
 using namespace rtgs_dev;
 using rtgs_dev::fused::k_render;
@@ -106,21 +103,12 @@ __device__ __forceinline__ void flush_shade_stats(const RenderParams& P, const S
 }
 
 // ---- mode 0: the two halves as separate launches -------------------------------------------------------------
-#ifndef K1_CTAS
-#define K1_CTAS 4
-#endif
-#ifndef LISTS_STATIC_SMEM
-#define LISTS_STATIC_SMEM (LISTS_STACK_ENTRIES <= 320)   // 8 warps x (stack + 960 + 256) ints fit the 48 KB static limit
-#endif
+constexpr int K1_CTAS = 4;
+static_assert(sizeof(ListsShared) * WARPS_PER_CTA <= 48 * 1024, "k_tile_lists: static shared-memory limit");
 template <bool STATS>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, K1_CTAS) k_tile_lists(const __grid_constant__ RenderParams P) {
-#if LISTS_STATIC_SMEM
     __shared__ ListsShared smem[WARPS_PER_CTA];
     ListsShared& ws = smem[threadIdx.x >> 5];
-#else
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    ListsShared& ws = reinterpret_cast<ListsShared*>(smem_raw)[threadIdx.x >> 5];
-#endif
     const int lane = threadIdx.x & 31;
     ListsState S;
     const int ngroups = P.ntiles / TILES_PER_GROUP;
@@ -178,12 +166,8 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, HEAVY_CTAS) k_heavy_lists(
     }
 }
 
-#ifndef K2_WARPS
-#define K2_WARPS 10
-#endif
-#ifndef K2_CTAS
-#define K2_CTAS 2
-#endif
+constexpr int K2_WARPS = 10;
+constexpr int K2_CTAS = 2;
 constexpr int SHADE_WARPS = K2_WARPS;   // warps per CTA
 static_assert(sizeof(ShadeShared) * K2_WARPS * K2_CTAS <= 227 * 1024, "shared-memory budget per SM");
 
@@ -290,21 +274,6 @@ __global__ void __launch_bounds__(SHADE_WARPS * 32, K2_CTAS) k_frame(const __gri
                        fb = __ldcg(P.counters + CTR_FALLBACK) + __ldcg(P.counters + CTR_FALLBACK2);
         *reinterpret_cast<volatile int*>(P.mirror) = (int)min(pool, 0x7fffffffu);
         if (fb != 0) *reinterpret_cast<volatile int*>(P.mirror + 1) = 1;
-#if RTGS_CDP
-        if (P.tail_launch && fb != 0) {
-            // device-side tail launch: runs when this grid has finished, before anything queued behind it on the
-            // stream; the fused kernel's last CTA completes the frame instead
-            RenderParams Q = P;
-            Q.use_fallback_list = 3;
-            Q.final_kernel = 1;
-            int grid = (int)min((fb + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (unsigned)P.tail_grid);
-            k_render<16, STATS, DEPTH><<<grid, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<16>) * WARPS_PER_CTA,
-                                         cudaStreamTailLaunch>>>(Q);
-        } else
-#endif
-        if (P.final_kernel) {
-            frame_complete(P);
-        }
     }
 }
 
@@ -462,25 +431,18 @@ int persistent_blocks(rtgs_scene* s, Kernel kernel, int threads, size_t smem, in
             return RTGS_ERR_CUDA;
         }
         cache[dev] = nb;
-        if (getenv("RTGS_DEBUG_OCC")) fprintf(stderr, "rtgs: %s: %d CTAs/SM, %zu B dynamic smem\n", name, nb, smem);
     }
     *out = cache[dev];
     return RTGS_OK;
 }
 
 template <int K, bool STATS, bool DEPTH>
-int prepare_render_k(rtgs_scene* s, int* blocks) {
-    static int cache[16] = {0};
-    return persistent_blocks(s, k_render<K, STATS, DEPTH>, WARPS_PER_CTA * 32, sizeof(fused::WarpShared<K>) * WARPS_PER_CTA,
-                             cache, "k_render", blocks);
-}
-
-template <int K, bool STATS, bool DEPTH>
 int launch_render_k(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const RenderParams& P, cudaStream_t stream) {
-    int nb = 0;
-    int r = prepare_render_k<K, STATS, DEPTH>(s, &nb);
-    if (r != RTGS_OK) return r;
+    static int cache[16] = {0};
     const size_t smem = sizeof(fused::WarpShared<K>) * WARPS_PER_CTA;
+    int nb = 0;
+    int r = persistent_blocks(s, k_render<K, STATS, DEPTH>, WARPS_PER_CTA * 32, smem, cache, "k_render", &nb);
+    if (r != RTGS_OK) return r;
     int grid = s->sm_count * nb;
     const int need = (P.ntiles + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
     if (grid > need) grid = need;
@@ -489,8 +451,7 @@ int launch_render_k(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const Ren
         // fallback tiles it runs on a quarter of the SMs (a cheaper launch); the first frame that does overflow
         // is still rendered correctly, just with fewer warps on its fallback tiles.
         const int seen = *reinterpret_cast<volatile int*>(fs.mirror + 1);
-        static const char* e = getenv("RTGS_FB_GRID");
-        const int small = e ? atoi(e) : (s->sm_count + 3) / 4;
+        const int small = (s->sm_count + 3) / 4;
         if (!seen && grid > small) grid = small;
     }
     if (grid < 1) grid = 1;
@@ -507,15 +468,14 @@ int launch_fused(rtgs_scene* s, const rtgs_scene::FrameScratch& fs, const Render
 template <bool STATS>
 int launch_tile_lists(rtgs_scene* s, const RenderParams& P, cudaStream_t stream) {
     static int cache[16] = {0};
-    const size_t smem = LISTS_STATIC_SMEM ? 0 : sizeof(ListsShared) * WARPS_PER_CTA;
     int nb = 0;
-    int r = persistent_blocks(s, k_tile_lists<STATS>, WARPS_PER_CTA * 32, smem, cache, "k_tile_lists", &nb);
+    int r = persistent_blocks(s, k_tile_lists<STATS>, WARPS_PER_CTA * 32, 0, cache, "k_tile_lists", &nb);
     if (r != RTGS_OK) return r;
     int grid = s->sm_count * nb;
     const int need = (P.ntiles / TILES_PER_GROUP + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
     if (grid > need) grid = need;
     if (grid < 1) grid = 1;
-    k_tile_lists<STATS><<<grid, WARPS_PER_CTA * 32, smem, stream>>>(P);
+    k_tile_lists<STATS><<<grid, WARPS_PER_CTA * 32, 0, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
@@ -550,7 +510,7 @@ int launch_heavy_lists(rtgs_scene* s, rtgs_scene::FrameScratch& fs, RenderParams
 }
 
 template <bool STATS, bool DEPTH>
-int launch_shade_tiles(rtgs_scene* s, const RenderParams& P, cudaStream_t stream, bool dependent) {
+int launch_shade_tiles(rtgs_scene* s, const RenderParams& P, cudaStream_t stream) {
     static int cache[16] = {0};
     const size_t smem = sizeof(ShadeShared) * SHADE_WARPS;
     int nb = 0;
@@ -560,39 +520,18 @@ int launch_shade_tiles(rtgs_scene* s, const RenderParams& P, cudaStream_t stream
     const int need = (P.ntiles + SHADE_WARPS - 1) / SHADE_WARPS;
     if (grid > need) grid = need;
     if (grid < 1) grid = 1;
-    if (dependent) {
-        // programmatic dependent launch: may start as soon as the previous kernel on the stream has let its
-        // dependents go (fused.cuh: early_trigger); k_shade_tiles never waits for that kernel
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)grid);
-        cfg.blockDim = dim3(SHADE_WARPS * 32);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, k_shade_tiles<STATS, DEPTH>, P));
-        return RTGS_OK;
-    }
     k_shade_tiles<STATS, DEPTH><<<grid, SHADE_WARPS * 32, smem, stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return RTGS_OK;
 }
 
 template <bool STATS, bool DEPTH>
-int launch_frame(rtgs_scene* s, RenderParams& P, cudaStream_t stream) {
+int launch_frame(rtgs_scene* s, const RenderParams& P, cudaStream_t stream) {
     static int cache[16] = {0};
     const size_t smem = sizeof(FrameShared) * SHADE_WARPS;
     int nb = 0;
     int r = persistent_blocks(s, k_frame<STATS, DEPTH>, SHADE_WARPS * 32, smem, cache, "k_frame", &nb);
     if (r != RTGS_OK) return r;
-    if (P.tail_launch) {   // the device-side launch of the fused kernel needs its shared memory opted in as well
-        int nbk = 0;
-        if ((r = prepare_render_k<16, STATS, DEPTH>(s, &nbk)) != RTGS_OK) return r;
-        P.tail_grid = s->sm_count * nbk;
-    }
     int grid = s->sm_count * nb;
     // a warp does one group and four tiles per round: more warps than groups would only spin
     const int need = (P.ntiles / TILES_PER_GROUP + SHADE_WARPS - 1) / SHADE_WARPS;
@@ -622,32 +561,9 @@ int render_mode(const rtgs_scene* s) {
 // Heavy groups (heavy_lists.cuh): 0 (default) = the fused kernel renders their tiles, 1 = depth-capped lists once the
 // scene has shown heavy groups, 2 = from the first frame on.  Off by default: on the surface-like scene the two routes
 // cost the same (DESIGN.md §8), and the fused kernel is the simpler one.
-int rtgs_heavy_lists_mode(const rtgs_scene* s) {
-    if (s->opt_heavy_lists >= 0) return s->opt_heavy_lists;
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("RTGS_HEAVY_SLAB");
-        mode = e ? atoi(e) : 0;
-        if (mode < 0 || mode > 2) mode = 0;
-    }
-    return mode;
-}
+int rtgs_heavy_lists_mode(const rtgs_scene* s) { return s->opt_heavy_lists >= 0 ? s->opt_heavy_lists : 0; }
 
 namespace {
-// k_frame's fallback tiles: 1 (default) = its last CTA tail-launches the fused kernel from the device when there
-// are any; 0 = the host queues the fused kernel behind every frame (it returns at once when the list is empty).
-int tail_launch_mode() {
-#if !RTGS_CDP
-    return 0;   // built without relocatable device code: the host queues the fused kernel behind every frame
-#endif
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("RTGS_TAIL_LAUNCH");
-        mode = e ? (atoi(e) != 0) : 1;
-    }
-    return mode;
-}
-
 // Candidate-list scratch of a scene, sized for the tile count of the largest region rendered so far.
 // The pool starts at 16 chunks (496 candidates) per tile on average - tiles may take any share of it - and
 // doubles whenever the demand reported by the last finished frame (lists_group keeps counting past the end of
@@ -738,7 +654,6 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     P.geo = s->geo;
     P.shp = s->shp;
     P.shp_tex = s->shp_tex;
-    P.geo_tex = s->geo_tex;
     P.raw = s->raw;
     P.leafbox = s->leafbox;
     P.cam = make_camd(cam);
@@ -764,29 +679,20 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     P.fallback_tiles = nullptr;
     P.fallback_tiles2 = nullptr;
     P.use_fallback_list = 0;
-    P.early_trigger = 0;
     static const int heavy_fused = getenv("RTGS_HEAVY_FUSED") ? atoi(getenv("RTGS_HEAVY_FUSED")) : 1;
     P.heavy_fused = heavy_fused;
-    static const int heavy_limit = getenv("RTGS_HEAVY_LIMIT") ? atoi(getenv("RTGS_HEAVY_LIMIT")) : 1 << 30;
-    P.heavy_limit = s->opt_heavy_limit >= 0 ? s->opt_heavy_limit : heavy_limit;
+    P.heavy_limit = s->opt_heavy_limit >= 0 ? s->opt_heavy_limit : 1 << 30;   // default: the shared list's capacity
     P.heavy_slab = 0;
     P.heavy_groups = nullptr;
     P.tile_cap = nullptr;
     P.heavy_scratch = nullptr;
     P.heavy_defer_cap = 0;
-    static const int slab_rank = getenv("RTGS_SLAB_RANK") ? atoi(getenv("RTGS_SLAB_RANK")) : 24;
-    P.slab_rank = slab_rank < 0 ? 0 : (slab_rank > 31 ? 31 : slab_rank);
-    {
-        // batch threshold of the traversal stack: the tuned value, capped by what this tree's depth allows
-        static const int tuned = getenv("RTGS_LISTS_SINGLE") ? atoi(getenv("RTGS_LISTS_SINGLE")) : 112;
-        const int bound = lists_single_bound(s->max_depth);
-        P.lists_single = tuned < bound ? tuned : bound;
-        if (P.lists_single < 0) P.lists_single = 0;
-    }
+    // batch threshold of the traversal stack: the tuned value, capped by what this tree's depth allows (>= 4)
+    P.lists_single = min(LISTS_SINGLE, lists_single_bound(s->max_depth));
     P.nbands = 0;
     P.band_macro_cols = 1;
     P.macro_rows = mrows;
-    P.schedule = s->bands_active > 0 ? s->band_schedule : 0;
+    P.schedule = s->bands_active > 0 ? 2 : 0;
     P.band_done = s->band_done;
     P.band_flags = s->band_flags_cur_dev ? s->band_flags_cur_dev : s->band_flags_dev;
     P.mirror = fs.mirror_dev;
@@ -795,10 +701,8 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     P.arrive = s->sync_arrive;
     P.grant = s->sync_grant;
     P.grant_value = s->sync_grant_value;
-    P.tail_launch = 0;
     P.final_kernel = 0;
     P.self_clean = 0;
-    P.tail_grid = 0;
     P.out_depth = out_depth;
     // out_depth selects the DEPTH instantiation of every kernel that composites; without it the frame runs the kernels
     // of a plain render
@@ -854,22 +758,14 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
     if (mode == 2) {
         P.ready = fs.ready;
         P.seq = ++fs.frame_seq;
-        // banded host delivery counts tiles per band in both kernels: keep the host-side launch order there
-        const bool tail = tail_launch_mode() != 0;
-        P.tail_launch = tail ? 1 : 0;
-        P.final_kernel = tail ? 1 : 0;
-        P.self_clean = tail ? 1 : 0;
         if ((r = mark(0)) != RTGS_OK || (r = mark(1)) != RTGS_OK) return r;
         if ((r = RTGS_BY_FLAGS(launch_frame, s, P, stream)) != RTGS_OK) return r;
         if ((r = mark(2)) != RTGS_OK) return r;
-        if (ran) *ran = 2;
-        if (!tail) {
-            P.use_fallback_list = 3;
-            P.final_kernel = 1;
-            P.self_clean = 1;
-            if ((r = fused_kernel(16)) != RTGS_OK) return r;
-            if (ran) *ran = 6;
-        }
+        P.use_fallback_list = 1;
+        P.final_kernel = 1;
+        P.self_clean = 1;
+        if ((r = fused_kernel(16)) != RTGS_OK) return r;
+        if (ran) *ran = 6;
         return mark(3);
     }
     // Groups whose frustum overflows the traversal's shared-memory list ("heavy") go to the fused kernel.  With
@@ -888,31 +784,11 @@ static int launch_render_on(rtgs_scene* s, rtgs_scene::FrameScratch& fs, const r
         (r = want_stats ? launch_heavy_lists<true>(s, fs, P, stream) : launch_heavy_lists<false>(s, fs, P, stream)) != RTGS_OK)
         return r;
     if ((r = mark(1)) != RTGS_OK) return r;
-    // Tiles the traversal handed to the fused kernel (groups whose frustum holds ~1000 Gaussians or more, or a list
-    // pool that ran out) are known before the shading starts.  RTGS_HEAVY_OVERLAP=1 renders them FIRST and launches the
-    // shading as a programmatic dependent of that launch which it does not wait for, so that the fused kernel's tail
-    // runs underneath the shading.  Measured on the surface-like scene: 2.36 -> 2.26 ms for frames launched one
-    // after the other, but 1058 -> 948 Mrays/s for the two-stream sweep (frames already overlap there and the fused
-    // kernel holds whole SMs), so it is off by default.  The closing launch renders both hand-over lists.
-    static const bool overlap = getenv("RTGS_HEAVY_OVERLAP") != nullptr && atoi(getenv("RTGS_HEAVY_OVERLAP")) != 0;
-    const bool heavy_first = overlap && !want_stats && s->bands_active == 0 &&
-                             *reinterpret_cast<volatile int*>(fs.mirror + 1) != 0;
-    if (heavy_first) {
-        P.use_fallback_list = 1;
-        P.early_trigger = 1;
-        if ((r = RTGS_BY_FLAGS(launch_fused, s, fs, P, stream, 16)) != RTGS_OK) return r;
-        P.use_fallback_list = 0;
-        P.early_trigger = 0;
-        if ((r = RTGS_BY_FLAGS(launch_shade_tiles, s, P, stream, true)) != RTGS_OK) return r;
-    } else {
-        if ((r = RTGS_BY_FLAGS(launch_shade_tiles, s, P, stream, false)) != RTGS_OK) return r;
-    }
+    if ((r = RTGS_BY_FLAGS(launch_shade_tiles, s, P, stream)) != RTGS_OK) return r;
     if ((r = mark(2)) != RTGS_OK) return r;
-    P.use_fallback_list = heavy_first ? 2 : 3;
+    // the closing launch renders both hand-over lists
+    P.use_fallback_list = 1;
     P.final_kernel = 1;
-    static const bool stats_fallback_only = getenv("RTGS_STATS_FALLBACK_ONLY") != nullptr;   // diagnostic
-    if (want_stats && stats_fallback_only)
-        CUDA_TRY(cudaMemsetAsync(s->stats_dev, 0, ST_TOTAL * sizeof(unsigned long long), stream));
     if ((r = fused_kernel(16)) != RTGS_OK) return r;
     if (ran) *ran = 7;
     return mark(3);

@@ -39,12 +39,11 @@ struct TileDesc {
 };
 constexpr int TILE_CAPPED = 1 << 30;
 
-// CTR_FALLBACK / CTR_WORK3: tiles the traversal hands to k_render (list pool exhausted, or a group whose frustum holds
-// too many candidates) and the cursor of the launch that renders them; CTR_FALLBACK2 / CTR_WORK4: tiles the shading
-// hands over (three hits within rounding at the K-th place) and their cursor.  Two lists, because the first one is
-// complete BEFORE the shading starts and its tiles are rendered concurrently with it (render.cu).
+// CTR_FALLBACK: tiles the traversal hands to k_render (list pool exhausted, or a group whose frustum holds too many
+// candidates); CTR_FALLBACK2: tiles the shading hands over (three hits within rounding at the K-th place, or a
+// depth-capped list that fell short); CTR_WORK3: the cursor of the closing k_render launch, which renders both lists.
 enum { CTR_WORK = 0, CTR_POOL = 1, CTR_FALLBACK = 2, CTR_WORK2 = 3, CTR_WORK3 = 4, CTR_DONE = 5, CTR_DONE2 = 6,
-       CTR_FALLBACK2 = 7, CTR_WORK4 = 8, CTR_DONE3 = 9,
+       CTR_FALLBACK2 = 7,
        CTR_HEAVY = 10, CTR_WORK5 = 11,   // heavy groups queued by the traversal / the cursor of k_heavy_lists
        CTR_HEAVY_FAILED = 12,            // ... of them handed on to k_render (statistics)
        CTR_COUNT = 16 };
@@ -66,7 +65,6 @@ struct RenderParams {
     const float4* nodes4;     // two-level nodes (k_tile_lists)
     const float4* geo;
     const float4* shp;
-    cudaTextureObject_t geo_tex;   // (experiment SHADE_GEO_TEX) the geometry records as a linear float4 texture
     cudaTextureObject_t shp_tex;   // the same records as a linear float4 texture, or 0 (too many for one texture): eval_colour
                                    // fetches part of a record through the texture path, the rest with 256-bit loads
     const float4* raw;
@@ -89,10 +87,8 @@ struct RenderParams {
     int pool_chunks;
     int* fallback_tiles;      // ntiles: tiles handed over by the traversal (lists_group)
     int* fallback_tiles2;     // ntiles: tiles handed over by the shading (shade_tile)
-    int use_fallback_list;    // k_render: 0 = every tile of the region; bit 0 = the tiles of fallback_tiles, bit 1 =
-                              // those of fallback_tiles2 (both: the first list, then the second)
-    int early_trigger;        // k_render: let the next kernel on the stream start at once (programmatic dependent
-                              // launch): the shading that follows does not depend on this launch
+    int use_fallback_list;    // k_render: 0 = every tile of the region; 1 = the tiles of fallback_tiles, then those of
+                              // fallback_tiles2
     int heavy_fused;          // k_tile_lists: a group whose list overflows shared memory goes to k_render (distance pruning)
     int heavy_limit;          // ... "overflows" = more candidates than this (<= the capacity of the shared-memory list)
     // depth-capped lists of heavy groups (heavy_lists.cuh; all unused while heavy_slab == 0)
@@ -101,11 +97,11 @@ struct RenderParams {
     float* tile_cap;          // ntiles: every Gaussian that can enter a ray of the tile nearer than this is in its list
     int2* heavy_scratch;      // per warp of k_heavy_lists: 2 x heavy_defer_cap deferred (node, depth bits) entries
     int heavy_defer_cap;
-    int slab_rank;            // the cap of a pass = the slab_rank-th smallest of the 32 per-lane nearest deferred depths
     int lists_single;         // lists_group pops one node per step while its stack holds more entries than this (tile_lists.cuh)
     // band completion (host-pipelined framebuffer copy, rtgs_render_host): the frame is cut into nbands bands of
     // band_macro_cols 32-pixel columns; a band is finished when all its tile ids have been rendered or skipped
-    int nbands, band_macro_cols, macro_rows, schedule;
+    int nbands, band_macro_cols, macro_rows;
+    int schedule;             // macro-column order (macro_column): 0 = left to right, 2 = rotated (banded launches)
     unsigned int* band_done;  // device counters, one per band
     int* band_flags;          // mapped pinned host memory: set to 1 by the warp that finishes the band
     int* mirror;              // mapped pinned host memory: [0] list-pool demand of the frame, [1] a frame had fallback tiles
@@ -122,11 +118,8 @@ struct RenderParams {
     unsigned int* arrive;
     const unsigned int* grant;
     unsigned int grant_value;
-    int tail_launch;          // k_frame: the last CTA launches the fused kernel for the fallback tiles itself
-                              // (device-side tail launch) instead of the host queueing a third kernel per frame
     int final_kernel;         // this launch is the frame's last kernel: its last CTA completes the frame (frame_complete)
     int self_clean;           // ... and zeroes the work counters for the next frame (no memset between frames)
-    int tail_grid;            // CTAs of a device-side k_render launch (2 per SM)
     float* out_depth;         // DEPTH instantiations: composited ray distance per pixel, indexed like out_T; may be null
 };
 
@@ -261,8 +254,9 @@ __device__ __forceinline__ void ldg256(const void* p, float4& a, float4& b) {
 // Order in which the macro-tile columns are scheduled (position -> column).  0: left to right (device renders:
 // best locality and a cheap tail).  The banded framebuffer copy of rtgs_render_host wants bands to finish no
 // faster than the DMA drains them at the END of the frame, so that nothing piles up behind the render:
-// 1: from the image edges inwards (0, last, 1, last-1 ...; for a centred scene cheap columns first, expensive
-// last); 2: rotated, the rightmost fifth first, then left to right.
+// 2: rotated, the rightmost fifth first, then left to right (banded launches).  1, from the image edges inwards, is no
+// longer launched; its branch stays because without it ptxas gives k_heavy_lists more spills, and the branch-free
+// rotation (a modulo) cost k_frame 0.9 %.
 __host__ __device__ __forceinline__ int macro_column(int macro_rows, int pos, int schedule) {
     if (schedule == 1) return (pos & 1) ? macro_rows - 1 - (pos >> 1) : (pos >> 1);
     if (schedule == 2) {
@@ -278,8 +272,8 @@ __device__ __forceinline__ int macro_column(const RenderParams& P, int pos) {
 // Work item k of a launch -> tile / group id (>= `total` when the launch is exhausted).  per_col = ids per
 // macro-tile column.  A stripe-sharded launch (RTGS_OPT_STRIPE) enumerates only the columns it owns: pulling
 // and skipping the foreign ids costs an atomic round trip each, and with 7/8 of them foreign that was most of
-// k_tile_lists at 8 GPUs.  (Banded launches and the rotated schedules keep the plain order: their band counters
-// expect every id to be reported.)
+// k_tile_lists at 8 GPUs.  (Banded launches, the rotated schedule, keep the plain order: their band counters expect
+// every id to be reported.)
 __device__ __forceinline__ int work_to_id(const RenderParams& P, int k, int per_col, int total) {
     if (P.stripe_mod <= 1 || P.schedule != 0 || P.nbands > 0) return k;
     const int c = k / per_col;
@@ -572,16 +566,8 @@ __device__ __forceinline__ void stage_candidate(const RenderParams& P, const Til
                                                 float4 (&rec)[REC_QUADS], float (&poly)[6], float& t_lo) {
     const CamD& cam = P.cam;
     float4 g0, g1, g2, g3;
-#if SHADE_GEO_TEX
-    {   // experiment: the 64-byte geometry record through the texture path as well
-        const int t0 = s * 4;
-        g0 = tex1Dfetch<float4>(P.geo_tex, t0); g1 = tex1Dfetch<float4>(P.geo_tex, t0 + 1);
-        g2 = tex1Dfetch<float4>(P.geo_tex, t0 + 2); g3 = tex1Dfetch<float4>(P.geo_tex, t0 + 3);
-    }
-#else
     ldg256(P.geo + (int64_t)s * 4 + 0, g0, g1);
     ldg256(P.geo + (int64_t)s * 4 + 2, g2, g3);
-#endif
     const double W00 = g1.x, W01 = g1.y, W02 = g1.z, W10 = g1.w, W11 = g2.x, W12 = g2.y, W20 = g2.z, W21 = g2.w,
                  W22 = g3.x;
     auto Wmul = [&](const d3& v) {
@@ -687,15 +673,9 @@ __device__ __forceinline__ PreciseHit precise_test(const RenderParams& P, const 
     return h;
 }
 
-#ifndef SHADE_SH_TEX
-#define SHADE_SH_TEX 8     // quads (of 12) of an SH record fetched through the texture path; even.  Measured on the
-#endif                     // bench scene (k_shade_tiles): 0 -> 0.585 ms, 4 -> 0.554, 6 -> 0.544, 8 -> 0.536, 10 -> 0.537, 12 -> 0.551
-#ifndef SHADE_GEO_TEX
-#define SHADE_GEO_TEX 0
-#endif
-#ifndef SHADE_SH_TEX_RUNTIME
-#define SHADE_SH_TEX_RUNTIME 1   // 1: scenes too large for one linear texture fall back to loads at run time (P.shp_tex == 0)
-#endif
+// Quads (of 12) of an SH record fetched through the texture path; even.  Measured on the bench scene (k_shade_tiles):
+// 0 -> 0.585 ms, 4 -> 0.554, 6 -> 0.544, 8 -> 0.536, 10 -> 0.537, 12 -> 0.551.
+constexpr int SHADE_SH_TEX = 8;
 constexpr long long SH_TEX_MAX_RECORDS = (1ll << 27) / 12;   // one linear texture holds 2^27 texels
 static_assert(SHADE_SH_TEX >= 0 && SHADE_SH_TEX <= 12 && SHADE_SH_TEX % 2 == 0, "SHADE_SH_TEX: even, 0..12");
 // rgb = color + eval_sh(normalize(dir))  (gaussian.py:199-200) of the Gaussian at sorted position s.
@@ -710,8 +690,7 @@ __device__ __forceinline__ void eval_colour(const RenderParams& P, int s, const 
         // the rest as 256-bit loads (LSU pipe).  The LSU pipe is what bounds the shading (shared-memory gathers + these
         // loads: 85 % busy before); the texture path has wavefront throughput of its own.  The handle must be
         // warp-uniform (a per-lane choice among several textures made the fetches 35 % slower than no texture at
-        // all), so scenes beyond one linear texture (2^27 texels = 11 M records) take the all-LSU path.
-#if SHADE_SH_TEX_RUNTIME
+        // all), so scenes beyond one linear texture (2^27 texels = 11 M records) take the all-LSU path (P.shp_tex == 0).
         if (P.shp_tex == 0) {
 #pragma unroll
             for (int f = 0; f < SHADE_SH_TEX / 2; ++f) {
@@ -720,9 +699,7 @@ __device__ __forceinline__ void eval_colour(const RenderParams& P, int s, const 
                 v[8 * f] = x.x; v[8 * f + 1] = x.y; v[8 * f + 2] = x.z; v[8 * f + 3] = x.w;
                 v[8 * f + 4] = y.x; v[8 * f + 5] = y.y; v[8 * f + 6] = y.z; v[8 * f + 7] = y.w;
             }
-        } else
-#endif
-        {
+        } else {
 #pragma unroll
             for (int f = 0; f < SHADE_SH_TEX; ++f) {
                 const float4 x = tex1Dfetch<float4>(P.shp_tex, s * 12 + f);

@@ -31,17 +31,6 @@
 
 namespace rtgs_dev {
 
-#ifndef SHADE_POOL_LDG
-#define SHADE_POOL_LDG 0   // experiment: candidate chunks through the read-only (L1) path; only safe with separate launches
-#endif
-#if SHADE_POOL_LDG
-#define POOL_LOAD __ldg
-#else
-#define POOL_LOAD __ldcg
-#endif
-#ifndef SHADE_SLOT_ORDER
-#define SHADE_SLOT_ORDER 0
-#endif
 constexpr int SHADE_K = 16;          // k-buffer entries (depth <= 16)
 constexpr float TIE_BAND = 2e-6f;    // relative: float32 entry distances closer than this are compared in float64
 constexpr int SHADE_BATCH = REC_BATCH;   // staged candidates per batch (a chunk fills 31)
@@ -95,15 +84,16 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
     if (desc_count > 0) {
         make_tile_rays(cam, i0, j0, pi, pj, active, tr);
         int left = desc_count;
-        // one coalesced 128-byte read per chunk: lanes 0..30 candidates, lane 31 the next chunk
-        int cur = POOL_LOAD(P.pool + (int64_t)desc.head * CHUNK_INTS + lane);
+        // one coalesced 128-byte read per chunk: lanes 0..30 candidates, lane 31 the next chunk (L2 only: in k_frame
+        // the chunks are written by other warps of the same launch)
+        int cur = __ldcg(P.pool + (int64_t)desc.head * CHUNK_INTS + lane);
 #pragma unroll 1
         while (left > 0) {
             const int m = (left - 1) % CHUNK_IDS + 1;
             left -= m;
             const int s = cur;
             const int next = __shfl_sync(FULL, cur, CHUNK_INTS - 1);
-            if (left > 0) cur = POOL_LOAD(P.pool + (int64_t)next * CHUNK_INTS + lane);   // prefetch
+            if (left > 0) cur = __ldcg(P.pool + (int64_t)next * CHUNK_INTS + lane);   // prefetch
             // ---- stage ---------------------------------------------------------------------
             const int m4 = (m + 3) & ~3;
             if (lane < m) {
@@ -265,34 +255,6 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
         sh_direction(cam, i0, j0, pi, pj, active, dx, dy, dz);
         sh_basis(dx, dy, dz, Y);
         const int nmine = min(cnt, P.depth);
-#if SHADE_SLOT_ORDER
-        // Weights first: w_k = T_k alpha_k depends on the alphas and their depth order only, so the ordered pass
-        // touches no colour data; the colour sum  accum = sum_k w_k rgb_k  is then taken in SLOT order.  Slots fill
-        // in list order, which all rays of the tile share, so lanes that hold the same Gaussian tend to reach it
-        // in the same iteration and share its SH record (one L1 wavefront set instead of several).
-#pragma unroll 1
-        for (int k = 0; k < cnt; ++k) {
-            const int slot = (int)((perm >> (4 * k)) & 15u);
-            const float alpha = ws.kb_a[slot][lane];
-            const bool use = k < nmine && T >= P.t_cut;
-            ws.kb_a[slot][lane] = use ? T * alpha : 0.0f;
-            if (use) {
-                T *= 1.0f - alpha;
-                ++nl;
-            }
-        }
-#pragma unroll 1
-        for (int slot = 0; slot < maxcnt; ++slot) {
-            const float wgt = slot < cnt ? ws.kb_a[slot][lane] : 0.0f;
-            if (wgt != 0.0f) {
-                float r, g, b;
-                eval_colour(P, ws.kb_i[slot][lane], Y, r, g, b);
-                cr = fmaf(wgt, r, cr);
-                cg = fmaf(wgt, g, cg);
-                cb = fmaf(wgt, b, cb);
-            }
-        }
-#else
         const int nloop = min(maxcnt, P.depth);
 #pragma unroll 1
         for (int k = 0; k < nloop; ++k) {
@@ -310,9 +272,7 @@ __device__ __forceinline__ void shade_tile(const RenderParams& P, ShadeShared& w
                 ++nl;
             }
         }
-#endif
         if constexpr (DEPTH) {
-            static_assert(!(DEPTH && SHADE_SLOT_ORDER), "SHADE_SLOT_ORDER overwrites the alphas composite_depth reads");
             D = composite_depth(P, i0, j0, pi, pj, active, nmine, min(maxcnt, P.depth), [&](int k, int& s, float& a) {
                 const int slot = (int)((perm >> (4 * k)) & 15u);
                 s = ws.kb_i[slot][lane];

@@ -26,9 +26,7 @@
 
 namespace rtgs_dev {
 
-#ifndef LISTS_NODES_PER_STEP
-#define LISTS_NODES_PER_STEP 16
-#endif
+constexpr int LISTS_NODES_PER_STEP = 16;
 constexpr int LISTS_TAKE = LISTS_NODES_PER_STEP;
 static_assert(LISTS_TAKE == 16 || LISTS_TAKE == 32, "nodes per traversal step: 16 (lane pair per node) or 32");
 
@@ -36,12 +34,12 @@ static_assert(LISTS_TAKE == 16 || LISTS_TAKE == 32, "nodes per traversal step: 1
 // Above P.lists_single entries one node is popped per step (depth first): growth <= 3 per two-level step, i.e.
 // <= 3 * ceil(depth / 2) over a whole descent, `depth` being the depth of the scene's deepest leaf (measured by
 // the build, lbvh.cu: k_max_depth; <= RTGS_MAX_TREE_DEPTH).  The host sets
-//   lists_single = min(tuned value, LISTS_STACK_CAP - 3 * LISTS_TAKE - 3 * ceil(depth / 2))    (render.cu)
+//   lists_single = min(LISTS_SINGLE, LISTS_STACK_CAP - 3 * LISTS_TAKE - 3 * ceil(depth / 2))    (render.cu)
 // so the stack cannot overflow whatever the tree looks like; shallow trees (every real scene: ~30 levels for 1 M
-// Gaussians) get the batch size that is fastest, the deepest possible tree degrades to depth-first early.
-#ifndef LISTS_STACK_ENTRIES
-#define LISTS_STACK_ENTRIES 256
-#endif
+// Gaussians) get the batch threshold that is fastest (LISTS_SINGLE), the deepest possible tree degrades to
+// depth-first early.
+constexpr int LISTS_SINGLE = 112;
+constexpr int LISTS_STACK_ENTRIES = 256;
 constexpr int LISTS_STACK_CAP = LISTS_STACK_ENTRIES;
 static_assert(LISTS_STACK_CAP - 3 * LISTS_TAKE - 3 * ((RTGS_MAX_TREE_DEPTH + 1) / 2) >= 4,
               "lists_group: stack too small for the deepest tree");
